@@ -13,6 +13,7 @@ figure BASELINE.json's 2 ms target refers to).
   python bench.py --gpus N --steps K --warmup W            (our arm; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W   (CPU oracle port, rank 0 only)
   python bench.py --workload c5 [--points P] [--verify]    (BASELINE config 5: one cloud in slab mode, torchrun for N > 1)
+  python bench.py ... --dump-outputs DIR                   (also write what the last timed step computed, see dump_outputs)
 
 `value`  : frames resident in HBM before the timed region; CUDA events around each step (recorded after every
            handle's stream has drained), per-stage times from each handle's own events on its own stream.
@@ -121,6 +122,23 @@ def make_frames(rank, count, base_seed=20020):
     return [synth.make_frame(seed=base_seed + rank * 1000 + i) for i in range(count)]
 
 
+DUMP_FRAMES = 16        # --dump-outputs: the last frames of the last timed step
+DUMP_ROWS = 1 << 15     # rows kept of one array of one frame
+
+
+def dump_outputs(out_dir, results):
+    """results: [(frame index within the step, Segmenter)].  Writes what Segmenter.fetch_result() hands a caller for each frame
+    -- the labelled voxel cloud and the merge log -- as out_dir/frame<k>_<name>.npy: float32 stays float32, the uint32 arrays
+    become float64 (exact).  An array of more than DUMP_ROWS rows keeps DUMP_ROWS of them, drawn by np.random.default_rng(k) and
+    kept in order.  At most DUMP_FRAMES x 2 MiB = 32 MiB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    for k, seg in results:
+        for name, a in seg.fetch_result().items():
+            if a.shape[0] > DUMP_ROWS:
+                a = a[np.sort(np.random.default_rng(k).choice(a.shape[0], DUMP_ROWS, replace=False))]
+            np.save(os.path.join(out_dir, "frame%04d_%s.npy" % (k, name)), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def shared_config(workload):
     """The `config` both arms print (the driver compares the two dicts): what is measured, nothing about how."""
     flags = {"c2": "--CVX --AL -t 0.2", "c3": "--EQ 200 -t 0.2", "c5": "-v 0.01 -s 0.1 --CVX --AL -t 0.2"}[workload]
@@ -201,8 +219,9 @@ def cpu_baseline(frame, FLAGS=FLAGS):
 
 
 # ------------------------------------------------------------------------------------------------
-def sweep_leg(args, env, workload, steps):
-    """One measured leg of the frame sweep (C2 or C3): resident throughput, host-buffer throughput, single-frame latency."""
+def sweep_leg(args, env, workload, steps, dump_dir=None):
+    """One measured leg of the frame sweep (C2 or C3): resident throughput, host-buffer throughput, single-frame latency.
+    dump_dir: rank 0 writes the results of the last timed step's final frames there (dump_outputs)."""
     import torch
     import f3ps
     from f3ps import sweep
@@ -264,6 +283,11 @@ def sweep_leg(args, env, workload, steps):
     clocks = sampler.stop()
     t_dev = sum(a.elapsed_time(b) for a, b in ev) / 1e3          # seconds, this rank
     counts = pool.segs[0].counts()
+    if dump_dir and rank == 0:
+        # the handle that ran frame k of a step: BatchPool alternates two sets of F handles between groups of F frames,
+        # FramePool deals the frames round-robin over its F handles; each handle still holds the last frame it ran
+        last = {(k // F % 2 * F if args.pool == "batch" else 0) + k % F: k for k in range(F * R)}
+        dump_outputs(dump_dir, sorted((k, pool.segs[h]) for h, k in last.items())[-DUMP_FRAMES:])
 
     # end-to-end through the public API with host buffers (H2D of the points, D2H of the labelled cloud + merge log)
     for i in range(2):
@@ -328,7 +352,7 @@ def run_ours(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     env = (dist, world, rank, local_rank, dev)
-    m = sweep_leg(args, env, args.workload, args.steps)
+    m = sweep_leg(args, env, args.workload, args.steps, args.dump_outputs)
     c3 = sweep_leg(args, env, "c3", max(2, args.steps // 2)) if (args.workload == "c2" and not args.no_c3) else None
 
     if rank == 0:
@@ -443,6 +467,8 @@ def run_slab(args):
     torch.cuda.synchronize()
     launches = ss.seg.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [(0, ss.seg)])              # every rank holds the whole cloud's result
     keys = sorted(stage)
     t = torch.tensor([sum(times) / 1e3] + [stage[k] for k in keys], dtype=torch.float64, device=dev)
     if world > 1:
@@ -506,7 +532,11 @@ def main():
     ap.add_argument("--no-c3", action="store_true", help="c2: skip the C3 leg")
     ap.add_argument("--points", type=int, default=50_000_000, help="c5: points of the merged scan")
     ap.add_argument("--verify", action="store_true", help="c5: compare the slab result with one handle processing the whole cloud")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the labelled voxel clouds and merge logs of the "
+                    "last step's final %d frames (c5: of the cloud) as DIR/frame<k>_<name>.npy, rows sampled beyond %d" % (DUMP_FRAMES, DUMP_ROWS))
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has none")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "c5":

@@ -56,7 +56,7 @@ def test_oracle_reproduces_reference_clustering(oracle_mod, name, impl):
     assert np.array_equal(bits(o.array("out_xyz")), bits(want["out_xyz"]))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/clustering.cpp"), reason="the reference tree exists in the build container only")
+@pytest.mark.reference("src/clustering.cpp")
 def test_oracle_reproduces_reference_clustering_live(oracle_mod):
     """fresh hub graphs (other seeds, sizes and flag sets than the committed ones) through the compiled reference class"""
     sys.path.insert(0, os.path.join(ROOT, "tools"))
@@ -121,7 +121,7 @@ def test_oracle_reproduces_reference_all_thresh(oracle_mod, name):
     assert np.float32(bt) == best[0] and abs(bp["fscore"] - best[4]) <= 2e-7
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/color_utilities.cpp"), reason="the reference tree exists in the build container only")
+@pytest.mark.reference("src/color_utilities.cpp")
 def test_oracle_colour_distances_equal_reference_live(oracle_mod):
     """ColorUtilities::lab_ciede00 / rgb_eucl of the compiled reference on 200,000 random pairs (hue wrap-arounds, greys, identical
     colours, the corners of the gamut) against the oracle's restatement: bit for bit (same libm, same float / double mix)."""
@@ -151,7 +151,7 @@ def test_oracle_colour_distances_equal_reference_live(oracle_mod):
     assert np.array_equal(bits(head), bits(ref_de[:6100:7]))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/clustering.cpp"), reason="the reference tree exists in the build container only")
+@pytest.mark.reference("src/clustering.cpp")
 def test_reference_exception_behaviour_live():
     """The exception types of the compiled reference, case by case: what host/facade.cpp throws and what the C ABI's status codes map to
     (F3PS_ERR_LOGIC / F3PS_ERR_INVALID_ARGUMENT / std::out_of_range; tests/test_gpu_parity.py::test_error_behaviour_matches_reference,

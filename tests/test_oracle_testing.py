@@ -40,7 +40,7 @@ def test_restatement_equals_reference_testing_class_golden():
     assert exact >= len(d["cases"]) - 4                          # (36 of 38 bit-identical when the fixture was made)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/testing.cpp"), reason="the reference tree exists in the build container only")
+@pytest.mark.reference("src/testing.cpp")
 def test_restatement_equals_reference_testing_class_live():
     """fresh random clouds through the compiled reference class (not only the committed ones)"""
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "ref"])

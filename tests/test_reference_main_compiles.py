@@ -3,14 +3,15 @@
 getSupervoxelAdjacencyList / label2color / set_initialstate / all_thresh / best_thresh / cluster / get_currentstate /
 Testing::eval_performance -- are compiled VERBATIM against include/supervoxel_clustering/ (g++ -fsyntax-only).  Only what the
 reference takes from Boost and from PCL's console / io modules is replaced by compile-only stand-ins; every class and method
-on the path must exist in the shim with a signature those lines accept.  Runs where /root/reference exists (the build container)."""
+on the path must exist in the shim with a signature those lines accept.  Runs when F3PS_REFERENCE_DIR names a checkout of the
+original project."""
 import os
 import subprocess
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src/supervoxel_clustering.cpp"
+REF = os.path.join(os.environ.get("F3PS_REFERENCE_DIR", ""), "src", "supervoxel_clustering.cpp")
 
 HARNESS = r'''
 #include <cmath>
@@ -65,7 +66,7 @@ int reference_main_body(std::vector<std::string> file_list, bool disable_transfo
 '''
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="the reference tree is only present in the build container")
+@pytest.mark.reference("src/supervoxel_clustering.cpp")
 def test_reference_main_hot_path_compiles_against_the_shim(tmp_path):
     lines = open(REF).read().splitlines()
     body = "\n".join(lines[302:457])

@@ -23,6 +23,8 @@ OUT = os.path.join(ROOT, "tests", "golden", "clustering_ref.npz")
 
 
 def ref_lib():
+    if not os.path.isdir(os.environ.get("F3PS_REFERENCE_DIR", "")):
+        raise SystemExit("set F3PS_REFERENCE_DIR to a checkout of the original project: oracle/_ref/libref_clustering.so is built from its sources")
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s"])
     lib = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_clustering.so"))
     lib.ref_cluster.restype = C.c_int

@@ -17,6 +17,8 @@ OUT = os.path.join(ROOT, "tests", "golden", "testing_ref.json")
 
 
 def ref_lib():
+    if not os.path.isdir(os.environ.get("F3PS_REFERENCE_DIR", "")):
+        raise SystemExit("set F3PS_REFERENCE_DIR to a checkout of the original project: oracle/_ref/libref_clustering.so is built from its sources")
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "ref"])
     lib = C.CDLL(LIB)
     lib.ref_testing_eval.restype = C.c_int
