@@ -111,10 +111,8 @@ struct f3ps_ctx {
     f3ps::DevBuf pos_data_buf, merge_scratch, adj_pool, merge_trace;
     unsigned merge_trace_first = 0;
     const float4* pos_data = nullptr;   // voxel (x,y,z,rgba) in position order (what the merge folds stream)
-    int merge_path = 0;                 // 1 = resident kernel, 2 = general kernel (last f3ps_merge)
-    bool force_general_merge = false;   // f3ps_set_merge_kernel(ctx, 2)
-    bool merge_take_over = false;       // f3ps_merge_batch -> f3ps_merge: continue the replay the batch grid stopped (state after n merges), do not restart
-    int merge_kernel_choice = 0;        // 0 auto, 1 resident single CTA, 2 general, 3 resident with its tables in L2, 4 / 5 = 1 / 3 with phase counters
+    int merge_path = 0;                 // what the last replay ran (f3ps_counts.merge_path)
+    int merge_kernel_choice = 0;        // 0 auto, 2 general, 3 resident with its tables in L2, 4 = auto with phase counters in the shared-memory variant, 5 = 3 with phase counters
     f3ps::MergeLog ML{};
     unsigned n_pos = 0;           // positions of the label-ordered voxel list
     const unsigned* order = nullptr;
@@ -136,6 +134,5 @@ struct f3ps_ctx {
     int expand_cluster_ctas = 0;        // cap of the cluster size (0 = by V, at most 16)
     int expand_path = 0;                // what the last f3ps_expand launched: 1 cooperative / shared grid, 2 cluster
     bool expand_cluster_attr_set = false;
-    bool general_attr_set = false;
     bool lambda_attr_set = false;
 };

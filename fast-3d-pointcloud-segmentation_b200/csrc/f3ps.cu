@@ -758,50 +758,62 @@ unsigned lean_ecap_for(unsigned E, int threads = kFastThreads) {
     const unsigned nb = std::max(1u, (E + owners - 1u) / owners);
     return nb <= 32u ? std::max(32u, (E + 31u) & ~31u) : 0u;
 }
-// one frame alone runs the 768-thread build (80 registers) when its edges fit 21 worker warps
-void (*lean_kernel_for(bool prof, bool solo))(FastArgs) {
-    if (solo) return prof ? merge_fast_kernel<true, kFastThreadsSolo> : merge_fast_kernel<false, kFastThreadsSolo>;
-    return prof ? merge_fast_kernel<true, kFastThreads> : merge_fast_kernel<false, kFastThreads>;
-}
 // adjacency pool of the resident kernel (edge ids, 2 bytes each): the initial lists plus room for the lists that outgrow their block
 constexpr size_t kLeanPoolSlack = 1u << 20;
-int lean_pool(f3ps_ctx* ctx, unsigned E, FastArgs& A, bool big = false) {      // (edge ids: 2 bytes, BIG variant 4)
-    const size_t entries = 2 * (size_t)E + (big ? 8 : 1) * kLeanPoolSlack;
-    F3PS_CUDA_OK(ctx->adj_pool.ensure(entries * (big ? 4 : 2)));
-    A.adj_pool = ctx->adj_pool.as<unsigned short>(); A.pool_cap = (unsigned)entries;
-    return F3PS_OK;
-}
+constexpr size_t kSmemMax = 227u * 1024u;
 // The opt-in to > 48 KB of dynamic shared memory is per function AND per device: remember it per (device, function).
-int lean_attr(f3ps_ctx* ctx, const void* kern) {
+int smem_opt_in(f3ps_ctx* ctx, const void* kern, size_t bytes) {
     static std::mutex m;
     static std::set<std::pair<int, const void*>> done;
     std::lock_guard<std::mutex> l(m);
     if (done.count({ctx->device, kern})) return F3PS_OK;
-    F3PS_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    F3PS_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
     done.insert({ctx->device, kern});
     return F3PS_OK;
 }
+// Which kernel replays a handle's merges.  The kinds carry the merge_path of a replay that stays on one kernel.
+enum MergeKind { kMergeShared = 1, kMergeGeneral = 2, kMergeL2 = 3 };
+struct MergePlan {
+    MergeKind kind;
+    bool prof;               // resident kernel built with phase counters (kernel choice 4 / 5)
+    bool to_l2;              // kMergeShared: a merge with more adjacency entries than worker threads continues on the L2 variant
+    int threads; unsigned S_cap, E_cap; size_t smem;     // resident kernel: block size, table capacities, dynamic shared memory
+};
+// the resident kernel with its big tables in global memory, for graphs that do not fit an SM (16-bit region ids, 32-bit edge ids;
+// 16 bytes of shared memory per block of 32 edges bound E near 380,000)
+MergePlan plan_l2(const f3ps_ctx* ctx) {
+    const unsigned S = ctx->S, E = ctx->E;
+    MergePlan p{kMergeL2, ctx->merge_kernel_choice == 5, false, kFastThreads, (S + 7u) & ~7u, (E + 31u) & ~31u, 0};
+    p.smem = FastSmem(nullptr, p.S_cap, p.E_cap, (char*)16).bytes;
+    if (ctx->n_pos == 0 || S >= 65535u || p.E_cap > (1u << 20) || p.smem > kSmemMax) p.kind = kMergeGeneral;
+    return p;
 }
+MergePlan plan_merge(const f3ps_ctx* ctx) {
+    const unsigned S = ctx->S, E = ctx->E; const int choice = ctx->merge_kernel_choice;
+    MergePlan l2 = plan_l2(ctx);
+    if (choice == 2) l2.kind = kMergeGeneral;
+    // the resident kernel with its tables in shared memory when the graph fits one SM (kernels_merge_lean.cuh)
+    const unsigned S_cap = (S + 7u) & ~7u, E_cap = lean_ecap_for(E);
+    if (choice == 2 || choice == 3 || choice == 5 || !E_cap || S > 4096u || ctx->n_pos == 0) return l2;
+    const size_t smem = FastSmem(nullptr, S_cap, E_cap).bytes;
+    if (smem > kSmemMax) return l2;
+    // one frame alone runs the 768-thread build (80 registers) when its edges fit 21 worker warps and a merge wider than its 672
+    // worker threads can continue on the L2 variant
+    const bool to_l2 = l2.kind == kMergeL2, solo = to_l2 && lean_ecap_for(E, kFastThreadsSolo) != 0u;
+    return MergePlan{kMergeShared, choice == 4, to_l2, solo ? kFastThreadsSolo : kFastThreads, S_cap, E_cap, smem};
 }
-int f3ps_merge(f3ps_ctx* ctx, float threshold) {
-    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
-    if (ctx->progress < P_EXPANDED)                            // std::logic_error of Clustering::cluster (src/clustering.cpp:671-673)
-        return ctx_fail(ctx, F3PS_ERR_LOGIC, "Cannot call 'cluster' before setting an initial state with 'set_initialstate'");
-    cudaSetDevice(ctx->device);
-    int rc;
-    if (ctx->progress < P_GRAPH) { rc = f3ps_graph(ctx); if (rc) return rc; }   // if (!init_initial_weights) init_weights()  (:675-676)
-    rc = mark(ctx, 7); if (rc) return rc;
-    const unsigned S = ctx->S, E = ctx->E, P = ctx->n_pos; const size_t Sc = std::max(1u, S), Ec = std::max(1u, E), Pc = std::max(1u, P);
-    // cluster(float) always restarts from initial_state (:678) -- unless f3ps_merge_batch hands over a replay its grid stopped in front
-    // of a merge with too many adjacency entries (the working state and the counters are then those after n merges)
-    const bool take_over = ctx->merge_take_over;
-    ctx->merge_take_over = false;
-    const size_t eb = std::min(ctx->edge_init.cap, ctx->edge_work.cap);
-    if (!take_over) {
-        F3PS_CUDA_OK(cudaMemcpyAsync(ctx->reg_work.p, ctx->reg_init.p, region_bytes(Sc), cudaMemcpyDeviceToDevice, ctx->stream));
-        F3PS_CUDA_OK(cudaMemcpyAsync(ctx->edge_work.p, ctx->edge_init.p, eb, cudaMemcpyDeviceToDevice, ctx->stream));
-        F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl), 0, sizeof(MergeCtl), ctx->stream));
-    }
+// cluster(float) restarts from initial_state (src/clustering.cpp:678): working regions and edges, merge counters
+int merge_restart(f3ps_ctx* ctx) {
+    F3PS_CUDA_OK(cudaMemcpyAsync(ctx->reg_work.p, ctx->reg_init.p, region_bytes(std::max(1u, ctx->S)), cudaMemcpyDeviceToDevice, ctx->stream));
+    F3PS_CUDA_OK(cudaMemcpyAsync(ctx->edge_work.p, ctx->edge_init.p, std::min(ctx->edge_init.cap, ctx->edge_work.cap), cudaMemcpyDeviceToDevice, ctx->stream));
+    F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl), 0, sizeof(MergeCtl), ctx->stream));
+    return F3PS_OK;
+}
+// start of a replay: restart (unless the working state is the one to continue from), merge log, output buffers
+int merge_begin(f3ps_ctx* ctx, bool restart) {
+    int rc = mark(ctx, 7); if (rc) return rc;
+    if (restart && (rc = merge_restart(ctx))) return rc;
+    const size_t Sc = std::max(1u, ctx->S), Pc = std::max(1u, ctx->n_pos);
     F3PS_CUDA_OK(ctx->mlog.ensure(Sc * 20));
     char* lp = (char*)ctx->mlog.p;
     ctx->ML.a = (unsigned*)lp; ctx->ML.b = (unsigned*)(lp + Sc * 4); ctx->ML.w = (float*)(lp + Sc * 8);
@@ -811,136 +823,144 @@ int f3ps_merge(f3ps_ctx* ctx, float threshold) {
     F3PS_CUDA_OK(ctx->vox_segment.ensure(Pc * 4));
     F3PS_CUDA_OK(cudaMemsetAsync(ctx->vox_segment.p, 0xff, Pc * 4, ctx->stream));
     F3PS_CUDA_OK(cudaMemsetAsync(SC(n_out), 0, 4, ctx->stream));
-    if (S) {
-        EdgeParams ep = edge_params(ctx);
-        // resident kernel when the graph fits one SM (kernels_merge_lean.cuh), else the general one
-        const unsigned S_cap = (S + 7u) & ~7u;
-        const unsigned E_cap = std::max(32u, lean_ecap_for(E));
-        const size_t fast_bytes = FastSmem(nullptr, S_cap, E_cap).bytes;
-        const bool single_ok = lean_ecap_for(E) && S <= 4096u && fast_bytes <= 227u * 1024u && P > 0 && ctx->merge_kernel_choice != 3 && ctx->merge_kernel_choice != 5;
-        // graphs that do not fit an SM: the same kernel with its big tables in global memory (16-bit region ids, 32-bit edge ids;
-        // 16 bytes of shared memory per block of 32 edges bound E near 380,000)
-        const unsigned E_big = (E + 31u) & ~31u;
-        const bool big_ok = !single_ok && P > 0 && S < 65535u && E_big <= (1u << 20) && ctx->merge_kernel_choice != 1 &&
-                            FastSmem(nullptr, S_cap, E_big, (char*)16).bytes <= 227u * 1024u;
-        bool fast = !ctx->force_general_merge && (single_ok || big_ok);
-        // a graph that fits an SM but has a merge with more adjacency entries than worker threads continues on the L2 variant (which
-        // loops over the entries) instead of handing single merges to the general kernel
-        const bool can_switch = single_ok && P > 0 && ctx->merge_kernel_choice != 1 && FastSmem(nullptr, S_cap, E_big, (char*)16).bytes <= 227u * 1024u;
-        bool use_big = !single_ok;
-        // general kernel (any graph); resume: continue from the state the resident kernel left; stop_after: hand back after that many merges
-        auto launch_general = [&](bool resume, unsigned stop_after) -> int {
-            const size_t per = ((size_t)Ec * 4 + 255) & ~(size_t)255, per8 = ((size_t)Ec * 8 + 255) & ~(size_t)255;
-            unsigned n2 = 2048; while (n2 < Ec) n2 <<= 1;
-            const size_t perS = ((size_t)Sc * 4 + 255) & ~(size_t)255, sortb = (size_t)n2 * sizeof(MergeSortRec);
-            F3PS_CUDA_OK(ctx->merge_scratch.ensure(6 * per + 2 * per8 + per + per8 + perS + sortb));
-            char* sp = (char*)ctx->merge_scratch.p;
-            MergeScratch scr;
-            scr.st[0] = (long long*)sp; sp += per8; scr.st[1] = (long long*)sp; sp += per8;
-            scr.sortbuf = (MergeSortRec*)sp; sp += sortb;
-            scr.e[0] = (int*)sp; sp += per; scr.e[1] = (int*)sp; sp += per; scr.w[0] = (float*)sp; sp += per; scr.w[1] = (float*)sp; sp += per;
-            scr.x[0] = (unsigned*)sp; sp += per; scr.x[1] = (unsigned*)sp; sp += per; scr.cls = (unsigned char*)sp; sp += per;
-            scr.mark = (unsigned*)sp; sp += perS;
-            const size_t dyn = (size_t)kMergeSortSmem * sizeof(MergeSortRec);
-            if (!ctx->general_attr_set) {
-                F3PS_CUDA_OK(cudaFuncSetAttribute(merge_kernel<unsigned>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-                F3PS_CUDA_OK(cudaFuncSetAttribute(merge_kernel<unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-                ctx->general_attr_set = true;
-            }
-            if (S < 65536u)
-                LAUNCH(ctx, merge_kernel<unsigned>, 1, kMergeThreads, dyn, ctx->R1, ctx->E1, SC(n_edges), SC(xctl.n_sv), ep, SC(lambda), threshold, ctx->run_start.as<unsigned>(),
-                       ctx->run_end.as<unsigned>(), ctx->order, ctx->gxyz, ctx->sv_label.as<unsigned>(), ctx->ML, (unsigned)Sc, SC(mctl), scr, (unsigned*)sp, ctx->pos_data, resume ? 1 : 0, stop_after);
-            else
-                LAUNCH(ctx, merge_kernel<unsigned long long>, 1, kMergeThreads, dyn, ctx->R1, ctx->E1, SC(n_edges), SC(xctl.n_sv), ep, SC(lambda), threshold, ctx->run_start.as<unsigned>(),
-                       ctx->run_end.as<unsigned>(), ctx->order, ctx->gxyz, ctx->sv_label.as<unsigned>(), ctx->ML, (unsigned)Sc, SC(mctl), scr, (unsigned long long*)sp, ctx->pos_data, resume ? 1 : 0, stop_after);
-            return F3PS_OK;
-        };
-        // resident kernel (shared-memory tables, or the BIG variant with its tables in L2)
-        auto launch_resident = [&](bool resume) -> int {
-            FastArgs A;
-            A.R = ctx->R1; A.E = ctx->E1; A.n_edges_ptr = SC(n_edges); A.n_sv_ptr = SC(xctl.n_sv); A.ep = ep; A.lambda_dev = SC(lambda);
-            A.threshold = threshold; A.run_start = ctx->run_start.as<unsigned>(); A.run_end = ctx->run_end.as<unsigned>();
-            A.pos_data = ctx->pos_data; A.sv_label = ctx->sv_label.as<unsigned>(); A.mlog = ctx->ML; A.log_cap = (unsigned)Sc;
-            A.ctl = SC(mctl); A.S_cap = S_cap;
-            A.E_cap = !use_big ? E_cap : E_big;
-            A.big = nullptr; A.big_cursor = nullptr; A.resume = resume ? 1 : 0;
-            const bool solo = !use_big && lean_ecap_for(E, kFastThreadsSolo) != 0u && can_switch;      // (a wider merge than 672 entries continues on the L2 variant)
-            void (*kern)(FastArgs) = !use_big ? lean_kernel_for(ctx->merge_kernel_choice == 4, solo) : (ctx->merge_kernel_choice == 5 ? merge_fast_big_kernel<true> : merge_fast_big_kernel<false>);
-            size_t launch_bytes = fast_bytes;
-            if (use_big) {
-                const size_t bb = (FastSmem::big_bytes(S_cap, E_big) + 255) & ~(size_t)255;
-                F3PS_CUDA_OK(ctx->lean_big.ensure(bb + lean_cursor_bytes(S_cap) + LeanWideScratch::bytes));
-                A.big = (char*)ctx->lean_big.p; A.big_cursor = (unsigned*)((char*)ctx->lean_big.p + bb);
-                launch_bytes = FastSmem(nullptr, S_cap, E_big, A.big).bytes;
-            }
-            int r = lean_attr(ctx, (const void*)kern); if (r) return r;
-            r = lean_pool(ctx, E, A, use_big); if (r) return r;
-            A.trace = nullptr; A.trace_first = ctx->merge_trace_first;
-            if (ctx->merge_kernel_choice == 4 && !use_big && !resume) {
-                F3PS_CUDA_OK(ctx->merge_trace.ensure(256 * 32 * 4));
-                F3PS_CUDA_OK(cudaMemsetAsync(ctx->merge_trace.p, 0, 256 * 32 * 4, ctx->stream));
-                A.trace = ctx->merge_trace.as<unsigned>();
-            }
-            kern<<<1, solo ? kFastThreadsSolo : kFastThreads, launch_bytes, ctx->stream>>>(A);
-            ctx->launches++;
-            F3PS_CUDA_OK(cudaPeekAtLastError());
-            return F3PS_OK;
-        };
-        rc = mark(ctx, 9); if (rc) return rc;
-        if (!fast) { rc = launch_general(false, 0); if (rc) return rc; ctx->merge_path = 2; }
-        else {
-            // The resident kernel stops IN FRONT of a merge whose two adjacency lists hold more entries than it has worker threads
-            // (nothing of that merge has happened; its state is that after n merges).  The general kernel then replays exactly that
-            // merge from the same state and hands back; after kHandOvers such hand-overs (a scene full of hubs) it keeps the rest.
-            constexpr int kHandOvers = 16;
-            ctx->merge_path = single_ok ? 1 : 3;
-            bool resume = false;
-            for (int hand = 0;; ++hand) {
-                unsigned err = kFastErrTouched;                  // (take-over: the batch grid already stopped in front of a wide merge)
-                if (!(take_over && hand == 0)) {
-                    rc = launch_resident(resume); if (rc) return rc;
-                    rc = pull_scalars(ctx); if (rc) return rc;   // did the resident kernel finish?
-                    err = ctx->h_sc->mctl.error;
-                }
-                if (err == 0) break;
-                if (err == kFastErrTouched) {
-                    F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl.error), 0, 4, ctx->stream));
-                    if (!use_big && can_switch) { use_big = true; resume = true; ctx->merge_path = 6; continue; }   // same state, tables in L2 from here on
-                    ctx->merge_path = single_ok ? 4 : 5;
-                    rc = launch_general(true, hand < kHandOvers ? 1u : 0u); if (rc) return rc;
-                    if (hand >= kHandOvers) break;
-                    resume = true;
-                    continue;
-                }
-                // adjacency pool / stamp range exhausted: start over on the general kernel
-                F3PS_CUDA_OK(cudaMemcpyAsync(ctx->reg_work.p, ctx->reg_init.p, region_bytes(Sc), cudaMemcpyDeviceToDevice, ctx->stream));
-                F3PS_CUDA_OK(cudaMemcpyAsync(ctx->edge_work.p, ctx->edge_init.p, eb, cudaMemcpyDeviceToDevice, ctx->stream));
-                F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl), 0, sizeof(MergeCtl), ctx->stream));
-                rc = launch_general(false, 0); if (rc) return rc;
-                ctx->merge_path = 2;
-                break;
-            }
-        }
-        rc = mark(ctx, 10); if (rc) return rc;
-        LAUNCH(ctx, dense_label_kernel, 1, 1024, 0, ctx->R1, SC(xctl.n_sv), ctx->run_start.as<unsigned>(), ctx->run_end.as<unsigned>(), ctx->run_out_off.as<unsigned>(),
-               ctx->run_dense.as<unsigned>(), ctx->region_dense.as<unsigned>(), SC(n_out));
-        if (P) LAUNCH(ctx, labeled_cloud_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), P, ctx->order, ctx->run_start.as<unsigned>(),
-                      ctx->run_out_off.as<unsigned>(), ctx->run_dense.as<unsigned>(), ctx->gxyz, ctx->out_xyz.as<float>(), ctx->out_label.as<unsigned>(),
-                      ctx->out_voxel.as<unsigned>(), ctx->vox_segment.as<unsigned>(), ctx->graph_from_host ? nullptr : ctx->sorted_label,
-                      ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>());
+    return F3PS_OK;
+}
+// the resident kernel's arguments for one frame; resume: continue from the state in the working arrays (counters in mctl)
+int fast_args(f3ps_ctx* ctx, const MergePlan& p, float threshold, bool resume, FastArgs& A) {
+    const bool big = p.kind == kMergeL2;
+    A.R = ctx->R1; A.E = ctx->E1; A.n_edges_ptr = SC(n_edges); A.n_sv_ptr = SC(xctl.n_sv); A.ep = edge_params(ctx); A.lambda_dev = SC(lambda);
+    A.threshold = threshold; A.run_start = ctx->run_start.as<unsigned>(); A.run_end = ctx->run_end.as<unsigned>();
+    A.pos_data = ctx->pos_data; A.sv_label = ctx->sv_label.as<unsigned>(); A.mlog = ctx->ML; A.log_cap = std::max(1u, ctx->S);
+    A.ctl = SC(mctl); A.S_cap = p.S_cap; A.E_cap = p.E_cap; A.resume = resume ? 1 : 0;
+    A.big = nullptr; A.big_cursor = nullptr;
+    if (big) {
+        const size_t bb = (FastSmem::big_bytes(p.S_cap, p.E_cap) + 255) & ~(size_t)255;
+        F3PS_CUDA_OK(ctx->lean_big.ensure(bb + lean_cursor_bytes(p.S_cap) + LeanWideScratch::bytes));
+        A.big = (char*)ctx->lean_big.p; A.big_cursor = (unsigned*)((char*)ctx->lean_big.p + bb);
     }
-    rc = mark(ctx, 8); if (rc) return rc;
-    rc = pull_scalars(ctx); if (rc) return rc;
+    const size_t entries = 2 * (size_t)ctx->E + (big ? 8 : 1) * kLeanPoolSlack;     // (edge ids: 2 bytes, L2 variant 4)
+    F3PS_CUDA_OK(ctx->adj_pool.ensure(entries * (big ? 4 : 2)));
+    A.adj_pool = ctx->adj_pool.as<unsigned short>(); A.pool_cap = (unsigned)entries;
+    A.trace = nullptr; A.trace_first = ctx->merge_trace_first;
+    if (p.prof && !big) {
+        F3PS_CUDA_OK(ctx->merge_trace.ensure(256 * 32 * 4));
+        F3PS_CUDA_OK(cudaMemsetAsync(ctx->merge_trace.p, 0, 256 * 32 * 4, ctx->stream));
+        A.trace = ctx->merge_trace.as<unsigned>();
+    }
+    return F3PS_OK;
+}
+int launch_resident(f3ps_ctx* ctx, const MergePlan& p, float threshold, bool resume) {
+    FastArgs A;
+    int rc = fast_args(ctx, p, threshold, resume, A); if (rc) return rc;
+    void (*kern)(FastArgs) = p.kind == kMergeL2 ? (p.prof ? merge_fast_big_kernel<true> : merge_fast_big_kernel<false>)
+                           : p.threads == kFastThreadsSolo ? (p.prof ? merge_fast_kernel<true, kFastThreadsSolo> : merge_fast_kernel<false, kFastThreadsSolo>)
+                           : (p.prof ? merge_fast_kernel<true, kFastThreads> : merge_fast_kernel<false, kFastThreads>);
+    rc = smem_opt_in(ctx, (const void*)kern, kSmemMax); if (rc) return rc;
+    LAUNCH(ctx, kern, 1, p.threads, p.smem, A);
+    return F3PS_OK;
+}
+// the general kernel (any graph) from the initial state; PK = one packed incidence word per edge (16 + 16 or 32 + 32 bits)
+template <typename PK>
+int launch_general(f3ps_ctx* ctx, float threshold) {
+    const size_t Sc = std::max(1u, ctx->S), Ec = std::max(1u, ctx->E);
+    const size_t per = (Ec * 4 + 255) & ~(size_t)255, per8 = (Ec * 8 + 255) & ~(size_t)255;
+    unsigned n2 = 2048; while (n2 < Ec) n2 <<= 1;
+    const size_t perS = (Sc * 4 + 255) & ~(size_t)255, sortb = (size_t)n2 * sizeof(MergeSortRec);
+    F3PS_CUDA_OK(ctx->merge_scratch.ensure(6 * per + 2 * per8 + per + per8 + perS + sortb));
+    char* sp = (char*)ctx->merge_scratch.p;
+    MergeScratch scr;
+    scr.st[0] = (long long*)sp; sp += per8; scr.st[1] = (long long*)sp; sp += per8;
+    scr.sortbuf = (MergeSortRec*)sp; sp += sortb;
+    scr.e[0] = (int*)sp; sp += per; scr.e[1] = (int*)sp; sp += per; scr.w[0] = (float*)sp; sp += per; scr.w[1] = (float*)sp; sp += per;
+    scr.x[0] = (unsigned*)sp; sp += per; scr.x[1] = (unsigned*)sp; sp += per; scr.cls = (unsigned char*)sp; sp += per;
+    scr.mark = (unsigned*)sp; sp += perS;
+    const size_t dyn = (size_t)kMergeSortSmem * sizeof(MergeSortRec);
+    int rc = smem_opt_in(ctx, (const void*)merge_kernel<PK>, dyn); if (rc) return rc;
+    LAUNCH(ctx, merge_kernel<PK>, 1, kMergeThreads, dyn, ctx->R1, ctx->E1, SC(n_edges), SC(xctl.n_sv), edge_params(ctx), SC(lambda), threshold,
+           ctx->run_start.as<unsigned>(), ctx->run_end.as<unsigned>(), ctx->order, ctx->gxyz, ctx->sv_label.as<unsigned>(), ctx->ML, (unsigned)Sc,
+           SC(mctl), scr, (PK*)sp, ctx->pos_data);
+    return F3PS_OK;
+}
+// Clustering::get_labeled_cloud: dense segment ids, then the labelled voxel cloud
+int merge_labels(f3ps_ctx* ctx) {
+    int rc = mark(ctx, 10); if (rc) return rc;
+    const unsigned P = ctx->n_pos;
+    LAUNCH(ctx, dense_label_kernel, 1, 1024, 0, ctx->R1, SC(xctl.n_sv), ctx->run_start.as<unsigned>(), ctx->run_end.as<unsigned>(), ctx->run_out_off.as<unsigned>(),
+           ctx->run_dense.as<unsigned>(), ctx->region_dense.as<unsigned>(), SC(n_out));
+    if (P) LAUNCH(ctx, labeled_cloud_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), P, ctx->order, ctx->run_start.as<unsigned>(),
+                  ctx->run_out_off.as<unsigned>(), ctx->run_dense.as<unsigned>(), ctx->gxyz, ctx->out_xyz.as<float>(), ctx->out_label.as<unsigned>(),
+                  ctx->out_voxel.as<unsigned>(), ctx->vox_segment.as<unsigned>(), ctx->graph_from_host ? nullptr : ctx->sorted_label,
+                  ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>());
+    return F3PS_OK;
+}
+// after the replay's scalars reached the host
+int merge_done(f3ps_ctx* ctx) {
     if (ctx->h_sc->mctl.error) return ctx_fail(ctx, F3PS_ERR_CAPACITY, "merge kernel reported an internal capacity error");
     ctx->n_out = ctx->h_sc->n_out;
     ctx->progress = P_MERGED;
     return F3PS_OK;
 }
 
+// kStartContinue: a batch grid stopped this frame in front of a merge with more adjacency entries than worker threads (the
+// working state and the counters are those after n merges).  kStartGeneral: the batch grid ran out of adjacency pool or stamps.
+enum MergeStart { kStartFresh, kStartContinue, kStartGeneral };
+int merge_one(f3ps_ctx* ctx, float threshold, MergeStart start) {
+    int rc = merge_begin(ctx, start != kStartContinue); if (rc) return rc;
+    if (ctx->S) {
+        MergePlan p = plan_merge(ctx);
+        if (start == kStartGeneral) p.kind = kMergeGeneral;
+        ctx->merge_path = p.kind;
+        rc = mark(ctx, 9); if (rc) return rc;
+        if (p.kind != kMergeGeneral) {
+            unsigned err = kFastErrTouched;
+            if (start == kStartFresh) {
+                rc = launch_resident(ctx, p, threshold, false); if (rc) return rc;
+                rc = pull_scalars(ctx); if (rc) return rc;   // did the resident kernel finish?
+                err = ctx->h_sc->mctl.error;
+            }
+            // The shared-memory variant stops IN FRONT of a merge whose two adjacency lists hold more entries than it has worker
+            // threads (nothing of that merge has happened): the L2 variant continues from that state.
+            if (err == kFastErrTouched && p.to_l2) {
+                F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl.error), 0, 4, ctx->stream));
+                p = plan_l2(ctx);
+                ctx->merge_path = 6;
+                rc = launch_resident(ctx, p, threshold, true); if (rc) return rc;
+                rc = pull_scalars(ctx); if (rc) return rc;
+                err = ctx->h_sc->mctl.error;
+            }
+            // Any other stop (adjacency pool or stamp range exhausted, a merge with more than 65,534 entries on the L2 variant): the
+            // general kernel replays the whole sequence from the initial state.
+            if (err) {
+                rc = merge_restart(ctx); if (rc) return rc;
+                p.kind = kMergeGeneral;
+                ctx->merge_path = kMergeGeneral;
+            }
+        }
+        if (p.kind == kMergeGeneral) {
+            rc = ctx->S < 65536u ? launch_general<unsigned>(ctx, threshold) : launch_general<unsigned long long>(ctx, threshold);
+            if (rc) return rc;
+        }
+        rc = merge_labels(ctx); if (rc) return rc;
+    }
+    rc = mark(ctx, 8); if (rc) return rc;
+    rc = pull_scalars(ctx); if (rc) return rc;
+    return merge_done(ctx);
+}
+}
+}
+int f3ps_merge(f3ps_ctx* ctx, float threshold) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    if (ctx->progress < P_EXPANDED)                            // std::logic_error of Clustering::cluster (src/clustering.cpp:671-673)
+        return ctx_fail(ctx, F3PS_ERR_LOGIC, "Cannot call 'cluster' before setting an initial state with 'set_initialstate'");
+    cudaSetDevice(ctx->device);
+    if (ctx->progress < P_GRAPH) { int rc = f3ps_graph(ctx); if (rc) return rc; }   // if (!init_initial_weights) init_weights()  (:675-676)
+    return merge_one(ctx, threshold, kStartFresh);
+}
+
 // Clustering::cluster(threshold) for MANY frames with ONE launch of the resident merge kernel: CTA i of the grid replays frame i.
 // A sweep that keeps frames in flight on independent streams is capped by the 32 hardware queues of a context (at most 32
 // single-CTA merge kernels overlap); one grid of n CTAs runs n frames side by side.  Every handle must be on the same device,
-// with its graph built (f3ps_graph); handles whose graph does not fit the resident kernel run f3ps_merge on their own.
+// with its graph built (f3ps_graph); handles whose plan is not the shared-memory kernel without phase counters run on their own.
 // Results per handle are exactly those of f3ps_merge(handle, threshold).
 int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
     if (!ctxs || n < 1) return F3PS_ERR_INVALID_ARGUMENT;
@@ -953,54 +973,24 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
     cudaSetDevice(ctxs[0]->device);
     int rc;
     std::vector<int> batch, solo;
-    std::vector<int> slots_of(n, 0);                         // per handle: edge capacity of its tables
+    std::vector<MergePlan> plans(n);
     for (int i = 0; i < n; ++i) {
         f3ps_ctx* ctx = ctxs[i];
         if (ctx->progress < P_GRAPH) { rc = f3ps_graph(ctx); if (rc) return rc; }
-        const unsigned S = ctx->S, E = ctx->E, P = ctx->n_pos;
-        const unsigned ecap = lean_ecap_for(E);
-        const bool ok = S > 0 && ecap && S <= 4096u && P > 0 && !ctx->force_general_merge;
-        slots_of[i] = (int)ecap;
-        (ok ? batch : solo).push_back(i);
-    }
-    {   // every frame brings its own table capacities (the layout is per CTA); the launch asks for the largest footprint
-        std::vector<int> keep;
-        for (int i : batch) {
-            const unsigned S_cap = (ctxs[i]->S + 7u) & ~7u;
-            if (FastSmem(nullptr, S_cap, (unsigned)slots_of[i]).bytes <= 227u * 1024u) keep.push_back(i); else solo.push_back(i);
-        }
-        batch.swap(keep);
+        plans[i] = plan_merge(ctx);
+        (ctx->S > 0 && plans[i].kind == kMergeShared && !plans[i].prof ? batch : solo).push_back(i);
     }
     for (size_t g0 = 0; g0 < batch.size(); g0 += kFastBatchMax) {
         const size_t g1 = std::min(batch.size(), g0 + (size_t)kFastBatchMax);
         static thread_local FastBatch B;                     // 32 KB: not on the stack
-        size_t bytes = 0;
+        size_t bytes = 0;                                    // every frame brings its own table capacities (the layout is per CTA)
         f3ps_ctx* lead = ctxs[batch[g0]];
         for (size_t k = g0; k < g1; ++k) {
             f3ps_ctx* ctx = ctxs[batch[k]];
-            rc = mark(ctx, 7); if (rc) return rc;
-            const unsigned S = ctx->S, P = ctx->n_pos; const size_t Sc = std::max(1u, S), Pc = std::max(1u, P);
-            F3PS_CUDA_OK(cudaMemcpyAsync(ctx->reg_work.p, ctx->reg_init.p, region_bytes(Sc), cudaMemcpyDeviceToDevice, ctx->stream));   // cluster(float) restarts (:678)
-            const size_t eb = std::min(ctx->edge_init.cap, ctx->edge_work.cap);
-            F3PS_CUDA_OK(cudaMemcpyAsync(ctx->edge_work.p, ctx->edge_init.p, eb, cudaMemcpyDeviceToDevice, ctx->stream));
-            F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl), 0, sizeof(MergeCtl), ctx->stream));
-            F3PS_CUDA_OK(ctx->mlog.ensure(Sc * 20));
-            char* lp = (char*)ctx->mlog.p;
-            ctx->ML.a = (unsigned*)lp; ctx->ML.b = (unsigned*)(lp + Sc * 4); ctx->ML.w = (float*)(lp + Sc * 8);
-            ctx->ML.edges_left = (unsigned*)(lp + Sc * 12); ctx->ML.regions_left = (unsigned*)(lp + Sc * 16);
-            F3PS_CUDA_OK(ctx->run_out_off.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->run_dense.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->region_dense.ensure(Sc * 4));
-            F3PS_CUDA_OK(ctx->out_xyz.ensure(Pc * 12)); F3PS_CUDA_OK(ctx->out_label.ensure(Pc * 4)); F3PS_CUDA_OK(ctx->out_voxel.ensure(Pc * 4));
-            F3PS_CUDA_OK(ctx->vox_segment.ensure(Pc * 4));
-            F3PS_CUDA_OK(cudaMemsetAsync(ctx->vox_segment.p, 0xff, Pc * 4, ctx->stream));
-            F3PS_CUDA_OK(cudaMemsetAsync(SC(n_out), 0, 4, ctx->stream));
-            FastArgs& A = B.a[k - g0];
-            A.R = ctx->R1; A.E = ctx->E1; A.n_edges_ptr = SC(n_edges); A.n_sv_ptr = SC(xctl.n_sv); A.ep = edge_params(ctx); A.lambda_dev = SC(lambda);
-            A.threshold = threshold; A.run_start = ctx->run_start.as<unsigned>(); A.run_end = ctx->run_end.as<unsigned>();
-            A.pos_data = ctx->pos_data; A.sv_label = ctx->sv_label.as<unsigned>(); A.mlog = ctx->ML; A.log_cap = (unsigned)Sc;
-            A.ctl = SC(mctl); A.S_cap = (S + 7u) & ~7u; A.E_cap = (unsigned)slots_of[batch[k]];
-            rc = lean_pool(ctx, ctx->E, A); if (rc) return rc;
-            A.trace = nullptr; A.trace_first = 0; A.big = nullptr; A.big_cursor = nullptr; A.resume = 0;
-            bytes = std::max(bytes, FastSmem(nullptr, A.S_cap, A.E_cap).bytes);
+            const MergePlan& p = plans[batch[k]];
+            rc = merge_begin(ctx, true); if (rc) return rc;
+            rc = fast_args(ctx, p, threshold, false, B.a[k - g0]); if (rc) return rc;
+            bytes = std::max(bytes, p.smem);
             rc = mark(ctx, 9); if (rc) return rc;
             if (ctx->stream != lead->stream) {               // the lead's stream runs the grid: it waits for everybody's set-up
                 F3PS_CUDA_OK(cudaEventRecord(ctx->ev_batch, ctx->stream));
@@ -1009,51 +999,28 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
         }
         {
             f3ps_ctx* ctx = lead;
-            void (*kern)(const FastBatch) = merge_fast_batch_kernel;
-            rc = lean_attr(ctx, (const void*)kern); if (rc) return rc;
-            kern<<<(unsigned)(g1 - g0), kFastThreads, bytes, ctx->stream>>>(B);
-            ctx->launches++;
-            F3PS_CUDA_OK(cudaPeekAtLastError());
+            rc = smem_opt_in(ctx, (const void*)merge_fast_batch_kernel, kSmemMax); if (rc) return rc;
+            LAUNCH(ctx, merge_fast_batch_kernel, (unsigned)(g1 - g0), kFastThreads, bytes, B);
             F3PS_CUDA_OK(cudaEventRecord(ctx->ev_batch, ctx->stream));
         }
         for (size_t k = g0; k < g1; ++k) {                   // every handle continues on its own stream after the grid
             f3ps_ctx* ctx = ctxs[batch[k]];
             if (ctx->stream != lead->stream) F3PS_CUDA_OK(cudaStreamWaitEvent(ctx->stream, lead->ev_batch, 0));
-            ctx->merge_path = 1;
-            rc = mark(ctx, 10); if (rc) return rc;
-            const unsigned P = ctx->n_pos;
-            LAUNCH(ctx, dense_label_kernel, 1, 1024, 0, ctx->R1, SC(xctl.n_sv), ctx->run_start.as<unsigned>(), ctx->run_end.as<unsigned>(), ctx->run_out_off.as<unsigned>(),
-                   ctx->run_dense.as<unsigned>(), ctx->region_dense.as<unsigned>(), SC(n_out));
-            if (P) LAUNCH(ctx, labeled_cloud_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), P, ctx->order, ctx->run_start.as<unsigned>(),
-                          ctx->run_out_off.as<unsigned>(), ctx->run_dense.as<unsigned>(), ctx->gxyz, ctx->out_xyz.as<float>(), ctx->out_label.as<unsigned>(),
-                          ctx->out_voxel.as<unsigned>(), ctx->vox_segment.as<unsigned>(), ctx->graph_from_host ? nullptr : ctx->sorted_label,
-                          ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>());
+            ctx->merge_path = kMergeShared;
+            rc = merge_labels(ctx); if (rc) return rc;
             rc = mark(ctx, 8); if (rc) return rc;
         }
     }
-    // graphs that do not fit the resident kernel: one by one (general kernel), next to the grids already in flight
-    for (int i : solo) { rc = f3ps_merge(ctxs[i], threshold); if (rc) return rc; }
-    // results only after EVERY chunk's grid is in flight (a batch larger than one parameter block must not run its chunks back to back)
-    {
-        for (size_t k = 0; k < batch.size(); ++k) {
-            f3ps_ctx* ctx = ctxs[batch[k]];
-            rc = pull_scalars(ctx); if (rc) return rc;
-            if (ctx->h_sc->mctl.error == kFastErrTouched) {  // the frame's CTA stopped in front of a merge with more adjacency entries than worker
-                ctx->merge_take_over = true;                 // threads: this frame alone continues from that state (general kernel for that merge, then resident again)
-                rc = f3ps_merge(ctx, threshold); if (rc) return rc;
-                continue;
-            }
-            if (ctx->h_sc->mctl.error) {                     // adjacency pool / stamp range exhausted: this frame alone, general kernel, from the start
-                const bool was = ctx->force_general_merge;
-                ctx->force_general_merge = true;
-                rc = f3ps_merge(ctx, threshold);
-                ctx->force_general_merge = was;
-                if (rc) return rc;
-                continue;
-            }
-            ctx->n_out = ctx->h_sc->n_out;
-            ctx->progress = P_MERGED;
-        }
+    // the other handles one by one, next to the grids already in flight
+    for (int i : solo) { rc = merge_one(ctxs[i], threshold, kStartFresh); if (rc) return rc; }
+    // results only after EVERY chunk's grid is in flight (a batch larger than one parameter block must not run its chunks back to back);
+    // a frame whose CTA stopped continues alone
+    for (int i : batch) {
+        f3ps_ctx* ctx = ctxs[i];
+        rc = pull_scalars(ctx); if (rc) return rc;
+        const unsigned err = ctx->h_sc->mctl.error;
+        rc = err ? merge_one(ctx, threshold, err == kFastErrTouched ? kStartContinue : kStartGeneral) : merge_done(ctx);
+        if (rc) return rc;
     }
     return F3PS_OK;
 }
@@ -1089,8 +1056,7 @@ int f3ps_set_blocking_wait(f3ps_ctx* ctx, int blocking) {
 }
 
 int f3ps_set_merge_kernel(f3ps_ctx* ctx, int which) {
-    if (!ctx || which < 0 || which > 5) return F3PS_ERR_INVALID_ARGUMENT;
-    ctx->force_general_merge = which == 2;
+    if (!ctx || which < 0 || which > 5 || which == 1) return F3PS_ERR_INVALID_ARGUMENT;
     ctx->merge_kernel_choice = which;
     return F3PS_OK;
 }

@@ -160,7 +160,7 @@ __global__ void __launch_bounds__(kMergeThreads, 1) merge_kernel(RegionArrays R,
         const unsigned* __restrict__ n_sv_ptr, EdgeParams ep, const float* __restrict__ lambda_dev, float threshold,
         const unsigned* __restrict__ run_start, const unsigned* __restrict__ run_end, const unsigned* __restrict__ order,
         const float4* __restrict__ vox_xyz, const unsigned* __restrict__ sv_label, MergeLog mlog, unsigned log_cap, MergeCtl* ctl, MergeScratch scr,
-        PK* __restrict__ pk, const float4* __restrict__ pos_data, int resume, unsigned stop_after) {   // resume: continue a replay the resident kernel handed over (ctl holds its counters); stop_after > 0: hand back after that many merges
+        PK* __restrict__ pk, const float4* __restrict__ pos_data) {
     typedef PkOps<PK> P;
     extern __shared__ __align__(16) unsigned char dyn_smem[];     // kMergeSortSmem sort records
     __shared__ float s_rw[32]; __shared__ long long s_rs[32]; __shared__ int s_ri[32];
@@ -182,14 +182,7 @@ __global__ void __launch_bounds__(kMergeThreads, 1) merge_kernel(RegionArrays R,
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const unsigned nE = *n_edges_ptr;
     if (lambda_dev) ep.lambda = *lambda_dev;
-    if (tid == 0) {
-        s_nm = 0; s_ealive = nE; s_ralive = *n_sv_ptr; s_counter = (long long)nE; s_fold = 0; s_maxT = 0;
-        if (resume) {       // state arrays (regions, edges, stamps, ropes, log prefix) are those after ctl->n_merges merges
-            s_nm = ctl->n_merges; s_ealive = ctl->edges_alive; s_ralive = ctl->regions_alive;
-            s_counter = ctl->counter > (long long)nE ? ctl->counter : (long long)nE; s_fold = ctl->fold_steps; s_maxT = ctl->max_touched;
-        }
-    }
-    const unsigned nm0 = resume ? ctl->n_merges : 0u;
+    if (tid == 0) { s_nm = 0; s_ealive = nE; s_ralive = *n_sv_ptr; s_counter = (long long)nE; s_fold = 0; s_maxT = 0; }
     const float INF = __int_as_float(0x7f800000);
     enum { C_KEEP = 0, C_FRONT = 1, C_BACK = 2, C_DUP = 3 };
     // strip of this thread and its cached minimum
@@ -246,7 +239,6 @@ __global__ void __launch_bounds__(kMergeThreads, 1) merge_kernel(RegionArrays R,
         const int head = s_head;
         PHASE(0);
         if (head < 0 || !(s_head_w < threshold)) break;          // strict <, src/clustering.cpp:388-389
-        if (stop_after && s_nm - nm0 >= stop_after) break;        // (s_nm is stable here: written before the barriers above)
         const unsigned a = E.a[head], b = E.b[head];
         __syncthreads();
         if (tid == 0) {

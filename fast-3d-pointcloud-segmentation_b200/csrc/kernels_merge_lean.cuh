@@ -24,10 +24,10 @@
 // BIG -- the per-edge / per-region tables in global memory with per-block minima in shared memory (S < 65535, 32-bit edge ids,
 // E bounded by 16 bytes of shared memory per block of 32 edges: C4 / C5-size scenes).  Shared-memory variant: a merge whose two
 // adjacency lists hold more than 928 entries is not started: every role stops in front of it, the state written back is that
-// after n merges, and the host lets merge_kernel (kernels_merge.cuh) replay that one merge from the same state and relaunches
-// this kernel with A.resume (f3ps.cu: f3ps_merge).  BIG variant: such a merge runs in lean_wide_merge (every worker thread loops
-// over the entries, per-entry state in a global scratch); only beyond 65,534 entries does it hand over.  An exhausted adjacency
-// pool or stamp range restarts the replay on merge_kernel.
+// after n merges, and the host relaunches the BIG variant from that state with A.resume (f3ps.cu: merge_one).  BIG variant:
+// such a merge runs in lean_wide_merge (every worker thread loops over the entries, per-entry state in a global scratch); it
+// stops only in front of a merge with more than 65,534 entries.  That stop, an exhausted adjacency pool or an exhausted stamp
+// range makes the host replay the whole sequence again on merge_kernel (kernels_merge.cuh), from the initial state.
 #pragma once
 #include "kernels_merge.cuh"
 
@@ -80,7 +80,7 @@ struct FastArgs {
     MergeCtl* ctl;
     unsigned short* adj_pool; unsigned pool_cap;   // adjacency lists (edge ids: 16 bits, BIG variant 32 bits), bump-allocated; capacity in entries
     unsigned* trace; unsigned trace_first;         // PROF only: clock() of 32 points of 256 merges starting at trace_first (f3ps_get_merge_trace)
-    int resume;                              // continue a replay from the state in the edge / region arrays (counters in *ctl): set after the general kernel took one merge this kernel could not
+    int resume;                              // continue a replay from the state in the edge / region arrays (counters in *ctl): the BIG variant after the shared-memory one stopped
     char* big; unsigned* big_cursor;         // BIG variant only: the per-edge / per-region tables (12 E_cap + 26 S_cap bytes) and the set-up scratch (4 S_cap) in global memory; LeanWideScratch sits at big_cursor + lean_cursor_bytes(S_cap)
     unsigned S_cap, E_cap;                   // table capacities the shared-memory layout was sized for (E_cap = E rounded up to whole blocks of 32 edges)
 };

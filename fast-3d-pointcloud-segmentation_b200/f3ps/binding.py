@@ -265,7 +265,7 @@ class Segmenter:
         a = (C.c_uint64 * 32)()
         self._chk(self.L.f3ps_merge_profile(self.h, C.byref(a)))
         v = list(a)
-        if self.counts().merge_path in (1, 3):  # resident kernel; cycle counters only after set_merge_kernel(4) / (5)
+        if self.counts().merge_path in (1, 3, 6):  # resident kernel; cycle counters only after set_merge_kernel(4) / (5)
             return {"worker": dict(zip(["scan_publish", "wait_s1_head", "incidence_w1", "dedupe_spec_ciede", "wait_fold", "weights_stamps", "wait_w4"], v[0:7])),
                     "mean": dict(zip(["wait_voxels", "fold", "lab_publish", "wait_s1"], v[12:16])),
                     "cov": dict(zip(["wait_voxels", "fold", "eigen_publish", "wait_s1"], v[16:20])),

@@ -71,7 +71,7 @@ typedef struct f3ps_counts {
     int32_t max_touched;   /* largest number of edges re-weighted by one merge */
     int64_t fold_steps;    /* voxel steps folded by the merge loop (sum of |b|) */
     int32_t nan_weights;   /* edge weights that evaluated to NaN (regions with < 3 voxels) */
-    int32_t merge_path;    /* kernel the last f3ps_merge ran: 1 = resident (one SM, weight map in shared memory), 2 = general, 3 = resident with its tables in L2 (graphs too large for an SM), 4 / 5 = 1 / 3 with the general kernel taking the merges whose adjacency lists hold more entries than the kernel handles (1: 928, 3: 65,534) (and, after 16 such hand-overs, the rest); 6 = 1 up to the first merge with more than 928 adjacency entries, then 3 from that state */
+    int32_t merge_path;    /* kernel the last f3ps_merge ran: 1 = resident (one SM, weight map in shared memory), 2 = general (also: a resident replay that could not go on, replayed again from the start), 3 = resident with its tables in L2 (graphs too large for an SM), 6 = 1 up to the first merge with more than 928 adjacency entries, then 3 from that state */
 } f3ps_counts;
 
 /* ---- life cycle ------------------------------------------------------------ */
@@ -129,18 +129,21 @@ int f3ps_set_expand_kernel(f3ps_ctx* ctx, int which, int cluster_ctas);
 /* Clustering::cluster(threshold) for n handles (same device, graphs built) with ONE launch of the resident merge kernel:
  * CTA i replays frame i.  Independent streams share at most 32 hardware queues per context, so a sweep with one merge
  * kernel per stream never overlaps more than 32 of them; a grid has no such limit.  Same results per handle as f3ps_merge;
- * handles whose graph does not fit the resident kernel are clustered by f3ps_merge individually. */
+ * handles whose graph does not fit the resident kernel's shared memory, or whose kernel choice is not 0, are clustered
+ * individually, as f3ps_merge would. */
 int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold);
 /* How the host waits where it needs a size from the device: 0 = spin (lowest latency, the default), 1 = sleep on a
  * blocking event.  Sweeps that keep more frames in flight than there are host cores must use 1. */
 int f3ps_set_blocking_wait(f3ps_ctx* ctx, int blocking);
-/* which K7 kernel f3ps_merge uses: 0 = automatic (the resident kernel when the graph fits one SM's shared memory; the same kernel
- * with its per-edge / per-region tables in L2 when it does not but S < 65,535 and E < ~380,000 (16 bytes of shared memory per
- * 32 edges); else the general kernel -- which also takes over when a merge of the shared-memory kernel has more than 928
- * adjacency entries, or one of the L2 variant more than 65,534), 1 = resident in shared memory or general, 2 = always general,
- * 3 = resident with the tables in L2 even when the graph would fit an SM, 4 / 5 = 1 / 3 compiled with per-phase cycle counters
- * (4: and the merge trace; f3ps_merge_profile, f3ps_merge_trace).  All replay the same merge sequence; the switch exists for
- * tests and profiling. */
+/* which K7 kernel f3ps_merge and f3ps_merge_batch use: 0 = automatic (the resident kernel when the graph fits one SM's shared
+ * memory, continued on its L2 variant from the first merge with more than 928 adjacency entries; the L2 variant, with its
+ * per-edge / per-region tables in L2, when the graph does not fit but S < 65,535 and E < ~380,000 (16 bytes of shared memory
+ * per 32 edges); else the general kernel -- which also replays the whole sequence again when a resident kernel cannot go on:
+ * its adjacency pool or stamp range is exhausted, or a merge of the L2 variant has more than 65,534 adjacency entries),
+ * 2 = always general, 3 = the L2 variant even when the graph would fit an SM, 4 = 0 with the shared-memory kernel compiled
+ * with per-phase cycle counters and the merge trace, 5 = 3 with per-phase cycle counters (f3ps_merge_profile,
+ * f3ps_merge_trace); other values, 1 included, are F3PS_ERR_INVALID_ARGUMENT.  Only 0 lets f3ps_merge_batch put a handle into
+ * its grid.  All replay the same merge sequence; the switch exists for tests and profiling. */
 int f3ps_set_merge_kernel(f3ps_ctx* ctx, int which);
 /* Development aid of the resident kernel (kernel choice 4): SM clock values at 32 points of each of 256 consecutive merges,
  * starting at merge `first_merge` of the NEXT f3ps_merge; out (may be NULL to only set the window) receives the last

@@ -293,6 +293,8 @@ def test_resident_and_general_merge_kernels_agree(gpu, vga_frame, small_frame, m
                 assert same(fast[n], g.array(n)), (which, n)
             if which == 4:
                 assert g.merge_profile()["sum_T"] > 0 or g.counts().n_merges < 2
+        with pytest.raises(ValueError):                   # 1 is not a kernel choice
+            g.set_merge_kernel(1)
 
 
 def test_frames_in_flight_pool(gpu, oracle_mod, small_frame):
@@ -458,11 +460,10 @@ def test_full_size_properties_config4(gpu):
     assert len(out) == int((labels > 0).sum()) and out.max() + 1 == g.counts().n_segments
 
 
-@pytest.mark.parametrize("n_leaves,mode", [(1500, "lab_al"), (3000, "rgb_eq"), (9000, "rgb_ml")])
-def test_general_merge_kernel_hub_graph(gpu, oracle_mod, n_leaves, mode):
-    """Merges that touch thousands of edges (a region with thousands of neighbours, as floors and walls of dense scenes
-    have): the general kernel's sorted path (bitonic sort in shared / global memory, mark-based dedupe, ballot-scan tie
-    stamps) must replay the oracle's sequence exactly.  Hub + ring graph injected through set_graph."""
+def hub_graph(n_leaves, twins=False):
+    """Hub + ring graph for set_graph: hub 0 touches every leaf, hub 1 every other leaf, leaf i touches leaf i + 1.
+    twins: hub 1 touches every leaf too, and the hubs share colour and normal with a centroid offset perpendicular to it
+    (weight 0: the hubs merge first, a merge with 2 (n_leaves + 1) adjacency entries)."""
     rng = np.random.default_rng(n_leaves)
     S = n_leaves + 2
     sizes = rng.integers(3, 7, S)
@@ -477,10 +478,14 @@ def test_general_merge_kernel_hub_graph(gpu, oracle_mod, n_leaves, mode):
     cen = np.stack([vxyz[l].mean(0) for l in lists]).astype(np.float32)
     nrm = rng.normal(0, 1, (S, 3)).astype(np.float32)
     nrm /= np.linalg.norm(nrm, axis=1, keepdims=True)
+    if twins:
+        vrgba[:off[2]] = np.uint32(0xffffff)
+        nrm[:2] = (0, 0, 1)
+        cen[1] = cen[0] + np.float32([0.5, 0, 0])
     pairs = {(0, 1)}
     for i in range(2, S):
         pairs.add((0, i))                             # hub 0 touches everything
-        if i % 2:
+        if i % 2 or twins:
             pairs.add((1, i))                         # hub 1 touches half: duplicates (a,x)/(b,x) when the hubs merge
         if i + 1 < S:
             pairs.add((i, i + 1))
@@ -488,26 +493,38 @@ def test_general_merge_kernel_hub_graph(gpu, oracle_mod, n_leaves, mode):
     for i, j in sorted(pairs):
         adj += [(labels[i], labels[j]), (labels[j], labels[i])]
     adj = np.array(sorted(adj), np.uint32)
+    return vxyz, vrgba, labels, lists, cen, nrm, adj
+
+
+@pytest.mark.parametrize("n_leaves,mode", [(1500, "lab_al"), (3000, "rgb_eq"), (9000, "rgb_ml"), (33000, "rgb_ml")])
+def test_general_merge_kernel_hub_graph(gpu, oracle_mod, n_leaves, mode):
+    """Merges that touch thousands of edges (a region with thousands of neighbours, as floors and walls of dense scenes
+    have): the general kernel's sorted path (bitonic sort in shared / global memory, mark-based dedupe, ballot-scan tie
+    stamps) must replay the oracle's sequence exactly.  Hub + ring graph injected through set_graph.  With twin hubs the first
+    merge has more adjacency entries than the L2 variant handles (65,534): the general kernel replays from the start."""
+    twins = n_leaves >= 32767                         # (the hubs' merge then has more than 65,534 adjacency entries)
+    graph = hub_graph(n_leaves, twins)
+    S = n_leaves + 2
     flags = {"lab_al": dict(color_mode=0, geom_mode=1, merge_mode=1), "rgb_eq": dict(color_mode=1, geom_mode=0, merge_mode=2, bins=7),
              "rgb_ml": dict(color_mode=1, geom_mode=1, merge_mode=0, lam=0.5)}[mode]
-    thr = 0.95 if mode == "rgb_eq" else 0.3
+    thr = 0.08 if twins else 0.95 if mode == "rgb_eq" else 0.3   # (twins: below the hub's merges with leaves, which the oracle replays slowly)
     o = oracle_mod.Oracle(); o.set_merge_params(merge_impl=1, **flags)
-    o.set_graph(vxyz, vrgba, labels, lists, cen, nrm, adj); o.run(7, thr)
+    o.set_graph(*graph); o.run(7, thr)
     g = gpu.Segmenter(); g.set_merge_params(**flags)
-    g.set_graph(vxyz, vrgba, labels, lists, cen, nrm, adj)
+    g.set_graph(*graph)
     g.merge(thr)
     c = g.counts()
-    # (2: general kernel from the start; 4 / 5: the resident kernel up to the first merge that touches more edges than it has worker
-    # threads, then the general kernel continues from its state -- the hand-over is part of what this test pins against the oracle)
-    # -- or 3: the graph does not fit an SM, the resident kernel with its tables in L2 loops over the entries of such merges itself;
-    # 6: the shared-memory kernel up to the first such merge, then the L2 variant from that state)
-    assert c.merge_path in (2, 3, 4, 5, 6) and c.max_touched > 1024 and c.n_merges > 100, (c.merge_path, c.max_touched, c.n_merges)
+    # 6: the shared-memory kernel up to the first merge with more adjacency entries than it has worker threads, then the L2 variant
+    # from that state; 3: the graph does not fit an SM, the L2 variant loops over the entries of such merges itself; 2: a merge with
+    # more than 65,534 entries stops the L2 variant too, and the general kernel replays the whole sequence
+    path = 2 if twins else 6 if S <= 4096 else 3
+    assert c.merge_path == path and c.max_touched > 1024 and c.n_merges > 100, (c.merge_path, c.max_touched, c.n_merges)
     first = (c.merge_path, g.array("merges_ab").copy(), g.array("final_ab").copy(), g.array("final_w").copy(), g.array("merges_w").copy())
     g.set_merge_kernel(2); g.merge(thr)                  # the general kernel alone replays the same sequence
     assert g.counts().merge_path == 2 and np.array_equal(g.array("merges_ab"), first[1]) and np.array_equal(g.array("final_ab"), first[2])
-    g.set_merge_kernel(3); g.merge(thr)                  # tables in L2: merges with more than 928 adjacency entries run in lean_wide_merge, no hand-over
+    g.set_merge_kernel(3); g.merge(thr)                  # tables in L2: merges with more than 928 adjacency entries run in lean_wide_merge
     c3 = g.counts()
-    assert c3.merge_path == 3 and c3.max_touched > 1024 and c3.n_merges == c.n_merges, (c3.merge_path, c3.max_touched, c3.n_merges)
+    assert c3.merge_path == (2 if twins else 3) and c3.max_touched > 1024 and c3.n_merges == c.n_merges, (c3.merge_path, c3.max_touched, c3.n_merges)
     assert np.array_equal(g.array("merges_ab"), first[1]) and np.array_equal(g.array("final_ab"), first[2])
     assert same(g.array("final_w"), first[3]) and same(g.array("merges_w"), first[4])
     g.set_merge_kernel(0); g.merge(thr)
@@ -527,8 +544,8 @@ def test_general_merge_kernel_hub_graph(gpu, oracle_mod, n_leaves, mode):
 
 def test_merge_batch_equals_individual_merges(gpu):
     """f3ps_merge_batch: ONE launch of the resident merge kernel, CTA i = frame i, gives every handle exactly what
-    f3ps_merge gives it alone -- mixed sizes (different slot counts), a handle forced onto the general kernel, a handle
-    whose largest merge overflows the resident kernel's touched list, and the pipelined BatchPool."""
+    f3ps_merge gives it alone -- mixed sizes (different slot counts), handles forced onto the general kernel and onto the
+    L2 variant, a handle whose largest merge overflows the resident kernel's touched list, and the pipelined BatchPool."""
     from f3ps import synth, sweep
     frames = [synth.make_frame(seed=500 + i, width=160, height=120) for i in range(9)] + [synth.make_frame(seed=20021)]
     solo = []
@@ -539,8 +556,8 @@ def test_merge_batch_equals_individual_merges(gpu):
     segs = []
     for k, f in enumerate(frames):
         g = gpu.Segmenter(); g.set_vccs_params(); g.set_merge_params(**AL)
-        if k == 3:
-            g.set_merge_kernel(2)                         # this one must take the individual path
+        if k in (3, 4):
+            g.set_merge_kernel(k - 1)                     # general kernel / L2 variant: these take the individual path
         g.set_input(f); g.extract(); g.graph()
         segs.append(g)
     for rep in range(2):                                   # twice: cluster() restarts from the initial state
@@ -548,7 +565,7 @@ def test_merge_batch_equals_individual_merges(gpu):
         for k, g in enumerate(segs):
             for n, want in solo[k].items():
                 assert np.array_equal(g.array(n), want), (rep, k, n)
-            assert g.counts().merge_path == (2 if k == 3 else 1)
+            assert g.counts().merge_path == {3: 2, 4: 3}.get(k, 1)
     gpu.merge_batch(segs[:5], 0.1)                         # a lower threshold: a prefix
     for k, g in enumerate(segs[:5]):
         m = g.counts().n_merges
