@@ -128,7 +128,15 @@ struct f3ps_ctx {
     bool slab_frame = false; f3ps::FrameParams slab_fp{};
     bool slab_range = false; unsigned own_begin = 0, own_end = 0;
     f3ps::DevBuf slab_dest, slab_tot;
-    f3ps::DevBuf ev_parent, ev_when, ev_dense, ev_truth, ev_table;   // f3ps_eval_thresholds
+    f3ps::DevBuf ev_dense, ev_truth, ev_table;   // f3ps_eval_thresholds, f3ps_eval_label_pairs
+    // segmentation levels (f3ps_merge_levels; every merge records its own threshold as the one level).  The tables are built on
+    // the first getter call after the merge: forest, per-level merge counts and per-supervoxel labels, then the voxel table.
+    std::vector<float> lv_thr;          // thresholds of the recorded levels; empty: no merged state to read levels from
+    unsigned lv_M = 0;                  // merges of the replay the levels are prefixes of
+    int lv_built = 0;                   // 0 nothing, 1 level tables of lv_thr, 2 and the voxel table
+    std::vector<int32_t> lv_m_h, lv_nseg_h;
+    f3ps::DevBuf lv_small, lv_parent, lv_when, lv_dense, lv_seg, lv_vox, lv_points;
+    f3ps::DevBuf graph_vox;             // f3ps_set_graph: voxel index as passed in, per position
     f3ps::ExpandArgs slab_A{}; int slab_cur = 0; unsigned slab_k = 0; unsigned slab_sweeps = 0; int slab_round = 0; bool slab_expanding = false;
     int expand_kernel_choice = 0;       // f3ps_set_expand_kernel: 0 auto, 1 cooperative grid, 2 one cluster
     int expand_cluster_ctas = 0;        // cap of the cluster size (0 = by V, at most 16)

@@ -689,7 +689,7 @@ int f3ps_set_graph(f3ps_ctx* ctx, int64_t n_voxels, const float* voxel_xyz, cons
     std::sort(perm.begin(), perm.end(), [&](int x, int y) { return labels[x] < labels[y]; });
     std::map<uint32_t, unsigned> rank;
     std::vector<float4> h_xyz(std::max(1u, V));
-    std::vector<unsigned> h_start(std::max(1u, S)), h_end(std::max(1u, S)), h_label(std::max(1u, S)), h_posrun(std::max(1u, V));
+    std::vector<unsigned> h_start(std::max(1u, S)), h_end(std::max(1u, S)), h_label(std::max(1u, S)), h_posrun(std::max(1u, V)), h_vin(std::max(1u, V));
     std::vector<float4> h_cen(std::max(1u, S)), h_nrm(std::max(1u, S));
     unsigned pos = 0;
     for (unsigned r = 0; r < S; ++r) {
@@ -700,7 +700,7 @@ int f3ps_set_graph(f3ps_ctx* ctx, int64_t n_voxels, const float* voxel_xyz, cons
         for (int64_t i = voxel_offsets[s]; i < voxel_offsets[s + 1]; ++i, ++pos) {
             float w; uint32_t c = voxel_rgba[i] & 0x00ffffffu; memcpy(&w, &c, 4);
             h_xyz[pos] = make_float4(voxel_xyz[3 * i], voxel_xyz[3 * i + 1], voxel_xyz[3 * i + 2], w);
-            h_posrun[pos] = r;
+            h_posrun[pos] = r; h_vin[pos] = (unsigned)i;
         }
         h_end[r] = pos;
         h_cen[r] = make_float4(centroids_xyz[3 * s], centroids_xyz[3 * s + 1], centroids_xyz[3 * s + 2], 0.0f);
@@ -720,6 +720,7 @@ int f3ps_set_graph(f3ps_ctx* ctx, int64_t n_voxels, const float* voxel_xyz, cons
     const unsigned E = (unsigned)h_keys.size();
     const size_t Sc = std::max(1u, S), Vc = std::max(1u, V), Ec = std::max(1u, E);
     F3PS_CUDA_OK(ctx->vox_xyz.ensure(Vc * 16)); F3PS_CUDA_OK(ctx->lab_vals_a.ensure(Vc * 4)); F3PS_CUDA_OK(ctx->pos_run.ensure(Vc * 4));
+    F3PS_CUDA_OK(ctx->graph_vox.ensure(Vc * 4));
     F3PS_CUDA_OK(ctx->run_start.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->run_end.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->sv_label.ensure(Sc * 4));
     F3PS_CUDA_OK(ctx->reg_init.ensure(region_bytes(Sc))); F3PS_CUDA_OK(ctx->reg_work.ensure(region_bytes(Sc)));
     ctx->R0 = carve_regions(ctx->reg_init.p, Sc); ctx->R1 = carve_regions(ctx->reg_work.p, Sc);
@@ -728,6 +729,7 @@ int f3ps_set_graph(f3ps_ctx* ctx, int64_t n_voxels, const float* voxel_xyz, cons
     F3PS_CUDA_OK(ctx->edge_keys_a.ensure(Ec * 8));
     auto up = [&](void* d, const void* h, size_t bytes) { return bytes ? cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, ctx->stream) : cudaSuccess; };
     F3PS_CUDA_OK(up(ctx->vox_xyz.p, h_xyz.data(), (size_t)V * 16)); F3PS_CUDA_OK(up(ctx->pos_run.p, h_posrun.data(), (size_t)V * 4));
+    F3PS_CUDA_OK(up(ctx->graph_vox.p, h_vin.data(), (size_t)V * 4));
     F3PS_CUDA_OK(up(ctx->run_start.p, h_start.data(), (size_t)S * 4)); F3PS_CUDA_OK(up(ctx->run_end.p, h_end.data(), (size_t)S * 4));
     F3PS_CUDA_OK(up(ctx->sv_label.p, h_label.data(), (size_t)S * 4));
     F3PS_CUDA_OK(up(ctx->R0.centroid, h_cen.data(), (size_t)S * 16)); F3PS_CUDA_OK(up(ctx->R0.normal, h_nrm.data(), (size_t)S * 16));
@@ -812,6 +814,7 @@ int merge_restart(f3ps_ctx* ctx) {
 // start of a replay: restart (unless the working state is the one to continue from), merge log, output buffers
 int merge_begin(f3ps_ctx* ctx, bool restart) {
     int rc = mark(ctx, 7); if (rc) return rc;
+    ctx->lv_thr.clear(); ctx->lv_built = 0;
     if (restart && (rc = merge_restart(ctx))) return rc;
     const size_t Sc = std::max(1u, ctx->S), Pc = std::max(1u, ctx->n_pos);
     F3PS_CUDA_OK(ctx->mlog.ensure(Sc * 20));
@@ -893,10 +896,11 @@ int merge_labels(f3ps_ctx* ctx) {
                   ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>());
     return F3PS_OK;
 }
-// after the replay's scalars reached the host
-int merge_done(f3ps_ctx* ctx) {
+// after the replay's scalars reached the host; the merged state is one level, its threshold (f3ps_merge_levels records more)
+int merge_done(f3ps_ctx* ctx, float threshold) {
     if (ctx->h_sc->mctl.error) return ctx_fail(ctx, F3PS_ERR_CAPACITY, "merge kernel reported an internal capacity error");
     ctx->n_out = ctx->h_sc->n_out;
+    ctx->lv_thr.assign(1, threshold); ctx->lv_M = ctx->h_sc->mctl.n_merges;
     ctx->progress = P_MERGED;
     return F3PS_OK;
 }
@@ -944,7 +948,7 @@ int merge_one(f3ps_ctx* ctx, float threshold, MergeStart start) {
     }
     rc = mark(ctx, 8); if (rc) return rc;
     rc = pull_scalars(ctx); if (rc) return rc;
-    return merge_done(ctx);
+    return merge_done(ctx, threshold);
 }
 }
 }
@@ -1019,7 +1023,7 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
         f3ps_ctx* ctx = ctxs[i];
         rc = pull_scalars(ctx); if (rc) return rc;
         const unsigned err = ctx->h_sc->mctl.error;
-        rc = err ? merge_one(ctx, threshold, err == kFastErrTouched ? kStartContinue : kStartGeneral) : merge_done(ctx);
+        rc = err ? merge_one(ctx, threshold, err == kFastErrTouched ? kStartContinue : kStartGeneral) : merge_done(ctx, threshold);
         if (rc) return rc;
     }
     return F3PS_OK;
@@ -1662,6 +1666,132 @@ int f3ps_get_voxel_segments_device(f3ps_ctx* ctx, const uint32_t** device_ptr, i
     return F3PS_OK;
 }
 
+// ---- segmentation levels (kernels_levels.cuh) ---------------------------------------------------------
+extern "C++" {
+namespace {
+// merge forest of the last replay: parent and merge time per initial supervoxel
+int levels_forest(f3ps_ctx* ctx) {
+    const unsigned S = ctx->S, M = ctx->lv_M;
+    const size_t Sc = std::max(1u, S);
+    F3PS_CUDA_OK(ctx->lv_parent.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->lv_when.ensure(Sc * 4));
+    F3PS_CUDA_OK(cudaMemsetAsync(ctx->lv_when.p, 0xff, Sc * 4, ctx->stream));
+    if (M) LAUNCH(ctx, levels_forest_kernel, grid_for(M, 256), 256, 0, ctx->ML.a, ctx->ML.b, M, ctx->sv_label.as<unsigned>(), S,
+                  ctx->lv_parent.as<unsigned>(), ctx->lv_when.as<unsigned>());
+    return F3PS_OK;
+}
+// lv_small = thresholds, merges and segment counts of up to kMaxLevels levels
+unsigned* levels_m(f3ps_ctx* ctx) { return ctx->lv_small.as<unsigned>() + kMaxLevels; }
+unsigned* levels_nseg(f3ps_ctx* ctx) { return ctx->lv_small.as<unsigned>() + 2 * kMaxLevels; }
+// merges, segment counts and per-supervoxel labels (lv_seg[S][level_row(L)]) of L ascending thresholds, on the forest
+int levels_tables(f3ps_ctx* ctx, const float* thr, int L) {
+    const unsigned S = ctx->S; const int Lp = level_row(L);
+    const size_t Sc = std::max(1u, S);
+    F3PS_CUDA_OK(ctx->lv_small.ensure(3 * kMaxLevels * 4));
+    F3PS_CUDA_OK(ctx->lv_dense.ensure((size_t)L * Sc * 4)); F3PS_CUDA_OK(ctx->lv_seg.ensure((size_t)Lp * Sc * 4));
+    F3PS_CUDA_OK(cudaMemcpyAsync(ctx->lv_small.p, thr, (size_t)L * 4, cudaMemcpyHostToDevice, ctx->stream));
+    LAUNCH(ctx, levels_prefix_kernel, 1, 1024, 2 * L * 4, ctx->ML.w, ctx->lv_M, ctx->lv_small.as<float>(), L, levels_m(ctx));
+    LAUNCH(ctx, levels_dense_kernel, L, 1024, 0, ctx->lv_when.as<unsigned>(), S, levels_m(ctx), ctx->lv_dense.as<unsigned>(), levels_nseg(ctx));
+    if (S) LAUNCH(ctx, levels_roots_kernel, grid_for(S, 256), 256, 0, ctx->lv_parent.as<unsigned>(), ctx->lv_when.as<unsigned>(), levels_m(ctx),
+                  ctx->lv_dense.as<unsigned>(), S, L, Lp, ctx->lv_seg.as<unsigned>());
+    return F3PS_OK;
+}
+// the level tables of the handle's levels, built on first use after a merge; voxels: the voxel table [V][level_row(L)] as well
+int levels_ready(f3ps_ctx* ctx, bool voxels, const char* what) {
+    int rc = need(ctx, P_MERGED, what); if (rc) return rc;
+    if (ctx->lv_thr.empty()) return ctx_fail(ctx, F3PS_ERR_LOGIC, std::string(what) + ": no merged state");
+    cudaSetDevice(ctx->device);
+    const int L = (int)ctx->lv_thr.size(), Lp = level_row(L);
+    if (ctx->lv_built < 1) {
+        if ((rc = levels_forest(ctx)) || (rc = levels_tables(ctx, ctx->lv_thr.data(), L))) return rc;
+        ctx->lv_m_h.clear(); ctx->lv_nseg_h.clear();
+        ctx->lv_built = 1;
+    }
+    if (voxels && ctx->lv_built < 2) {
+        const unsigned V = ctx->V, P = ctx->n_pos;
+        F3PS_CUDA_OK(ctx->lv_vox.ensure(std::max<size_t>(1, (size_t)V * Lp) * 4));
+        F3PS_CUDA_OK(cudaMemsetAsync(ctx->lv_vox.p, 0xff, (size_t)V * Lp * 4, ctx->stream));
+        const bool host = ctx->graph_from_host;
+        if (P) LAUNCH(ctx, levels_voxel_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), P, host ? ctx->graph_vox.as<unsigned>() : ctx->order,
+                      host ? nullptr : ctx->sorted_label, host ? nullptr : ctx->owner0.as<unsigned>(), ctx->lv_seg.as<unsigned>(), Lp, ctx->lv_vox.as<unsigned>());
+        ctx->lv_built = 2;
+    }
+    return F3PS_OK;
+}
+// labels[L][n] = voxel table row pv[i] (pv == nullptr: row i).  Device memory: one launch, enqueued.  Host memory: through a
+// staging buffer of at most kLevelStageWords words, a chunk of points at a time (a 50 M-point cloud at 41 levels would
+// otherwise hold 8 GB of device memory for a copy).
+constexpr size_t kLevelStageWords = (size_t)1 << 24;
+int level_labels(f3ps_ctx* ctx, const int* pv, int64_t n, uint32_t* labels, int64_t capacity, int on_device) {
+    const int L = (int)ctx->lv_thr.size(), Lp = level_row(L);
+    const size_t words = (size_t)L * (size_t)n;
+    int rc = cap_check(ctx, (int64_t)words, capacity); if (rc) return rc;
+    if (!words) return F3PS_OK;
+    if (!labels) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "no output buffer");
+    const unsigned* table = ctx->lv_vox.as<unsigned>();
+    if (on_device) {
+        const int vec = ((uintptr_t)labels % 16 == 0 && n % 4 == 0) ? 1 : 0;
+        LAUNCH(ctx, level_point_labels_kernel, grid_for((n + 3) / 4, 256), 256, 0, pv, 0, (long long)n, table, L, Lp, (unsigned*)labels, vec);
+        return F3PS_OK;
+    }
+    const int64_t chunk = std::min<int64_t>(n, std::max<int64_t>(4, (int64_t)(kLevelStageWords / L) & ~(int64_t)3));
+    F3PS_CUDA_OK(ctx->lv_points.ensure((size_t)chunk * L * 4));
+    unsigned* stage = ctx->lv_points.as<unsigned>();
+    for (int64_t p0 = 0; p0 < n; p0 += chunk) {
+        const int64_t m = std::min(chunk, n - p0);
+        LAUNCH(ctx, level_point_labels_kernel, grid_for((m + 3) / 4, 256), 256, 0, pv ? pv + p0 : nullptr, (int)p0, (long long)m, table, L, Lp,
+               stage, m % 4 == 0 ? 1 : 0);
+        F3PS_CUDA_OK(cudaMemcpy2DAsync(labels + p0, (size_t)n * 4, stage, (size_t)m * 4, (size_t)m * 4, (size_t)L, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    return fin(ctx);
+}
+} // namespace
+} // extern "C++"
+
+int f3ps_merge_levels(f3ps_ctx* ctx, const float* thresholds, int n_levels) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    if (!thresholds || n_levels < 1 || n_levels > kMaxLevels) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "f3ps_merge_levels: 1 to 256 thresholds");
+    for (int k = 0; k < n_levels; ++k)
+        if (!std::isfinite(thresholds[k]) || (k && thresholds[k] < thresholds[k - 1]))
+            return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "f3ps_merge_levels: thresholds must be finite and non-decreasing");
+    int rc = f3ps_merge(ctx, thresholds[n_levels - 1]); if (rc) return rc;     // ONE replay; every level is a prefix of it
+    ctx->lv_thr.assign(thresholds, thresholds + n_levels);
+    return F3PS_OK;
+}
+
+int f3ps_get_levels(f3ps_ctx* ctx, int32_t* n_levels, float* thresholds, int32_t* n_merges, int32_t* n_segments, int32_t capacity) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    int rc = levels_ready(ctx, false, "f3ps_get_levels"); if (rc) return rc;
+    const int L = (int)ctx->lv_thr.size();
+    if (n_levels) *n_levels = L;
+    if (!thresholds && !n_merges && !n_segments) return F3PS_OK;
+    if ((rc = cap_check(ctx, L, capacity))) return rc;
+    if ((n_merges || n_segments) && ctx->lv_m_h.empty()) {
+        ctx->lv_m_h.resize(L); ctx->lv_nseg_h.resize(L);
+        if ((rc = d2h(ctx, ctx->lv_m_h.data(), levels_m(ctx), (size_t)L * 4)) || (rc = d2h(ctx, ctx->lv_nseg_h.data(), levels_nseg(ctx), (size_t)L * 4)) ||
+            (rc = fin(ctx))) { ctx->lv_m_h.clear(); return rc; }
+    }
+    for (int k = 0; k < L; ++k) {
+        if (thresholds) thresholds[k] = ctx->lv_thr[k];
+        if (n_merges) n_merges[k] = ctx->lv_m_h[k];
+        if (n_segments) n_segments[k] = ctx->lv_nseg_h[k];
+    }
+    return F3PS_OK;
+}
+
+int f3ps_get_level_voxel_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacity, int on_device) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    int rc = levels_ready(ctx, true, "f3ps_get_level_voxel_labels"); if (rc) return rc;
+    return level_labels(ctx, nullptr, ctx->V, labels, capacity, on_device);
+}
+
+int f3ps_get_level_point_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacity, int on_device) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    if (ctx->graph_from_host) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_get_level_point_labels: no input cloud, the graph was supplied by the caller");
+    if (ctx->slab_range) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_get_level_point_labels: slab mode, the handle holds no input cloud of its own voxels");
+    int rc = levels_ready(ctx, true, "f3ps_get_level_point_labels"); if (rc) return rc;
+    return level_labels(ctx, ctx->point_voxel.as<int>(), ctx->n_points, labels, capacity, on_device);
+}
+
 // ---- device self tests ------------------------------------------------------------------------------
 // =====================================================================================================
 // "next" row f1: Clustering::all_thresh (src/clustering.cpp:691-729) + Testing::eval_performance (src/testing.cpp:239-362).
@@ -1747,22 +1877,7 @@ int f3ps_eval_thresholds(f3ps_ctx* ctx, const uint32_t* truth_label, int64_t n_v
     cudaSetDevice(ctx->device);
     rc = f3ps_merge(ctx, thresholds[n_thresholds - 1]); if (rc) return rc;      // ONE replay; every threshold is a prefix of it
     const unsigned S = ctx->S, V = ctx->V, P = ctx->n_pos;
-    const unsigned M = ctx->h_sc->mctl.n_merges;
     if (ctx->n_out == 0) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "The pointcloud to be set as 'segm' cannot be empty");  // testing.cpp:413-416
-    // merge forest on the host (M, S are small): label -> rank, parent / time per initial supervoxel
-    std::vector<unsigned> la(M), lb(M), svl(S); std::vector<float> lw(M);
-    if (M) {
-        if ((rc = d2h(ctx, la.data(), ctx->ML.a, (size_t)M * 4))) return rc;
-        if ((rc = d2h(ctx, lb.data(), ctx->ML.b, (size_t)M * 4))) return rc;
-        if ((rc = d2h(ctx, lw.data(), ctx->ML.w, (size_t)M * 4))) return rc;
-    }
-    if ((rc = d2h(ctx, svl.data(), ctx->sv_label.p, (size_t)S * 4))) return rc;
-    if ((rc = fin(ctx))) return rc;
-    std::map<unsigned, unsigned> rank_of;
-    for (unsigned s = 0; s < S; ++s) rank_of[svl[s]] = s;
-    std::vector<unsigned> parent(S), when(S, 0xffffffffu);
-    for (unsigned s = 0; s < S; ++s) parent[s] = s;
-    for (unsigned i = 0; i < M; ++i) { const unsigned ra = rank_of[la[i]], rb = rank_of[lb[i]]; parent[rb] = ra; when[rb] = i; }
     // Testing::label_map on the truth: dense labels in ascending label order, segment sizes
     std::map<unsigned, unsigned> tmap;
     size_t n_truth_points = 0;
@@ -1778,34 +1893,34 @@ int f3ps_eval_thresholds(f3ps_ctx* ctx, const uint32_t* truth_label, int64_t n_v
     for (int64_t v = 0; v < n_extra; ++v) g[tmap[extra_truth_label[v]]]++;    // truth points outside the segmentation's voxels
     const unsigned Kc = Kt + 1;
     if ((size_t)S * Kc > ((size_t)1 << 28)) return ctx_fail(ctx, F3PS_ERR_CAPACITY, "contingency table above 2^28 cells");
-    const size_t Sc = std::max(1u, S);
-    F3PS_CUDA_OK(ctx->ev_parent.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->ev_when.ensure(Sc * 4)); F3PS_CUDA_OK(ctx->ev_dense.ensure(Sc * 4 + 4));
     F3PS_CUDA_OK(ctx->ev_truth.ensure((size_t)V * 4)); F3PS_CUDA_OK(ctx->ev_table.ensure(std::max<size_t>(1, (size_t)S * Kc) * 4));
-    F3PS_CUDA_OK(cudaMemcpyAsync(ctx->ev_parent.p, parent.data(), (size_t)S * 4, cudaMemcpyHostToDevice, ctx->stream));
-    F3PS_CUDA_OK(cudaMemcpyAsync(ctx->ev_when.p, when.data(), (size_t)S * 4, cudaMemcpyHostToDevice, ctx->stream));
     F3PS_CUDA_OK(cudaMemcpyAsync(ctx->ev_truth.p, tdense.data(), (size_t)V * 4, cudaMemcpyHostToDevice, ctx->stream));
-    unsigned* d_nseg = ctx->ev_dense.as<unsigned>() + Sc;
-    std::vector<unsigned> table;
+    // the segmentation at every threshold: the level tables of the replay, kMaxLevels thresholds at a time
+    rc = levels_forest(ctx); if (rc) return rc;
+    std::vector<unsigned> table, m_at(kMaxLevels), nseg_at(kMaxLevels);
     unsigned m_prev = 0xffffffffu;
-    for (int k = 0; k < n_thresholds; ++k) {
-        unsigned m = M;                                                       // first step whose head weight is >= t (strict <, :388-389)
-        for (unsigned i = 0; i < M; ++i) if (!(lw[i] < thresholds[k])) { m = i; break; }
-        if (n_merges_at) n_merges_at[k] = (int32_t)m;
-        if (m == m_prev) { perf[k] = perf[k - 1]; if (n_segments) n_segments[k] = n_segments[k - 1]; continue; }
-        m_prev = m;
-        LAUNCH(ctx, eval_dense_kernel, 1, 1024, 0, ctx->ev_when.as<unsigned>(), S, m, ctx->ev_dense.as<unsigned>(), d_nseg);
-        F3PS_CUDA_OK(cudaMemsetAsync(ctx->ev_table.p, 0, std::max<size_t>(1, (size_t)S * Kc) * 4, ctx->stream));
-        if (P) LAUNCH(ctx, eval_table_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), ctx->order, P, ctx->ev_parent.as<unsigned>(),
-                      ctx->ev_when.as<unsigned>(), ctx->ev_dense.as<unsigned>(), m, ctx->ev_truth.as<unsigned>(), Kc, ctx->ev_table.as<unsigned>());
-        unsigned n_seg = 0;
-        if ((rc = d2h(ctx, &n_seg, d_nseg, 4))) return rc;
+    for (int k0 = 0; k0 < n_thresholds; k0 += kMaxLevels) {
+        const int L = std::min(kMaxLevels, n_thresholds - k0);
+        rc = levels_tables(ctx, thresholds + k0, L); if (rc) return rc;
+        if ((rc = d2h(ctx, m_at.data(), levels_m(ctx), (size_t)L * 4)) || (rc = d2h(ctx, nseg_at.data(), levels_nseg(ctx), (size_t)L * 4))) return rc;
         if ((rc = fin(ctx))) return rc;
-        table.resize((size_t)n_seg * Kc);
-        if (n_seg) { if ((rc = d2h(ctx, table.data(), ctx->ev_table.p, (size_t)n_seg * Kc * 4))) return rc; if ((rc = fin(ctx))) return rc; }
-        perf[k] = testing_scores(table, n_seg, Kt, g, n_truth_points);
-        if (n_segments) n_segments[k] = (int32_t)n_seg;
+        for (int j = 0; j < L; ++j) {
+            const int k = k0 + j;
+            const unsigned m = m_at[j];                                           // first step whose head weight is >= t (strict <, :388-389)
+            if (n_merges_at) n_merges_at[k] = (int32_t)m;
+            if (m == m_prev) { perf[k] = perf[k - 1]; if (n_segments) n_segments[k] = n_segments[k - 1]; continue; }
+            m_prev = m;
+            const unsigned n_seg = nseg_at[j];
+            F3PS_CUDA_OK(cudaMemsetAsync(ctx->ev_table.p, 0, std::max<size_t>(1, (size_t)S * Kc) * 4, ctx->stream));
+            if (P) LAUNCH(ctx, eval_table_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), ctx->order, P, ctx->lv_seg.as<unsigned>(),
+                          level_row(L), j, ctx->ev_truth.as<unsigned>(), Kc, ctx->ev_table.as<unsigned>());
+            table.resize((size_t)n_seg * Kc);
+            if (n_seg) { if ((rc = d2h(ctx, table.data(), ctx->ev_table.p, (size_t)n_seg * Kc * 4))) return rc; if ((rc = fin(ctx))) return rc; }
+            perf[k] = testing_scores(table, n_seg, Kt, g, n_truth_points);
+            if (n_segments) n_segments[k] = (int32_t)n_seg;
+        }
     }
-    return F3PS_OK;
+    return F3PS_OK;      // the level tables now hold the sweep's thresholds: the handle's one level, the last, is rebuilt on demand
 }
 
 

@@ -2,52 +2,26 @@
 // + the counting part of Testing (src/testing.cpp:62-146) from ONE merge replay.
 // The reference re-clusters and re-intersects point sets for each of its 41 thresholds; continuing `cluster(state, t)` is the
 // same as never having stopped, so every threshold is a PREFIX of one merge log (SURVEY.md CS4).  On the device:
-//   merge log -> (parent, time) forest over the initial supervoxels; the region of supervoxel s after m merges is the
-//   root reached by following parents whose time < m; dense labels = rank among the alive roots (ascending label,
-//   get_labeled_cloud :640-663); contingency table = histogram over the labelled voxel cloud of (segment, truth label).
+//   merge log -> per-supervoxel segment labels at every threshold (the level tables of kernels_levels.cuh: dense labels in
+//   ascending label order, as get_labeled_cloud :640-663); contingency table = histogram over the labelled voxel cloud of
+//   (segment, truth label).
 // Intersections by exact xyz (Testing::count_intersect) become equality of the voxel index: both clouds are voxel
 // centroids of the same grid.
 #pragma once
 #include "kernels_merge.cuh"
+#include "kernels_levels.cuh"
 
 namespace f3ps {
 
-// one block: alive flags at prefix m -> dense label per alive root (exclusive scan in ascending rank = ascending label)
-__global__ void __launch_bounds__(1024) eval_dense_kernel(const unsigned* __restrict__ when, unsigned S, unsigned m,
-        unsigned* __restrict__ dense, unsigned* __restrict__ n_segments) {
-    __shared__ unsigned s_w[32]; __shared__ unsigned s_carry;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (unsigned base = 0; base < S; base += blockDim.x) {
-        const unsigned s = base + threadIdx.x;
-        const unsigned alive = (s < S && when[s] >= m) ? 1u : 0u;
-        unsigned v = alive;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const unsigned t = __shfl_up_sync(kFull, v, o); if (lane >= o) v += t; }
-        if (lane == 31) s_w[warp] = v;
-        __syncthreads();
-        unsigned wb = 0;
-        for (int w = 0; w < warp; ++w) wb += s_w[w];
-        const unsigned carry = s_carry;
-        if (s < S) dense[s] = alive ? carry + wb + v - 1u : 0xffffffffu;
-        __syncthreads();
-        if (threadIdx.x == blockDim.x - 1) s_carry = carry + wb + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *n_segments = s_carry;
-}
-
-// histogram over the labelled voxel cloud: position i belongs to initial supervoxel pos_run[i] and is voxel order[i]
+// histogram over the labelled voxel cloud: position i belongs to initial supervoxel pos_run[i] and is voxel order[i]; its
+// segment at level k is seg[s][k] (kernels_levels.cuh).  A phantom leaf counts twice, as it appears in the labelled cloud.
 __global__ void __launch_bounds__(256) eval_table_kernel(const unsigned* __restrict__ pos_run, const unsigned* __restrict__ order, unsigned n_pos,
-        const unsigned* __restrict__ parent, const unsigned* __restrict__ when, const unsigned* __restrict__ dense, unsigned m,
-        const unsigned* __restrict__ truth_dense, unsigned n_truth, unsigned* __restrict__ table) {
+        const unsigned* __restrict__ seg, int Lp, int k, const unsigned* __restrict__ truth_dense, unsigned n_truth, unsigned* __restrict__ table) {
     for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += gridDim.x * blockDim.x) {
-        unsigned s = pos_run[i];
+        const unsigned s = pos_run[i];
         if (s == 0xffffffffu) continue;                      // unowned voxel: absent from the segmentation
-        while (when[s] < m) s = parent[s];
         const unsigned v = order ? order[i] : i;
-        atomicAdd(&table[(size_t)dense[s] * n_truth + truth_dense[v]], 1u);
+        atomicAdd(&table[(size_t)seg[(size_t)s * Lp + k] * n_truth + truth_dense[v]], 1u);
     }
 }
 

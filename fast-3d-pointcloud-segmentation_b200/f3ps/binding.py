@@ -92,6 +92,10 @@ def lib():
         "f3ps_get_labeled_cloud": (C.c_int, [vp, vp, vp, vp, i64]),
         "f3ps_get_region_mean_color": (C.c_int, [vp, i32, vp]),
         "f3ps_get_voxel_segments_device": (C.c_int, [vp, C.POINTER(vp), C.POINTER(i64)]),
+        "f3ps_merge_levels": (C.c_int, [vp, vp, C.c_int]),
+        "f3ps_get_levels": (C.c_int, [vp, C.POINTER(i32), vp, vp, vp, i32]),
+        "f3ps_get_level_voxel_labels": (C.c_int, [vp, vp, i64, C.c_int]),
+        "f3ps_get_level_point_labels": (C.c_int, [vp, vp, i64, C.c_int]),
         "f3ps_stage_ms": (C.c_int, [vp, C.c_int, C.POINTER(f32)]),
         "f3ps_launch_count": (i64, [vp]),
         "f3ps_merge_profile": (C.c_int, [vp, C.POINTER(C.c_uint64 * 32)]),
@@ -135,7 +139,8 @@ EXPORTED = ["f3ps_create", "f3ps_destroy", "f3ps_last_error", "f3ps_version", "f
             "f3ps_get_voxel_neighbors", "f3ps_get_voxel_normals", "f3ps_get_seeds", "f3ps_get_voxel_labels",
             "f3ps_get_supervoxels", "f3ps_get_supervoxel_voxels", "f3ps_get_adjacency", "f3ps_get_edges", "f3ps_get_cdf",
             "f3ps_get_merge_log", "f3ps_get_state_regions", "f3ps_get_state_edges", "f3ps_get_labeled_cloud", "f3ps_get_region_mean_color",
-            "f3ps_get_voxel_segments_device", "f3ps_stage_ms", "f3ps_launch_count", "f3ps_merge_profile", "f3ps_merge_trace", "f3ps_expand_profile", "f3ps_test_rgb2lab",
+            "f3ps_get_voxel_segments_device", "f3ps_merge_levels", "f3ps_get_levels", "f3ps_get_level_voxel_labels",
+            "f3ps_get_level_point_labels", "f3ps_stage_ms", "f3ps_launch_count", "f3ps_merge_profile", "f3ps_merge_trace", "f3ps_expand_profile", "f3ps_test_rgb2lab",
             "f3ps_test_lab_ciede00", "f3ps_test_rgb_eucl", "f3ps_test_sort_pairs",
             "f3ps_merge_batch", "f3ps_set_expand_sharing", "f3ps_set_expand_kernel", "f3ps_refine", "f3ps_eval_thresholds", "f3ps_eval_label_pairs", "f3ps_slab_reset", "f3ps_slab_bbox", "f3ps_slab_set_frame", "f3ps_slab_keys", "f3ps_slab_route", "f3ps_slab_array",
             "f3ps_slab_set_voxels", "f3ps_slab_expand_begin", "f3ps_slab_expand_sweep", "f3ps_slab_expand_round_end",
@@ -366,6 +371,41 @@ class Segmenter:
         l = np.zeros(n, np.uint32); x = np.zeros((n, 3), np.float32); nn = np.zeros((n, 3), np.float32); k = np.zeros(n, np.int32)
         self._chk(self.L.f3ps_get_state_regions(self.h, _p(l), _p(x), _p(nn), _p(k), n))
         return l, x, nn, k
+
+    # ---- segmentation levels: several thresholds from one merge replay ----
+    def merge_levels(self, thresholds):
+        """One replay, merge(max(thresholds)), recording the segmentation at every threshold (1 to 256, finite, non-decreasing)."""
+        t = np.ascontiguousarray(thresholds, np.float32).ravel()
+        self._chk(self.L.f3ps_merge_levels(self.h, _p(t) if t.size else None, t.size))
+
+    def levels(self):
+        """{"thresholds", "n_merges", "n_segments"} of the recorded levels (a plain merge records one: its threshold)."""
+        n = self._n_levels()
+        t = np.zeros(n, np.float32); m = np.zeros(n, np.int32); s = np.zeros(n, np.int32)
+        self._chk(self.L.f3ps_get_levels(self.h, None, _p(t), _p(m), _p(s), n))
+        return {"thresholds": t, "n_merges": m, "n_segments": s}
+
+    def _n_levels(self):
+        n = C.c_int32()
+        self._chk(self.L.f3ps_get_levels(self.h, C.byref(n), None, None, None, 0))
+        return n.value
+
+    def voxel_labels(self):
+        """uint32 [L, V]: the segment of every voxel at every level (0xffffffff: no supervoxel owns it)."""
+        out = np.empty((self._n_levels(), self.counts().n_voxels), np.uint32)
+        self._chk(self.L.f3ps_get_level_voxel_labels(self.h, _p(out), out.size, 0))
+        return out
+
+    def point_labels(self):
+        """uint32 [L, N]: the segment of every input point at every level, in input order (0xffffffff: no voxel)."""
+        out = np.empty((self._n_levels(), self.counts().n_points), np.uint32)
+        self._chk(self.L.f3ps_get_level_point_labels(self.h, _p(out), out.size, 0))
+        return out
+
+    def point_labels_device(self, dev_ptr, capacity):
+        """point_labels() into a CUDA buffer of `capacity` uint32 elements (e.g. a torch tensor's data_ptr()), enqueued on the
+        handle's stream without waiting: sync() before reading it from another stream or the host."""
+        self._chk(self.L.f3ps_get_level_point_labels(self.h, C.c_void_p(dev_ptr), capacity, 1))
 
     def supervoxel_voxels(self):
         c = self.counts()

@@ -9,7 +9,8 @@
 // file "<stem>_<o>" in a -d sweep), --facade routes through the Clustering / SupervoxelClustering
 // classes instead of the fused path, --gpus N shards the files of a -d sweep over N GPUs (no collective), --inflight K =
 // files per group of a sweep: K1..K6 of a file on its own handle + stream, ONE merge launch per group (f3ps_merge_batch),
-// the next group's front stages overlapping it.
+// the next group's front stages overlapping it.  --levels t1,t2,... prints the segmentation at several thresholds from one
+// extra merge replay, --point-labels <file.pcd> writes the input cloud with every point's segment (one file per level).
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -46,6 +47,7 @@ struct Options {
     float thresh = 0; bool thresh_specified = true; bool rgb = false, cvx = false, ml = false, al = false, eq = false, disable_transform = false, verbose = false, facade = false;
     float lambda = 0; int bin_num = 0; std::string out;
     bool remove_label = false; uint32_t label_to_be_removed = 0; std::string test_filename = "test"; bool eval = true;
+    std::vector<float> levels; std::string point_labels;
 };
 struct FileScores { bool have_best = false; f3ps_performance best; std::vector<std::pair<float, f3ps_performance>> all; };
 
@@ -70,6 +72,8 @@ void usage(const char* a0) {
            "\t --NT                           (disables the single camera transform) \n"
            "\t --V                            (verbose: prints the merge sequence) \n"
            "\t -o <file.pcd>                  (writes the labelled voxel cloud) \n"
+           "\t --levels <t1,t2,...>           (prints the segment counts at these ascending thresholds, one extra merge replay) \n"
+           "\t --point-labels <file.pcd>      (writes every input point with its segment; with --levels one file <stem>_<k>.pcd per level)\n"
            "\t --facade                       (runs through the Clustering / SupervoxelClustering classes) \n"
            "\t --gpus <N>                     (shards the files of -d over N GPUs) \n"
            "\t --inflight <K>                 (frames in flight per GPU during a -d sweep, default 8) \n"
@@ -282,7 +286,10 @@ int process_file(const std::string& file, const Options& o, int device, std::str
     auto t0 = std::chrono::steady_clock::now();
     pcl::PointCloud<pcl::PointXYZL>::Ptr labeled(new pcl::PointCloud<pcl::PointXYZL>());
     size_t n_sv = 0, n_seg = 0, n_merges = 0; float stage[9] = {0};
+    float thresh = o.thresh;                                                 // of the final segmentation: -t or the sweep's choice
     std::vector<MergeStep> log;
+    std::unique_ptr<f3ps::Handle> local;                                     // -p: a handle of its own; sweeps reuse the worker's (buffers stay allocated)
+    f3ps::Handle* hp = nullptr;
     if (o.facade) {
         pcl::SupervoxelClustering<pcl::PointXYZRGBA> super(o.voxel_resolution, o.seed_resolution, device);
         super.setUseSingleCameraTransform(!o.disable_transform);
@@ -318,14 +325,13 @@ int process_file(const std::string& file, const Options& o, int device, std::str
         n_sv = supervoxel_clusters.size(); n_seg = segmentation.get_currentstate().first.size();
         log = segmentation.get_merge_log(); n_merges = log.size();
     } else {
-        std::unique_ptr<f3ps::Handle> local;                                 // -p: a handle of its own; sweeps reuse the worker's (buffers stay allocated)
         if (!worker) local.reset(new f3ps::Handle(device));
-        f3ps::Handle& h = worker ? *worker : *local;
+        hp = worker ? worker : local.get();
+        f3ps::Handle& h = *hp;
         h.check(f3ps_set_vccs_params(h.get(), o.voxel_resolution, o.seed_resolution, o.color_importance, o.spatial_importance,
                                      o.normal_importance, o.disable_transform ? 0 : 1, 0));
         h.check(f3ps_set_merge_params(h.get(), o.rgb ? F3PS_RGB_EUCL : F3PS_LAB_CIEDE00, o.cvx ? F3PS_CONVEX_NORMALS_DIFF : F3PS_NORMALS_DIFF, merging, lam, bins));
         h.check(f3ps_set_input(h.get(), cloud->points.data(), (int64_t)cloud->size(), 32, 0));
-        float thresh = o.thresh;
         std::vector<uint32_t> truth;
         if (o.thresh_specified && !o.eval) h.check(f3ps_run(h.get(), thresh));
         else {
@@ -359,10 +365,39 @@ int process_file(const std::string& file, const Options& o, int device, std::str
              cloud->size(), n_merges, n_seg, labeled->size(), ms, device); report += buf;
     if (!o.facade) { snprintf(buf, sizeof buf, "  stage ms: voxelize %.3f neighbors %.3f normals %.3f seeds %.3f expand %.3f graph %.3f merge %.3f total %.3f\n",
                               stage[0], stage[1], stage[2], stage[3], stage[4], stage[5], stage[6], stage[7]); report += buf; }
-    if (!o.out.empty()) {                                                // a sweep writes one file per input: <stem>_<o> next to -o's path
-        std::string out = o.out;
-        if (in_sweep) { const std::filesystem::path op(o.out); out = (op.parent_path() / (std::filesystem::path(file).stem().string() + "_" + op.filename().string())).string(); }
-        f3ps::savePCDFileASCII(out, *labeled);
+    // a sweep writes one file per input: <stem>_<o> next to -o's path
+    auto per_file = [&](const std::string& name) {
+        if (!in_sweep) return name;
+        const std::filesystem::path op(name);
+        return (op.parent_path() / (std::filesystem::path(file).stem().string() + "_" + op.filename().string())).string();
+    };
+    if (!o.out.empty()) f3ps::savePCDFileASCII(per_file(o.out), *labeled);
+    if (hp && (!o.levels.empty() || !o.point_labels.empty())) {         // one more replay; the segmentation above stays f3ps_merge(thresh)'s
+        f3ps::Handle& h = *hp;
+        const std::vector<float> thr = o.levels.empty() ? std::vector<float>(1, thresh) : o.levels;
+        h.check(f3ps_merge_levels(h.get(), thr.data(), (int)thr.size()));
+        const int L = (int)thr.size();
+        std::vector<int32_t> nm(L), ns(L);
+        h.check(f3ps_get_levels(h.get(), nullptr, nullptr, nm.data(), ns.data(), L));
+        if (!o.levels.empty())
+            for (int k = 0; k < L; ++k) { snprintf(buf, sizeof buf, "level %d: threshold %f -> %d merges -> %d segments\n", k, thr[k], nm[k], ns[k]); report += buf; }
+        if (!o.point_labels.empty()) {
+            const size_t N = cloud->size();
+            std::vector<uint32_t> lab((size_t)L * N);
+            h.check(f3ps_get_level_point_labels(h.get(), lab.data(), (int64_t)lab.size(), 0));
+            const std::filesystem::path base(per_file(o.point_labels));
+            pcl::PointCloud<pcl::PointXYZL> pc;
+            pc.resize(N);
+            for (int k = 0; k < L; ++k) {
+                for (size_t i = 0; i < N; ++i) {
+                    const auto& q = cloud->points[i]; auto& p = pc.points[i];
+                    p.x = q.x; p.y = q.y; p.z = q.z; p.label = lab[(size_t)k * N + i];
+                }
+                const std::string name = o.levels.empty() ? base.string()
+                    : (base.parent_path() / (base.stem().string() + "_" + std::to_string(k) + base.extension().string())).string();
+                f3ps::savePCDFileASCII(name, pc);
+            }
+        }
     }
     return 0;
 }
@@ -456,6 +491,20 @@ int main(int argc, char** argv) {
     if (o.remove_label) { int r = 0; parse(argc, argv, "-r", r); o.label_to_be_removed = (uint32_t)r; }
     if (find_switch(argc, argv, "-f")) parse(argc, argv, "-f", o.test_filename);
     o.eval = !find_switch(argc, argv, "--no-eval");
+    std::string levels;
+    if (parse(argc, argv, "--levels", levels)) {
+        for (const char* c = levels.c_str(); *c;) {
+            char* end = nullptr;
+            o.levels.push_back(strtof(c, &end));
+            if (end == c || (*end && *end != ',')) { fprintf(stderr, "--levels takes comma-separated thresholds\n"); return 1; }
+            c = *end ? end + 1 : end;
+        }
+        if (o.levels.empty()) { fprintf(stderr, "--levels takes comma-separated thresholds\n"); return 1; }
+    }
+    parse(argc, argv, "--point-labels", o.point_labels);
+    if ((!o.levels.empty() || !o.point_labels.empty()) && (o.facade || find_switch(argc, argv, "--slabs"))) {
+        fprintf(stderr, "--levels and --point-labels run on the direct path of one GPU per file: drop --facade / --slabs\n"); return 1;
+    }
     int gpus = 1; parse(argc, argv, "--gpus", gpus); gpus = std::max(1, gpus);
     int inflight = 8; parse(argc, argv, "--inflight", inflight); inflight = std::max(1, inflight);
     setenv("CUDA_DEVICE_MAX_CONNECTIONS", "32", 0);                     // before the CUDA context exists (see f3ps_create)
@@ -473,8 +522,9 @@ int main(int argc, char** argv) {
             // -d sweep: files are independent (fresh SupervoxelClustering + Clustering per file in the reference, :348,408).
             // `inflight` frames per GPU, each on its own handle / stream / host thread; reports are printed in file order.
             std::mutex emu; std::string first_error;
-            if (o.thresh_specified && o.out.empty()) {
-                // groups of `inflight` files per GPU: front stages per file, ONE merge launch per group
+            if (o.thresh_specified && o.out.empty() && o.levels.empty() && o.point_labels.empty()) {
+                // groups of `inflight` files per GPU: front stages per file, ONE merge launch per group (-o, --levels and
+                // --point-labels need the per-file path below)
                 std::vector<std::vector<size_t>> share((size_t)gpus);
                 for (size_t i = 0; i < file_list.size(); ++i) share[i % (size_t)gpus].push_back(i);
                 std::vector<std::thread> th;

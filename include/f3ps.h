@@ -196,6 +196,26 @@ int f3ps_get_labeled_cloud(f3ps_ctx* ctx, float* xyz /*[n][3]*/, uint32_t* label
 /* per-voxel final segment label (dense, 0xffffffff = unowned) resident on the device; for device consumers */
 int f3ps_get_voxel_segments_device(f3ps_ctx* ctx, const uint32_t** device_ptr, int64_t* n);
 
+/* ---- segmentation levels: the segmentation at several thresholds from one merge replay ----
+ * Level k is the segmentation f3ps_merge(thresholds[k]) gives: the first m_k merges of the replay, m_k = the first merge log
+ * entry whose weight is not below the threshold (M if none).  Labels are dense 0..K-1 per level, in ascending region label
+ * order as f3ps_get_labeled_cloud numbers them.  A voxel no supervoxel owns gets 0xffffffff, a phantom leaf its owner's segment;
+ * after f3ps_set_graph voxel i is the i-th voxel passed in.  A point gets its voxel's label, 0xffffffff without a voxel.
+ * Every merged state has levels: f3ps_merge, f3ps_run and f3ps_merge_batch leave one (their threshold), f3ps_eval_thresholds
+ * its last threshold.  The level tables are computed on the first getter call after a merge, on the handle's stream; before
+ * any merge the getters return F3PS_ERR_LOGIC. */
+/* ONE replay, f3ps_merge(thresholds[n_levels - 1]), recording n_levels levels; the handle is then in exactly the state of that
+ * f3ps_merge.  1 <= n_levels <= 256 finite, non-decreasing thresholds, else F3PS_ERR_INVALID_ARGUMENT. */
+int f3ps_merge_levels(f3ps_ctx* ctx, const float* thresholds, int n_levels);
+/* any output may be NULL; capacity in levels */
+int f3ps_get_levels(f3ps_ctx* ctx, int32_t* n_levels, float* thresholds, int32_t* n_merges, int32_t* n_segments, int32_t capacity);
+/* labels[L][V] / labels[L][N], level-major; capacity = uint32 elements the buffer holds (>= L*V / L*N).
+ * on_device != 0: `labels` is device memory; the write is enqueued on the handle's stream and the call does not wait.
+ * on_device == 0: the labels reach the host through a device staging buffer of at most 64 MB, kept by the handle.
+ * Point labels are F3PS_ERR_LOGIC after f3ps_set_graph (no input cloud) and in slab mode (after f3ps_slab_set_voxels). */
+int f3ps_get_level_voxel_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacity, int on_device);
+int f3ps_get_level_point_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacity, int on_device);
+
 /* ---- slab mode: one very large cloud cut into spatial slabs, one per GPU (SURVEY.md section 8e; BASELINE config 5) ----
  * Replaces, for one scan too large or too slow for one device, the same calls as above
  * (pcl::SupervoxelClustering::extract, supervoxel_clustering.cpp:357).  A slab is a contiguous range of the x-major
