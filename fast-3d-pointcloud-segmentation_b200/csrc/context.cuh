@@ -96,8 +96,7 @@ struct f3ps_ctx {
     f3ps::DevBuf own_a, own_b, dst_a, dst_b, st0, st1, phantom, phantom_leaf, lab_count, lab_count2, lab_fill;
     f3ps::DevBuf cen_xyz, cen_rgb, cen_nrm, lab_keys_a, lab_keys_b, lab_vals_a, lab_vals_b, seg_start, seg_end;
     int expand_blocks_per_sm = 0, sm_count = 0;
-    bool expand_coop_cap = false;       // expand_ctas caps the grid of the cooperative launch instead
-    int expand_ctas = 0;                // > 0: K5 as an ordinary grid of this many CTAs (f3ps_set_expand_sharing)
+    int expand_ctas = 0;                // > 0: cap of K5's cooperative grid (f3ps_set_expand_sharing)
     unsigned* sorted_label = nullptr; unsigned* sorted_vox = nullptr;
     // K6
     f3ps::DevBuf sv_label, rank_of_label, run_start, run_end, pos_run, edge_set, edge_keys_a, edge_keys_b, edge_vals_a, edge_vals_b;
@@ -124,7 +123,7 @@ struct f3ps_ctx {
     cudaEvent_t ev_batch = nullptr;    // f3ps_merge_batch: set-up done / grid done
     cudaEvent_t ev_wait = nullptr;     // blocking-sync event for sweeps (f3ps_set_blocking_wait)
     bool blocking_wait = false;
-    // slab mode (f3ps_slab_*): injected global frame, owned voxel range, K5 phase state
+    // slab mode (f3ps_slab_*): injected global frame, owned voxel range
     bool slab_frame = false; f3ps::FrameParams slab_fp{};
     bool slab_range = false; unsigned own_begin = 0, own_end = 0;
     f3ps::DevBuf slab_dest, slab_tot;
@@ -137,10 +136,8 @@ struct f3ps_ctx {
     std::vector<int32_t> lv_m_h, lv_nseg_h;
     f3ps::DevBuf lv_small, lv_parent, lv_when, lv_dense, lv_seg, lv_vox, lv_points;
     f3ps::DevBuf graph_vox;             // f3ps_set_graph: voxel index as passed in, per position
-    f3ps::ExpandArgs slab_A{}; int slab_cur = 0; unsigned slab_k = 0; unsigned slab_sweeps = 0; int slab_round = 0; bool slab_expanding = false;
     int expand_kernel_choice = 0;       // f3ps_set_expand_kernel: 0 auto, 1 cooperative grid, 2 one cluster
     int expand_cluster_ctas = 0;        // cap of the cluster size (0 = by V, at most 16)
-    int expand_path = 0;                // what the last f3ps_expand launched: 1 cooperative / shared grid, 2 cluster
     bool expand_cluster_attr_set = false;
     bool lambda_attr_set = false;
 };

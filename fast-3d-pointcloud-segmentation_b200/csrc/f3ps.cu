@@ -6,7 +6,6 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
-#include <condition_variable>
 #include <map>
 #include <mutex>
 #include <new>
@@ -431,19 +430,8 @@ int f3ps_seeds(f3ps_ctx* ctx) {
 // One cooperative launch runs createSupervoxelHelpers, every expansion round and makeSupervoxels' lists
 // (kernels_expand.cuh); the host only learns the number of surviving helpers afterwards.
 // Sweeps: cooperative launches run ONE AT A TIME on a device (measured: K5 of concurrent frames serialises at its solo
-// duration, 0.74 ms per frame, while K1..K4 and K6 scale with the streams), so a sweep may instead launch the expansion
-// kernel as an ordinary small grid (f3ps_set_expand_sharing).  Its software grid barrier needs all CTAs of a launch resident:
-// that holds as long as the CTAs of all expansion kernels in flight fit the SMs no long-running kernel occupies, which the
-// per-device counting semaphore below enforces (the caller states the bound).
-namespace {
-struct ExpandGate { std::mutex m; std::condition_variable cv; int in_flight = 0; int limit = 1; };
-ExpandGate g_expand_gate[16];
-struct ExpandTicket {
-    ExpandGate* g = nullptr;
-    explicit ExpandTicket(ExpandGate* gate) : g(gate) { std::unique_lock<std::mutex> l(g->m); g->cv.wait(l, [&] { return g->in_flight < g->limit; }); ++g->in_flight; }
-    ~ExpandTicket() { { std::lock_guard<std::mutex> l(g->m); --g->in_flight; } g->cv.notify_one(); }
-};
-}
+// duration, 0.74 ms per frame, while K1..K4 and K6 scale with the streams), so a sweep may cap the cooperative grid
+// (f3ps_set_expand_sharing) or run K5 as one thread-block cluster per frame (f3ps_set_expand_kernel).
 
 static int expand_prepare(f3ps_ctx* ctx, ExpandArgs& A) {
     const unsigned V = ctx->V, S0 = ctx->S0; const size_t Vc = std::max(1u, V), Sc = (size_t)S0 + 2, Lc = Vc + Sc;
@@ -511,18 +499,6 @@ static int expand_launch(f3ps_ctx* ctx, bool keep_centroids) {
         cfg.attrs = attr; cfg.numAttrs = 1;
         F3PS_CUDA_OK(cudaLaunchKernelEx(&cfg, expand_cluster_kernel, A));
         ctx->launches++;
-        ctx->expand_path = 2;
-        return expand_finish(ctx);
-    }
-    ctx->expand_path = 1;
-    if (V && ctx->expand_ctas > 0 && !ctx->expand_coop_cap) {
-        // shared mode: a small ordinary grid, bounded concurrency (see ExpandGate); held until the kernel has finished
-        ExpandTicket ticket(&g_expand_gate[ctx->device & 15]);
-        const int64_t want = ((int64_t)V + kExpandThreads - 1) / kExpandThreads;
-        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(want, ctx->expand_ctas));
-        expand_persistent_kernel<<<grid, kExpandThreads, 0, ctx->stream>>>(A);
-        ctx->launches++;
-        F3PS_CUDA_OK(cudaPeekAtLastError());
         return expand_finish(ctx);
     }
     if (V) {
@@ -535,7 +511,7 @@ static int expand_launch(f3ps_ctx* ctx, bool keep_centroids) {
         }
         const int64_t want = ((int64_t)V + kExpandThreads - 1) / kExpandThreads;
         int grid = (int)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)std::min(ctx->expand_blocks_per_sm, 2) * ctx->sm_count));
-        if (ctx->expand_coop_cap && ctx->expand_ctas > 0) grid = std::min(grid, ctx->expand_ctas);   // sweeps: fewer CTAs per frame, more frames side by side
+        if (ctx->expand_ctas > 0) grid = std::min(grid, ctx->expand_ctas);   // sweeps: fewer CTAs per frame, more frames side by side
         void* args[] = {&A};
         F3PS_CUDA_OK(cudaLaunchCooperativeKernel((const void*)expand_persistent_kernel, dim3(grid), dim3(kExpandThreads), args, 0, ctx->stream));
         ctx->launches++;
@@ -1029,20 +1005,11 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
     return F3PS_OK;
 }
 
-// ctas_per_frame = 0: K5 is one cooperative launch over the whole GPU (lowest latency for a single frame, the default).
-// ctas_per_frame > 0: K5 is an ordinary grid of that many CTAs and at most max_concurrent such kernels are in flight on the
-// device (process-wide); the caller guarantees ctas_per_frame * max_concurrent <= SMs not held by long-running kernels.
+// ctas_per_frame = 0: K5's cooperative grid covers the whole GPU (lowest latency for a single frame, the default);
+// ctas_per_frame > 0 caps it at that many CTAs.  max_concurrent must be 0.
 int f3ps_set_expand_sharing(f3ps_ctx* ctx, int ctas_per_frame, int max_concurrent) {
-    if (!ctx || ctas_per_frame < 0 || ctas_per_frame > 2 * kSMs || max_concurrent < 0 ||
-        (ctas_per_frame > 0 && max_concurrent > 0 && (int64_t)ctas_per_frame * max_concurrent > kSMs))
-        return F3PS_ERR_INVALID_ARGUMENT;
+    if (!ctx || ctas_per_frame < 0 || ctas_per_frame > 2 * kSMs || max_concurrent != 0) return F3PS_ERR_INVALID_ARGUMENT;
     ctx->expand_ctas = ctas_per_frame;
-    ctx->expand_coop_cap = ctas_per_frame > 0 && max_concurrent == 0;       // still a cooperative launch, only a smaller grid
-    if (ctas_per_frame > 0 && max_concurrent > 0) {
-        ExpandGate& g = g_expand_gate[ctx->device & 15];
-        { std::lock_guard<std::mutex> l(g.m); g.limit = max_concurrent; }
-        g.cv.notify_all();
-    }
     return F3PS_OK;
 }
 
@@ -1085,7 +1052,7 @@ int f3ps_run(f3ps_ctx* ctx, float threshold) {
 // Slab mode (SURVEY.md section 8e row 2; BASELINE config 5): one cloud, one slab of the x-major Morton key space per
 // GPU.  The per-rank pieces live here; the host driver (f3ps/slab.py) issues the exchanges between them on this
 // handle's stream: all-reduce of the bounding box and the key histogram, all-to-all of the points, all-gather of the
-// voxel slices, the normal slices and -- per expansion sweep -- the steal-table slices.
+// voxel slices and the normal slices.  From f3ps_seeds on, every rank runs the ordinary stages on the whole table.
 extern "C++" {
 namespace {
 template <typename KeyT>
@@ -1116,7 +1083,7 @@ int slab_route_typed(f3ps_ctx* ctx, PointLoader pl, const SlabSplitters& sp, int
 
 int f3ps_slab_reset(f3ps_ctx* ctx) {
     if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
-    ctx->slab_frame = false; ctx->slab_range = false; ctx->slab_expanding = false;
+    ctx->slab_frame = false; ctx->slab_range = false;
     ctx->progress = std::min(ctx->progress, (int)P_INPUT);
     return F3PS_OK;
 }
@@ -1200,22 +1167,13 @@ int f3ps_slab_route(f3ps_ctx* ctx, int world, const uint64_t* splitters, void* d
 // device arrays the driver exchanges in place (pointer, elements, bytes per element)
 int f3ps_slab_array(f3ps_ctx* ctx, int which, void** ptr, int64_t* n, int* elem_bytes) {
     if (!ctx || !ptr || !n || !elem_bytes) return F3PS_ERR_INVALID_ARGUMENT;
-    const int64_t V = ctx->V, L = (int64_t)ctx->S0 + 2;
-    const ExpandArgs& A = ctx->slab_A;
+    const int64_t V = ctx->V;
     switch (which) {
     case F3PS_SLAB_VOX_XYZ: *ptr = ctx->vox_xyz.p; *n = V; *elem_bytes = 16; break;
     case F3PS_SLAB_VOX_RGB: *ptr = ctx->vox_rgb.p; *n = V; *elem_bytes = 16; break;
     case F3PS_SLAB_VOX_KEY: *ptr = ctx->vox_key.p; *n = V; *elem_bytes = 8; break;
     case F3PS_SLAB_VOX_NORMAL: *ptr = ctx->vox_normal.p; *n = V; *elem_bytes = 16; break;
     case F3PS_SLAB_VOX_CURV: *ptr = ctx->vox_curv.p; *n = V; *elem_bytes = 4; break;
-    case F3PS_SLAB_STEAL: if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "no expansion in progress");
-        *ptr = A.st[ctx->slab_k & 1]; *n = V; *elem_bytes = 4; break;
-    case F3PS_SLAB_OWNER_NEXT: if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "no expansion in progress");
-        *ptr = A.owner[ctx->slab_cur ^ 1]; *n = V; *elem_bytes = 4; break;
-    case F3PS_SLAB_DIST: if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "no expansion in progress");
-        *ptr = A.dist[ctx->slab_cur]; *n = V; *elem_bytes = 4; break;
-    case F3PS_SLAB_COUNT: if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "no expansion in progress");
-        *ptr = A.count[(ctx->slab_k + 1) & 1]; *n = L; *elem_bytes = 4; break;     // tallies of the last sweep
     default: return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "unknown slab array");
     }
     return F3PS_OK;
@@ -1245,80 +1203,6 @@ int f3ps_slab_set_voxels(f3ps_ctx* ctx, const void* d_xyz, const void* d_rgb, co
     ctx->progress = P_VOXELS;
     return mark(ctx, 1);
 }
-
-// ---- K5 in slab mode: createSupervoxelHelpers, then per round {sweeps over the owned slice, round end}, then the tail ----
-int f3ps_slab_expand_begin(f3ps_ctx* ctx) {
-    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
-    int rc = need(ctx, P_SEEDS, "f3ps_slab_expand_begin"); if (rc) return rc;
-    if (!ctx->slab_range) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_expand_begin: not in slab mode");
-    cudaSetDevice(ctx->device);
-    rc = expand_prepare(ctx, ctx->slab_A); if (rc) return rc;
-    const ExpandArgs& A = ctx->slab_A;
-    ctx->slab_cur = 0; ctx->slab_k = 0; ctx->slab_sweeps = 0; ctx->slab_round = 0; ctx->slab_expanding = true;
-    if (ctx->V) {
-        LAUNCH(ctx, slab_expand_init_kernel, grid_for(ctx->V, 256), 256, 0, A);
-        if (ctx->S0) {
-            LAUNCH(ctx, slab_expand_seed_kernel, grid_for(ctx->S0, 256), 256, 0, A);
-            LAUNCH(ctx, slab_expand_phantom_kernel, grid_for(ctx->S0, 256), 256, 0, A);
-        }
-    }
-    return F3PS_OK;
-}
-
-// one sweep over [own_begin, own_end); *d_changed (device) = 1 if a steal-table entry of the slice moved.  Afterwards
-// F3PS_SLAB_STEAL is the table this sweep wrote: exchange its slices, all-reduce the flag (MAX), repeat until it is 0.
-int f3ps_slab_expand_sweep(f3ps_ctx* ctx, uint32_t* d_changed) {
-    if (!ctx || !d_changed) return F3PS_ERR_INVALID_ARGUMENT;
-    if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_expand_sweep: f3ps_slab_expand_begin has not run");
-    cudaSetDevice(ctx->device);
-    const ExpandArgs& A = ctx->slab_A;
-    F3PS_CUDA_OK(cudaMemsetAsync(d_changed, 0, 4, ctx->stream));
-    F3PS_CUDA_OK(cudaMemsetAsync(A.count[ctx->slab_k & 1], 0, ((size_t)ctx->S0 + 2) * 4, ctx->stream));
-    const unsigned nb = ctx->own_end - ctx->own_begin;
-    if (nb)
-        LAUNCH(ctx, slab_expand_sweep_kernel, grid_for(nb, kExpandThreads, kSMs * 2), kExpandThreads, 0, A, ctx->own_begin, ctx->own_end, ctx->slab_cur,
-               ctx->slab_k, d_changed);
-    ctx->slab_k++; ctx->slab_sweeps++;
-    return F3PS_OK;
-}
-
-// after the converged sweep of a round, with F3PS_SLAB_OWNER_NEXT slices exchanged and F3PS_SLAB_COUNT all-reduced (SUM):
-// helper lists, SupervoxelHelper::updateCentroid (every rank, whole cloud).  With zero expansion rounds call it once, without sweeps.
-int f3ps_slab_expand_round_end(f3ps_ctx* ctx) {
-    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
-    if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_expand_round_end: f3ps_slab_expand_begin has not run");
-    cudaSetDevice(ctx->device);
-    const ExpandArgs& A = ctx->slab_A;
-    const unsigned V = ctx->V, S0 = ctx->S0;
-    unsigned* cnt_final;
-    if (ctx->rounds > 0) { cnt_final = A.count[(ctx->slab_k + 1) & 1]; ctx->slab_cur ^= 1; }
-    else {
-        cnt_final = A.count[0];
-        if (V) LAUNCH(ctx, slab_expand_count0_kernel, grid_for(V, 256), 256, 0, A, ctx->slab_cur, cnt_final);
-    }
-    F3PS_CUDA_OK(cudaMemsetAsync(SC(xctl.cursor), 0, 4, ctx->stream));
-    if (V && S0) {
-        LAUNCH(ctx, slab_expand_alloc_kernel, grid_for(S0, 256), 256, 0, A, cnt_final);
-        LAUNCH(ctx, slab_expand_fill_kernel, grid_for(V, 256), 256, 0, A, ctx->slab_cur, ctx->slab_k);
-        LAUNCH(ctx, slab_expand_fold_kernel, grid_for((int64_t)S0 * 32, kExpandThreads, kSMs * 2), kExpandThreads, 0, A, cnt_final);
-    }
-    ctx->slab_round++;
-    return F3PS_OK;
-}
-
-// after the last round (F3PS_SLAB_DIST slices exchanged): clean labels, surviving helpers (makeSupervoxels)
-int f3ps_slab_expand_end(f3ps_ctx* ctx) {
-    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
-    if (!ctx->slab_expanding) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_expand_end: f3ps_slab_expand_begin has not run");
-    cudaSetDevice(ctx->device);
-    const ExpandArgs& A = ctx->slab_A;
-    const unsigned* cnt_final = ctx->rounds > 0 ? A.count[(ctx->slab_k + 1) & 1] : A.count[0];
-    if (ctx->V) LAUNCH(ctx, slab_expand_tail_kernel, 1 + grid_for(ctx->V, 1024, kSMs * 2), 1024, 0, A, ctx->slab_cur, cnt_final);
-    F3PS_CUDA_OK(cudaMemcpyAsync(SC(xctl.sweeps_total), &ctx->slab_sweeps, 4, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->slab_expanding = false;
-    return expand_finish(ctx);
-}
-
 
 int f3ps_merge_profile(f3ps_ctx* ctx, uint64_t cycles[32]) {
     if (!ctx || !cycles) return F3PS_ERR_INVALID_ARGUMENT;

@@ -104,10 +104,10 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() { unsigned long l
 // Active set: the result for n is a pure function of the round-start state and of the steal-table entries of its
 // NEIGHBOURS; when none of them moved in the previous sweep (chg_in), this sweep reproduces the previous one, whose owner /
 // distance are still in own1 / dst1 (same buffers for every sweep of a round) -- only the entry is carried over and the
-// helper sizes are tallied.  chg_in == nullptr (first sweep of a round, slab mode): everything is evaluated.
+// helper sizes are tallied.  chg_in == nullptr (first sweep of a round): everything is evaluated.
 __device__ __forceinline__ void expand_sweep_voxel(const ExpandArgs& A, const unsigned n, const unsigned* own0, const float* dst0,
         unsigned* own1, float* dst1, const unsigned* st_in, unsigned* st_out, unsigned* cnt, unsigned& any_change,
-        const unsigned char* chg_in = nullptr, unsigned char* chg_out = nullptr) {
+        const unsigned char* chg_in, unsigned char* chg_out) {
     const unsigned w0 = own0[n];
     float D = dst0[n];
     const unsigned st_n = st_in[n];
@@ -446,7 +446,6 @@ __global__ void __launch_bounds__(kExpandThreads, F3PS_EXPAND_MIN_BLOCKS) expand
 // driver runs one at a time).
 constexpr int kExpandClusterThreads = 1024;
 constexpr int kExpandClusterMax = 16;
-constexpr unsigned kExpandClusterMaxV = kExpandClusterThreads * kExpandClusterMax * 8u;    // <= 8 voxels per thread, else the cooperative grid
 __global__ void __launch_bounds__(kExpandClusterThreads, 1) expand_cluster_kernel(ExpandArgs A) {
     __shared__ ExpandSmem<kExpandClusterThreads> SM;
     expand_body<kExpandClusterThreads, true>(A, SM, blockIdx.x, gridDim.x);

@@ -4,11 +4,10 @@
 // (VoxelData::addPoint in input order, SupervoxelHelper::updateCentroid in idx order) keeps its order.
 //
 // The kernels here are the per-rank pieces between the exchanges; the exchanges themselves (NCCL all-reduce of
-// the bounding box / key histogram, all-to-all of the points, all-gather of voxel / steal-table slices) are issued
+// the bounding box / key histogram, all-to-all of the points, all-gather of voxel / normal slices) are issued
 // by the host driver on the same stream (f3ps/slab.py).
 #pragma once
 #include "kernels_vccs.cuh"
-#include "kernels_expand.cuh"
 
 namespace f3ps {
 
@@ -57,96 +56,6 @@ __global__ void __launch_bounds__(256) slab_pack_kernel(PointLoader pl, const un
         p.w = __uint_as_float(pl.rgba(i, p));
         out[j] = p;
     }
-}
-
-// ---- K5 in slab mode: the phases of expand_persistent_kernel as separate launches -------------------------------
-// (the grid barriers of the single-GPU kernel become stream order + the exchange of the slices the other ranks computed)
-__global__ void __launch_bounds__(256) slab_expand_init_kernel(ExpandArgs A) {
-    const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x, nthreads = gridDim.x * blockDim.x;
-    for (unsigned v = tid; v < A.V; v += nthreads) {
-        A.owner[0][v] = 0u; A.dist[0][v] = FLT_MAX; A.st[0][v] = kNoSteal; A.st[1][v] = kNoSteal; for (int s = 0; s < kPhSlots; ++s) A.phantom[(size_t)kPhSlots * v + s] = 0u;
-        A.owner[1][v] = 0u; A.dist[1][v] = FLT_MAX;
-    }
-    for (unsigned l = tid; l < A.S0 + 2; l += nthreads) {
-        A.cen.xyz[l] = make_float4(0, 0, 0, l >= 1 && l <= A.S0 ? 1.0f : 0.0f);
-        A.cen.rgb[l] = make_float4(0, 0, 0, 0); A.cen.nrm[l] = make_float4(0, 0, 0, 0);
-        A.phantom_leaf[l] = -1; A.count[0][l] = 0u; A.count[1][l] = 0u; A.off[l] = 0u;
-    }
-}
-__global__ void __launch_bounds__(256) slab_expand_seed_kernel(ExpandArgs A) {
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < A.S0; i += gridDim.x * blockDim.x) atomicMax(&A.owner[0][A.seeds[i]], i + 1u);
-}
-__global__ void __launch_bounds__(256) slab_expand_phantom_kernel(ExpandArgs A) {
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < A.S0; i += gridDim.x * blockDim.x) {
-        const unsigned u = (unsigned)A.seeds[i];
-        if ((A.owner[0][u] & kOwnMask) == i + 1u) continue;
-        bool placed = false;
-        for (int s = 0; s < kPhSlots && !placed; ++s) placed = atomicCAS(&A.phantom[(size_t)kPhSlots * u + s], 0u, i + 1u) == 0u;
-        if (!placed) atomicOr(&A.ctl->error, (unsigned)EXPAND_ERR_TRIPLE);
-        A.phantom_leaf[i + 1] = (int)u;
-        atomicOr(&A.owner[0][u], kOwnPhantom);
-    }
-}
-
-// one sweep over the voxels [begin, end) this rank owns; `changed` receives 1 when any steal-table entry moved
-__global__ void __launch_bounds__(kExpandThreads) slab_expand_sweep_kernel(ExpandArgs A, unsigned begin, unsigned end, int cur, unsigned k,
-                                                                           unsigned* __restrict__ changed) {
-    const unsigned* own0 = A.owner[cur]; const float* dst0 = A.dist[cur];
-    unsigned* own1 = A.owner[cur ^ 1]; float* dst1 = A.dist[cur ^ 1];
-    const unsigned* st_in = A.st[k & 1]; unsigned* st_out = A.st[(k + 1) & 1];
-    unsigned* cnt = A.count[k & 1];
-    unsigned any_change = 0;
-    for (unsigned n = begin + blockIdx.x * blockDim.x + threadIdx.x; n < end; n += gridDim.x * blockDim.x)
-        expand_sweep_voxel(A, n, own0, dst0, own1, dst1, st_in, st_out, cnt, any_change);
-    if (__syncthreads_or(any_change) && threadIdx.x == 0) atomicOr(changed, 1u);
-}
-
-// no expansion rounds: helper sizes straight from createSupervoxelHelpers (all voxels, every rank)
-__global__ void __launch_bounds__(256) slab_expand_count0_kernel(ExpandArgs A, int cur, unsigned* __restrict__ cnt) {
-    const unsigned* own = A.owner[cur];
-    for (unsigned n = blockIdx.x * blockDim.x + threadIdx.x; n < A.V; n += gridDim.x * blockDim.x) {
-        const unsigned w = own[n];
-        if (w & kOwnMask) atomicAdd(&cnt[w & kOwnMask], 1u);
-        if (w & kOwnPhantom) for (int s = 0; s < kPhSlots; ++s) { const unsigned h = A.phantom[(size_t)kPhSlots * n + s]; if (h) atomicAdd(&cnt[h], 1u); }
-    }
-}
-
-__global__ void __launch_bounds__(256) slab_expand_alloc_kernel(ExpandArgs A, const unsigned* __restrict__ cnt_final) {
-    const int lane = threadIdx.x & 31;
-    const unsigned gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-    for (unsigned base = gwarp * 32u; base < A.S0; base += nwarps * 32u) expand_alloc_warp(A, cnt_final, base, lane);
-}
-
-__global__ void __launch_bounds__(256) slab_expand_fill_kernel(ExpandArgs A, int cur, unsigned k) {
-    unsigned* own = A.owner[cur];
-    unsigned* st_a = A.st[0]; unsigned* st_b = A.st[1];
-    (void)k;
-    for (unsigned n = blockIdx.x * blockDim.x + threadIdx.x; n < A.V; n += gridDim.x * blockDim.x) {
-        expand_fill_voxel(A, own, n);
-        st_a[n] = kNoSteal; st_b[n] = kNoSteal;
-    }
-}
-
-__global__ void __launch_bounds__(kExpandThreads) slab_expand_fold_kernel(ExpandArgs A, const unsigned* __restrict__ cnt_final) {
-    __shared__ unsigned s_sorted[kExpandThreads / 32][32];
-    __shared__ float s_stage[kExpandThreads / 32][32][12];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const unsigned gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-    for (unsigned l = 1 + gwarp; l <= A.S0; l += nwarps) expand_fold_helper(A, cnt_final, l, lane, &s_sorted[wib][0], &s_stage[wib][0][0]);
-}
-
-__global__ void __launch_bounds__(1024) slab_expand_tail_kernel(ExpandArgs A, int cur, const unsigned* __restrict__ cnt_final) {
-    __shared__ unsigned s_warp[32];
-    __shared__ unsigned s_carry;
-    const unsigned S0 = A.S0;
-    const unsigned* own = A.owner[cur]; const float* dst = A.dist[cur];
-    if (blockIdx.x > 0) {
-        const unsigned tid = (blockIdx.x - 1) * blockDim.x + threadIdx.x, nthreads = (gridDim.x - 1) * blockDim.x;
-        for (unsigned n = tid; n < A.V; n += nthreads) { A.labels_out[n] = own[n] & kOwnMask; A.dist_out[n] = dst[n]; }
-        for (unsigned l = tid; l < S0 + 2; l += nthreads) A.seg_end[l] = (l >= 1 && l <= S0) ? A.off[l] + cnt_final[l] : 0u;
-        return;
-    }
-    expand_alive_scan(A, cnt_final, s_warp, &s_carry);
 }
 
 } // namespace f3ps

@@ -119,10 +119,6 @@ def lib():
         "f3ps_slab_route": (C.c_int, [vp, C.c_int, vp, vp, vp]),
         "f3ps_slab_array": (C.c_int, [vp, C.c_int, C.POINTER(vp), C.POINTER(i64), C.POINTER(C.c_int)]),
         "f3ps_slab_set_voxels": (C.c_int, [vp, vp, vp, vp, i64, i64, i64]),
-        "f3ps_slab_expand_begin": (C.c_int, [vp]),
-        "f3ps_slab_expand_sweep": (C.c_int, [vp, vp]),
-        "f3ps_slab_expand_round_end": (C.c_int, [vp]),
-        "f3ps_slab_expand_end": (C.c_int, [vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -143,8 +139,7 @@ EXPORTED = ["f3ps_create", "f3ps_destroy", "f3ps_last_error", "f3ps_version", "f
             "f3ps_get_level_point_labels", "f3ps_stage_ms", "f3ps_launch_count", "f3ps_merge_profile", "f3ps_merge_trace", "f3ps_expand_profile", "f3ps_test_rgb2lab",
             "f3ps_test_lab_ciede00", "f3ps_test_rgb_eucl", "f3ps_test_sort_pairs",
             "f3ps_merge_batch", "f3ps_set_expand_sharing", "f3ps_set_expand_kernel", "f3ps_refine", "f3ps_eval_thresholds", "f3ps_eval_label_pairs", "f3ps_slab_reset", "f3ps_slab_bbox", "f3ps_slab_set_frame", "f3ps_slab_keys", "f3ps_slab_route", "f3ps_slab_array",
-            "f3ps_slab_set_voxels", "f3ps_slab_expand_begin", "f3ps_slab_expand_sweep", "f3ps_slab_expand_round_end",
-            "f3ps_slab_expand_end"]
+            "f3ps_slab_set_voxels"]
 
 
 def _p(a):
@@ -230,7 +225,7 @@ class Segmenter:
     def set_merge_kernel(self, which): self._chk(self.L.f3ps_set_merge_kernel(self.h, which))
     def set_blocking_wait(self, on): self._chk(self.L.f3ps_set_blocking_wait(self.h, int(on)))
     def set_expand_kernel(self, which, cluster_ctas=0): self._chk(self.L.f3ps_set_expand_kernel(self.h, which, cluster_ctas))
-    def set_expand_sharing(self, ctas_per_frame, max_concurrent=1): self._chk(self.L.f3ps_set_expand_sharing(self.h, ctas_per_frame, max_concurrent))
+    def set_expand_sharing(self, ctas_per_frame, max_concurrent=0): self._chk(self.L.f3ps_set_expand_sharing(self.h, ctas_per_frame, max_concurrent))
     def extract(self): self._chk(self.L.f3ps_extract(self.h))
     def run(self, threshold=0.2): self._chk(self.L.f3ps_run(self.h, threshold))
     def sync(self): self._chk(self.L.f3ps_sync(self.h))
@@ -474,8 +469,7 @@ class Segmenter:
         return dict(zip(self.PERF_FIELDS, map(float, perf)))
 
     # ---- slab mode (per-rank pieces; f3ps/slab.py issues the exchanges between them) ----
-    SLAB_ARRAYS = {"vox_xyz": 0, "vox_rgb": 1, "vox_key": 2, "vox_normal": 3, "vox_curv": 4, "steal": 5, "owner_next": 6,
-                   "dist": 7, "count": 8}
+    SLAB_ARRAYS = {"vox_xyz": 0, "vox_rgb": 1, "vox_key": 2, "vox_normal": 3, "vox_curv": 4}
 
     def slab_reset(self): self._chk(self.L.f3ps_slab_reset(self.h))
     def slab_bbox(self, d_box8): self._chk(self.L.f3ps_slab_bbox(self.h, C.c_void_p(d_box8)))
@@ -500,11 +494,6 @@ class Segmenter:
 
     def slab_set_voxels(self, d_xyz, d_rgb, d_key, n_voxels, own_begin, own_end):
         self._chk(self.L.f3ps_slab_set_voxels(self.h, C.c_void_p(d_xyz), C.c_void_p(d_rgb), C.c_void_p(d_key), n_voxels, own_begin, own_end))
-
-    def slab_expand_begin(self): self._chk(self.L.f3ps_slab_expand_begin(self.h))
-    def slab_expand_sweep(self, d_changed): self._chk(self.L.f3ps_slab_expand_sweep(self.h, C.c_void_p(d_changed)))
-    def slab_expand_round_end(self): self._chk(self.L.f3ps_slab_expand_round_end(self.h))
-    def slab_expand_end(self): self._chk(self.L.f3ps_slab_expand_end(self.h))
 
     # ---- device self tests ----
     def test_rgb2lab(self, rgb255):

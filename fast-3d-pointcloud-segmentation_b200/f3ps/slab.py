@@ -14,9 +14,7 @@ Exchanges (all on the stream the handle runs on; NCCL over NVLink when the backe
       all-to-all of the points, 16 bytes each, to the rank owning their key range (stable: input order survives)
       all-gather of the voxel slices (40 bytes per voxel)                -> replicated voxel table
   K3  normals of the owned slice, all-gather of the slices (20 bytes per voxel)
-  K5  per sweep: the owned slice of the steal table (4 bytes per voxel) + a 4-byte convergence flag (MAX);
-      per round: owner words of the slice (4 bytes per voxel) + helper sizes (SUM)
-  K2 (hash + 27 probes), K4 (seed grid), the per-round helper lists / centroid folds and K6 run on the replicated
+  K2 (hash + 27 probes), K4 (seed grid), K5 (the expansion kernel of one handle) and K6 run on the replicated
   tables on every rank; K7 does not shard ("replicas only": one graph, strictly serial order) and is replayed by
   every rank, so every rank ends with the complete result and no broadcast is needed.
 """
@@ -129,37 +127,6 @@ class Comm:
                 self.dist.broadcast(part, src=r)
         return full
 
-    def gather_slices_flag(self, full, bounds, flag):
-        """gather_slices(full) + all-reduce MAX of the one-element `flag` in ONE collective: every rank contributes its
-        slice padded to the longest one with the flag appended (all-gather), the slices are copied into place.
-        Returns the reduced flag on the host."""
-        if not self.on or self.world == 1:
-            return int(flag.item())
-        if self.staged:
-            self.gather_slices(full, bounds)
-            self.all_reduce(flag, "max")
-            return int(flag.item())
-        torch = self.torch
-        width = full.shape[1]
-        lens = [int(bounds[r + 1] - bounds[r]) for r in range(self.world)]
-        cap = max(lens) * width + 1
-        key = (full.dtype, cap, full.device)
-        if getattr(self, "_gs_key", None) != key:
-            self._gs_send = torch.empty(cap, dtype=full.dtype, device=full.device)
-            self._gs_recv = torch.empty((self.world, cap), dtype=full.dtype, device=full.device)
-            self._gs_key = key
-        send, recv = self._gs_send, self._gs_recv
-        lo, hi = int(bounds[self.rank]), int(bounds[self.rank + 1])
-        if hi > lo:
-            send[:(hi - lo) * width].copy_(full[lo:hi].reshape(-1))
-        send[cap - 1:cap].copy_(flag.view(full.dtype))
-        self.dist.all_gather_into_tensor(recv, send)
-        self.bytes_moved += cap * full.element_size() * (self.world - 1)
-        for r in range(self.world):
-            if r != self.rank and lens[r]:
-                full[int(bounds[r]):int(bounds[r + 1])].copy_(recv[r, :lens[r] * width].view(lens[r], width))
-        return int(recv[:, cap - 1].max().item())
-
     def all_to_all_rows(self, send, send_counts, recv_counts):
         """send: [n, k] rows grouped by destination; returns [sum(recv_counts), k] rows grouped by source rank."""
         torch = self.torch
@@ -204,9 +171,7 @@ class SlabSegmenter:
 
     TOP_BITS = 12
 
-    SHARD_EXPAND_MIN_V = 4_000_000      # voxels: below this the per-sweep exchange costs more than sharding the sweeps saves
-
-    def __init__(self, comm, device=0, vccs=None, merge=None, shard_expand=None):
+    def __init__(self, comm, device=0, vccs=None, merge=None):
         import torch
         self.torch = torch
         self.comm = comm
@@ -218,10 +183,6 @@ class SlabSegmenter:
         self.seg.set_merge_params(**(merge or {}))
         self.info = {}
         self._views = {}
-        # K5: None = by size (sweeps sharded over the slabs with a steal-table exchange per sweep when V >= SHARD_EXPAND_MIN_V, else
-        # every rank runs the persistent expansion kernel on the replicated voxel table: measured on the 50 M-point scan, V = 0.6 M:
-        # 8.8 ms replicated against 13.9 / 18.0 / 37.6 ms sharded over 2 / 4 / 8 GPUs); True / False force it (tests run both)
-        self.shard_expand = shard_expand
 
     def close(self):
         self.seg.close()
@@ -310,38 +271,9 @@ class SlabSegmenter:
             tick("normals")
             seg.seeds()
             tick("seeds")
-            # ---- K5: sweeps over the owned slice, steal table exchanged after every sweep -- or, for a voxel table too small for
-            #      that to pay, the single-GPU persistent kernel on the replicated table (identical results, no exchange) ----
-            shard = self.shard_expand if self.shard_expand is not None else (comm.world > 1 and V >= self.SHARD_EXPAND_MIN_V)
-            sweeps = 0
-            rounds = 0
-            if not shard:
-                seg.expand()
-                sweeps = int(seg.counts().sweeps)
-            else:
-                seg.slab_expand_begin()
-                rounds = int(seg.counts().rounds)
-            flag = torch.zeros(1, dtype=torch.int32, device=self.device)
-            for _ in range(rounds):
-                for s in range(33):
-                    if s == 32:
-                        raise binding.F3psError("expansion fixed point not reached within 32 sweeps")
-                    seg.slab_expand_sweep(flag.data_ptr())
-                    sweeps += 1
-                    # the slices of the steal table this sweep wrote + the convergence flag, one collective
-                    changed = comm.gather_slices_flag(self._view("steal", torch.int32), vb, flag) if V else 0
-                    if changed == 0:
-                        break
-                if V:
-                    comm.gather_slices(self._view("owner_next", torch.int32), vb)
-                comm.all_reduce(self._view("count", torch.int32), "sum")
-                seg.slab_expand_round_end()
-            if shard:
-                if rounds == 0:
-                    seg.slab_expand_round_end()
-                elif V:
-                    comm.gather_slices(self._view("dist", torch.float32), vb)
-                seg.slab_expand_end()
+            # ---- K5 on the replicated table: the kernel of one handle, no exchange ----
+            seg.expand()
+            sweeps = int(seg.counts().sweeps)
             tick("expand")
             # ---- K6, K7 on the replicated tables ----
             seg.graph()

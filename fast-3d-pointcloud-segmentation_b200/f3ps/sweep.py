@@ -91,7 +91,9 @@ class BatchPool:
     kernels; a grid has no such cap.  Two handle sets alternate, so the front stages of group g+1 overlap the merge of group g.
     Results are those of Segmenter.run on every frame, in frame order."""
 
-    def __init__(self, batch=64, workers=None, device=0, vccs=None, merge=None, threshold=0.2, expand_ctas=0, sms=148, expand_cluster=8):
+    def __init__(self, batch=64, workers=None, device=0, vccs=None, merge=None, threshold=0.2, expand_ctas=0, expand_cluster=8):
+        if expand_ctas > 0:
+            raise ValueError("expand_ctas must be <= 0: -n caps K5's cooperative grid at n CTAs")
         from . import binding
         import os
         import threading
@@ -111,12 +113,8 @@ class BatchPool:
                     # by side -- cooperative launches run one at a time).  Measured on C2, groups of 96: 8 CTAs 427 Mpoints/s,
                     # cooperative grid capped at 24 CTAs 416; 1-2 CTAs per frame lose (the 32 hardware queues cap long kernels)
                     s.set_expand_kernel(2, expand_cluster)
-                elif expand_ctas and expand_ctas < 0:
-                    s.set_expand_sharing(-expand_ctas, 0)            # cooperative launch, grid capped: more frames side by side
                 elif expand_ctas:
-                    # optional (measured: no gain, K5 costs ~60 SM-ms per VGA frame either way): K5 as small ordinary grids: the merge grid of a group holds `batch` SMs for its whole duration, the
-                    # expansion kernels in flight must fit the rest (their software barrier needs co-residency)
-                    s.set_expand_sharing(expand_ctas, max(1, (sms - min(batch, sms - expand_ctas)) // expand_ctas))
+                    s.set_expand_sharing(-expand_ctas, 0)            # cooperative launch, grid capped: more frames side by side
         self.segs = self.sets[0] + self.sets[1]
         self.threshold = threshold
         self._threading = threading

@@ -17,7 +17,6 @@ namespace f3ps_host {
 
 namespace {
 constexpr int kTopBits = 12;
-constexpr int64_t kShardExpandMinV = 4000000;     // voxels: below this the per-sweep exchange costs more than sharding the sweeps saves
 
 struct Fail : std::runtime_error { int code; Fail(int c, const std::string& m) : std::runtime_error(m), code(c) {} };
 void cu(cudaError_t e, const char* what) { if (e != cudaSuccess) throw Fail(F3PS_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e)); }
@@ -144,11 +143,10 @@ void SlabRun::rank_main(int rank, const SlabShare& share, const SlabParams& p) {
         info.n_local = n_local;
         ok(f3ps_set_input(ctx, share.points, n_local, share.stride, share.on_device ? 1 : 0), "f3ps_set_input");
         // ---- K1a: the frame of the whole cloud (order-preserving encoded box: MIN of 3 words, MAX of 4) ----
-        uint32_t* d_small = (uint32_t*)small.ensure(((size_t)8 + ((size_t)1 << kTopBits) + 4) * 4 + (size_t)world * (size_t)world * 8 + 64);
+        uint32_t* d_small = (uint32_t*)small.ensure(((size_t)8 + ((size_t)1 << kTopBits)) * 4 + (size_t)world * (size_t)world * 8 + 64);
         uint32_t* d_box = d_small;
         uint32_t* d_hist = d_small + 8;
-        uint32_t* d_flag = d_hist + ((size_t)1 << kTopBits);
-        int64_t* d_mat = (int64_t*)(d_flag + 4);
+        int64_t* d_mat = (int64_t*)(d_hist + ((size_t)1 << kTopBits));
         cu(cudaMemsetAsync(d_box, 0, 32, st), "memset");
         ok(f3ps_slab_bbox(ctx, d_box), "f3ps_slab_bbox");
         all_reduce(d_box, 3, ncclUint32, ncclMin, 4);
@@ -237,44 +235,10 @@ void SlabRun::rank_main(int rank, const SlabShare& share, const SlabParams& p) {
         tick("normals");
         ok(f3ps_seeds(ctx), "f3ps_seeds");
         tick("seeds");
-        // ---- K5: sweeps over the owned slice with the steal table exchanged after every sweep -- or, for a voxel table too small
-        //      for that to pay, the single-GPU persistent kernel on the replicated table (identical results, no exchange) ----
-        const bool shard = p.shard_expand >= 0 ? p.shard_expand != 0 : (world > 1 && V >= kShardExpandMinV);
-        int sweeps = 0, rounds = 0;
-        if (!shard) {
-            ok(f3ps_expand(ctx), "f3ps_expand");
-            ok(f3ps_get_counts(ctx, &c), "f3ps_get_counts"); sweeps = c.sweeps;
-        } else {
-            ok(f3ps_slab_expand_begin(ctx), "f3ps_slab_expand_begin");
-            ok(f3ps_get_counts(ctx, &c), "f3ps_get_counts"); rounds = c.rounds;
-        }
-        for (int round = 0; round < rounds; ++round) {
-            for (int s = 0;; ++s) {
-                if (s == 32) throw Fail(F3PS_ERR_CAPACITY, "expansion fixed point not reached within 32 sweeps");
-                cu(cudaMemsetAsync(d_flag, 0, 4, st), "memset flag");
-                ok(f3ps_slab_expand_sweep(ctx, d_flag), "f3ps_slab_expand_sweep");
-                ++sweeps;
-                uint32_t changed = 0;
-                if (V) {                              // the slices of the steal table this sweep wrote + the convergence flag
-                    void* ptr; int64_t n; int eb;
-                    slab_array(F3PS_SLAB_STEAL, ptr, n, eb); gather_slices(ptr, vb, (size_t)eb);
-                    all_reduce(d_flag, 1, ncclUint32, ncclMax, 4);
-                    cu(cudaMemcpyAsync(&changed, d_flag, 4, cudaMemcpyDeviceToHost, st), "memcpy flag");
-                    cu(cudaStreamSynchronize(st), "sync");
-                }
-                if (!changed) break;
-            }
-            void* ptr; int64_t n; int eb;
-            if (V) { slab_array(F3PS_SLAB_OWNER_NEXT, ptr, n, eb); gather_slices(ptr, vb, (size_t)eb); }
-            slab_array(F3PS_SLAB_COUNT, ptr, n, eb); all_reduce(ptr, (size_t)n, ncclUint32, ncclSum, 4);
-            ok(f3ps_slab_expand_round_end(ctx), "f3ps_slab_expand_round_end");
-        }
-        if (shard) {
-            if (rounds == 0) ok(f3ps_slab_expand_round_end(ctx), "f3ps_slab_expand_round_end");
-            else if (V) { void* ptr; int64_t n; int eb; slab_array(F3PS_SLAB_DIST, ptr, n, eb); gather_slices(ptr, vb, (size_t)eb); }
-            ok(f3ps_slab_expand_end(ctx), "f3ps_slab_expand_end");
-        }
-        info.sweeps = sweeps;
+        // ---- K5 on the replicated table: the kernel of one handle, no exchange ----
+        ok(f3ps_expand(ctx), "f3ps_expand");
+        ok(f3ps_get_counts(ctx, &c), "f3ps_get_counts");
+        info.sweeps = c.sweeps;
         tick("expand");
         // ---- K6, K7 on the replicated tables: K7 does not shard ("replicas only"), every rank replays it ----
         ok(f3ps_graph(ctx), "f3ps_graph");

@@ -24,7 +24,6 @@ struct SlabParams {
     int bins = 500;
     float threshold = 0.2f;
     bool merge = true;
-    int shard_expand = -1;            // K5: -1 = by size (sharded sweeps with a per-sweep exchange only for tables >= 4 M voxels), 0 / 1 force it
 };
 
 // one rank's share of the cloud: host memory, or (on_device) memory of that rank's GPU -- the scans it recorded, already in HBM

@@ -1,7 +1,7 @@
 // slab_selftest -- slab mode from C++ over NCCL (slab_host.h) against ONE handle processing the whole cloud: a synthetic room scan
 // is cut into `gpus` contiguous shares (as if every GPU had recorded some of the scan positions), SlabRun segments it, and every
 // rank's voxel labels / distances, merge log and labelled cloud must equal the single handle's bit for bit.
-// usage: slab_selftest [--gpus N] [--points P] [--shard-expand -1|0|1] [--voxel v] [--seed s] [--threshold t] [--device-shares 0|1]
+// usage: slab_selftest [--gpus N] [--points P] [--voxel v] [--seed s] [--threshold t] [--device-shares 0|1]
 // (--device-shares 1: every rank's share is uploaded to its GPU first, as if the scans were already in HBM; the timed run starts from there)
 // prints one JSON line (stage ms = max over ranks); exit code 0 = identical.
 #include <cuda_runtime.h>
@@ -70,18 +70,17 @@ template <typename T> bool same(const std::vector<T>& a, const std::vector<T>& b
 }  // namespace
 
 int main(int argc, char** argv) {
-    int gpus = 0, shard = -1, device_shares = 0; int64_t n = 2000000; uint64_t seed = 7;
+    int gpus = 0, device_shares = 0; int64_t n = 2000000; uint64_t seed = 7;
     f3ps_host::SlabParams p; p.voxel_res = 0.01f; p.seed_res = 0.1f; p.geometric_distance = 1; p.merging = 1;      // BASELINE config 5: -v 0.01 -s 0.1 --CVX --AL
     for (int i = 1; i + 1 < argc; i += 2) {
         const std::string k = argv[i];
         if (k == "--gpus") gpus = atoi(argv[i + 1]); else if (k == "--points") n = atoll(argv[i + 1]);
-        else if (k == "--shard-expand") shard = atoi(argv[i + 1]); else if (k == "--voxel") p.voxel_res = (float)atof(argv[i + 1]);
+        else if (k == "--voxel") p.voxel_res = (float)atof(argv[i + 1]);
         else if (k == "--seed-res") p.seed_res = (float)atof(argv[i + 1]); else if (k == "--seed") seed = (uint64_t)atoll(argv[i + 1]);
         else if (k == "--threshold") p.threshold = (float)atof(argv[i + 1]);
         else if (k == "--device-shares") device_shares = atoi(argv[i + 1]);
         else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
     }
-    p.shard_expand = shard;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { fprintf(stderr, "slab_selftest: no CUDA device\n"); return 2; }
     if (gpus <= 0 || gpus > ndev) gpus = ndev;
@@ -125,9 +124,9 @@ int main(int argc, char** argv) {
         bytes = std::max(bytes, run.info(r).bytes_exchanged);
     }
     printf("{\"tool\": \"slab_selftest\", \"host\": \"c++/nccl\", \"gpus\": %d, \"points\": %lld, \"V\": %lld, \"S\": %d, \"E\": %d, \"merges\": %d, \"sweeps\": %d, "
-           "\"sharded_expand\": %s, \"device_shares\": %s, \"identical_to_one_handle\": %s, \"bytes_exchanged_max_rank\": %llu, \"one_handle_total_ms\": %.3f, \"stage_ms\": {",
+           "\"device_shares\": %s, \"identical_to_one_handle\": %s, \"bytes_exchanged_max_rank\": %llu, \"one_handle_total_ms\": %.3f, \"stage_ms\": {",
            gpus, (long long)n, (long long)run.info(0).V, ref.c.n_supervoxels, ref.c.n_edges, ref.c.n_merges, run.info(0).sweeps,
-           (shard >= 0 ? shard != 0 : (gpus > 1 && run.info(0).V >= 4000000)) ? "true" : "false", device_shares ? "true" : "false", identical ? "true" : "false", (unsigned long long)bytes, one_total);
+           device_shares ? "true" : "false", identical ? "true" : "false", (unsigned long long)bytes, one_total);
     for (size_t i = 0; i < order.size(); ++i) printf("%s\"%s\": %.3f", i ? ", " : "", order[i].c_str(), ms[order[i]]);
     printf("}}\n");
     if (!identical) fprintf(stderr, "slab_selftest: differs from the single handle on:%s\n", diff.c_str());

@@ -105,12 +105,10 @@ int f3ps_seeds(f3ps_ctx* ctx);      /* K4 selectInitialSupervoxelSeeds */
 int f3ps_expand(f3ps_ctx* ctx);     /* K5 expandSupervoxels */
 int f3ps_graph(f3ps_ctx* ctx);      /* K6 makeSupervoxels + getSupervoxelAdjacency + set_initialstate + init_weights */
 int f3ps_merge(f3ps_ctx* ctx, float threshold); /* K7 Clustering::cluster(threshold): restarts from the initial state */
-/* K5 launch mode.  ctas_per_frame = 0 (default): one cooperative launch over the whole GPU -- lowest latency for one frame, but
- * cooperative launches of concurrent frames run one at a time.  ctas_per_frame > 0: an ordinary grid of that many CTAs, at most
- * max_concurrent of them in flight on the device (process-wide gate); the caller guarantees that ctas_per_frame * max_concurrent
- * CTAs fit the SMs no long-running kernel occupies (the software grid barrier needs a launch's CTAs co-resident).
- * max_concurrent = 0 with ctas_per_frame > 0: still a cooperative launch, its grid capped at ctas_per_frame (a sweep trades the
- * latency of one frame for more frames side by side; the driver keeps guaranteeing co-residency). */
+/* Grid of K5's cooperative launch.  ctas_per_frame = 0 (default): the whole GPU -- lowest latency for one frame, but
+ * cooperative launches of concurrent frames run one at a time.  ctas_per_frame > 0: the grid is capped at that many CTAs (a
+ * sweep trades the latency of one frame for more frames side by side).  max_concurrent must be 0; other values, and
+ * ctas_per_frame outside 0..296, are F3PS_ERR_INVALID_ARGUMENT.  Same results from every setting. */
 int f3ps_set_expand_sharing(f3ps_ctx* ctx, int ctas_per_frame, int max_concurrent);
 /* pcl::SupervoxelClustering::refineSupervoxels(num_itr, clusters) (/root/reference/src/supervoxel_clustering.cpp:369-371) on the
  * result of f3ps_expand / f3ps_extract: per iteration SupervoxelHelper::refineNormals (voxel normals from the neighbours of the
@@ -119,8 +117,8 @@ int f3ps_set_expand_sharing(f3ps_ctx* ctx, int ctas_per_frame, int max_concurren
  * return the refined state; the supervoxel graph is rebuilt by the next f3ps_graph / f3ps_merge.  Calling it before f3ps_expand
  * is F3PS_ERR_LOGIC (PCL: "Supervoxels must be extracted before they can be refined"). */
 int f3ps_refine(f3ps_ctx* ctx, int num_itr);
-/* which K5 kernel f3ps_expand launches: 0 / 1 = the cooperative grid over the whole GPU (lowest latency for one frame: 0.8 ms on a
- * VGA frame, but ~50 SM-ms of mostly barrier waiting; f3ps_set_expand_sharing applies to it), 2 = ONE thread-block cluster per frame
+/* which K5 kernel f3ps_expand launches: 0 / 1 = the cooperative grid (lowest latency for one frame: 0.8 ms on a VGA frame, but
+ * ~50 SM-ms of mostly barrier waiting; f3ps_set_expand_sharing may cap it), 2 = ONE thread-block cluster per frame
  * (cluster_ctas = 1..16 CTAs of 1024 threads meeting at the hardware cluster barrier; 0 = two voxels per thread, at most 16): the
  * expansion is instruction-bound, so a small cluster does the same work in ~17 SM-ms and leaves the other SMs to the frames next to
  * it -- what directory sweeps use.  Same results from every choice.
@@ -226,16 +224,10 @@ int f3ps_get_level_point_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacit
  *   f3ps_set_input(local points) -> f3ps_slab_bbox -> [all-reduce MIN/MAX] -> f3ps_slab_set_frame -> f3ps_slab_keys
  *   -> [all-reduce SUM histogram; choose splitters] -> f3ps_slab_route -> [all-to-all points] -> f3ps_set_input(received,
  *   stride 16, on device) -> f3ps_voxelize -> [all-gather voxel slices] -> f3ps_slab_set_voxels -> f3ps_neighbors ->
- *   f3ps_normals (owned slice) -> [all-gather normal slices] -> f3ps_seeds -> f3ps_slab_expand_begin -> per round {
- *   f3ps_slab_expand_sweep -> [all-gather steal slices, all-reduce MAX flag] until 0; [all-gather owner slices, all-reduce SUM
- *   counts]; f3ps_slab_expand_round_end } -> [all-gather distance slices] -> f3ps_slab_expand_end -> f3ps_graph -> f3ps_merge.
- * K7 does not shard (strictly serial order over one graph): every rank replays it on the gathered graph. */
+ *   f3ps_normals (owned slice) -> [all-gather normal slices] -> f3ps_seeds -> f3ps_expand -> f3ps_graph -> f3ps_merge.
+ * From f3ps_seeds on every rank works on the whole gathered table; K7 does not shard (strictly serial order over one graph). */
 enum f3ps_slab_array_id {
-    F3PS_SLAB_VOX_XYZ = 0, F3PS_SLAB_VOX_RGB = 1, F3PS_SLAB_VOX_KEY = 2, F3PS_SLAB_VOX_NORMAL = 3, F3PS_SLAB_VOX_CURV = 4,
-    F3PS_SLAB_STEAL = 5,       /* steal table written by the last sweep [V] u32 */
-    F3PS_SLAB_OWNER_NEXT = 6,  /* owner words the converged sweep wrote [V] u32 */
-    F3PS_SLAB_DIST = 7,        /* stored distances of the current round state [V] f32 */
-    F3PS_SLAB_COUNT = 8        /* helper sizes tallied by the last sweep over the owned slice [S0 + 2] u32 */
+    F3PS_SLAB_VOX_XYZ = 0, F3PS_SLAB_VOX_RGB = 1, F3PS_SLAB_VOX_KEY = 2, F3PS_SLAB_VOX_NORMAL = 3, F3PS_SLAB_VOX_CURV = 4
 };
 int f3ps_slab_reset(f3ps_ctx* ctx);
 int f3ps_slab_bbox(f3ps_ctx* ctx, uint32_t* d_box8);
@@ -245,10 +237,6 @@ int f3ps_slab_route(f3ps_ctx* ctx, int world, const uint64_t* splitters, void* d
 int f3ps_slab_array(f3ps_ctx* ctx, int which, void** ptr, int64_t* n, int* elem_bytes);
 int f3ps_slab_set_voxels(f3ps_ctx* ctx, const void* d_xyz, const void* d_rgb, const void* d_key, int64_t n_voxels,
                          int64_t own_begin, int64_t own_end);
-int f3ps_slab_expand_begin(f3ps_ctx* ctx);
-int f3ps_slab_expand_sweep(f3ps_ctx* ctx, uint32_t* d_changed);
-int f3ps_slab_expand_round_end(f3ps_ctx* ctx);
-int f3ps_slab_expand_end(f3ps_ctx* ctx);
 
 /* ---- "next" row f1: the auto-threshold sweep ------------------------------------------------------------------------
  * Clustering::all_thresh (clustering.cpp:691-729) with Testing::eval_performance (testing.cpp:239-362) from ONE merge replay:

@@ -183,8 +183,8 @@ def test_phantom_seed_leaves(gpu, oracle_mod, seed, w, h):
 @pytest.mark.parametrize("seed,w,h", [(11, 160, 120), (52, 160, 120), (20020, 640, 480)], ids=["small", "phantom", "vga"])
 def test_expand_cluster_kernel_equals_cooperative_grid(gpu, oracle_mod, seed, w, h):
     """K5 has two launch shapes (f3ps_set_expand_kernel): the cooperative grid over the GPU (software grid barrier) and ONE
-    thread-block cluster per frame (hardware cluster barrier; what sweeps use).  Every cluster size gives the cooperative
-    grid's arrays bit for bit, and those are the oracle's."""
+    thread-block cluster per frame (hardware cluster barrier; what sweeps use).  Every cluster size, and the cooperative grid
+    capped by f3ps_set_expand_sharing, gives the cooperative grid's arrays bit for bit, and those are the oracle's."""
     pts = gpu.synth.make_frame(seed=seed, width=w, height=h)
     g, o = run_both(gpu, oracle_mod, pts, AL, 0.2, merge_impl=1)
     assert_parity(g, o, STAGE_ARRAYS)
@@ -198,8 +198,14 @@ def test_expand_cluster_kernel_equals_cooperative_grid(gpu, oracle_mod, seed, w,
     g.set_expand_kernel(1, 0); g.set_input(pts); g.run(0.2)
     for n in names:
         assert same(ref[n], g.array(n)), ("cooperative", n)
+    g.set_expand_sharing(24, 0); g.set_input(pts); g.run(0.2)      # the cooperative grid capped at 24 CTAs (BatchPool, expand_ctas=-24)
+    for n in names:
+        assert same(ref[n], g.array(n)), ("cooperative, 24 CTAs", n)
     with pytest.raises(ValueError):                      # F3PS_ERR_INVALID_ARGUMENT
         g.set_expand_kernel(2, 17)
+    with pytest.raises(ValueError):                      # max_concurrent != 0: K5 only runs as a cooperative grid or one cluster
+        g.set_expand_sharing(24, 4)
+    g.set_expand_sharing(0, 0)
 
 
 @pytest.mark.parametrize("seed,w,h,itr", [(11, 160, 120, 3), (52, 160, 120, 2), (20020, 640, 480, 3)], ids=["small", "phantom", "vga"])

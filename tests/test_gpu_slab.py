@@ -30,7 +30,7 @@ def _cloud(case):
     raise KeyError(case)
 
 
-def _worker(rank, world, port, case, shard, q):
+def _worker(rank, world, port, case, q):
     try:
         os.environ["MASTER_ADDR"] = "127.0.0.1"
         os.environ["MASTER_PORT"] = str(port)
@@ -48,7 +48,7 @@ def _worker(rank, world, port, case, shard, q):
         ref.set_vccs_params(**vccs); ref.set_merge_params(**merge)
         ref.set_input(pts); ref.run(thr)
         comm = slab.Comm(dist, torch)
-        ss = slab.SlabSegmenter(comm, device=0, vccs=vccs, merge=merge, shard_expand=shard)
+        ss = slab.SlabSegmenter(comm, device=0, vccs=vccs, merge=merge)
         info = ss.run(mine, thr)
         bad = []
         for name in ARRAYS:
@@ -73,15 +73,13 @@ def _worker(rank, world, port, case, shard, q):
         q.put((rank, ["exception: %s\n%s" % (e, traceback.format_exc())], None, 0, 0, 0, 0))
 
 
-@pytest.mark.parametrize("case,world,shard", [("small", 2, True), ("small", 3, True), ("vga_eq", 2, True), ("nt_rgb", 4, True), ("small", 2, None)],
-                         ids=["small-2", "small-3", "vga_eq-2", "nt_rgb-4", "small-2-replicated-k5"])
-def test_slab_equals_single_handle(case, world, shard):
-    """shard = True: K5's sweeps sharded over the slabs with the per-sweep exchange (what a voxel table of >= 4 M voxels gets);
-    None: the size rule, which for these clouds runs the persistent expansion kernel on the replicated table."""
+@pytest.mark.parametrize("case,world", [("small", 2), ("small", 3), ("vga_eq", 2), ("vga_eq", 3), ("nt_rgb", 4)],
+                         ids=["small-2ranks", "small-3ranks-empty-share", "vga_eq-2ranks", "vga_eq-3ranks", "nt_rgb-4ranks"])
+def test_slab_equals_single_handle(case, world):
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
-    procs = [ctx.Process(target=_worker, args=(r, world, port, case, shard, q)) for r in range(world)]
+    procs = [ctx.Process(target=_worker, args=(r, world, port, case, q)) for r in range(world)]
     for p in procs:
         p.start()
     res = sorted(q.get(timeout=600) for _ in range(world))

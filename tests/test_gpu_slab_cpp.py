@@ -26,16 +26,16 @@ def selftest():
     return exe
 
 
-@pytest.mark.parametrize("shard", [1, 0], ids=["sharded_sweeps", "replicated_expand"])
-def test_cpp_nccl_slab_mode_equals_one_handle(selftest, shard):
+@pytest.mark.parametrize("device_shares", [1, 0], ids=["device_shares", "host_shares"])
+def test_cpp_nccl_slab_mode_equals_one_handle(selftest, device_shares):
     import torch
     gpus = min(2, torch.cuda.device_count())
-    out = subprocess.run([selftest, "--gpus", str(gpus), "--points", "400000", "--shard-expand", str(shard), "--device-shares", str(shard)],
-                         capture_output=True, text=True, timeout=600)   # (sharded sweeps from device-resident shares, the replicated expansion from host memory)
+    out = subprocess.run([selftest, "--gpus", str(gpus), "--points", "400000", "--device-shares", str(device_shares)],
+                         capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stdout + out.stderr
     rec = json.loads(out.stdout.strip().splitlines()[-1])
     assert rec["identical_to_one_handle"] is True and rec["gpus"] == gpus
-    assert rec["V"] > 10000 and rec["merges"] > 10 and rec["sharded_expand"] == bool(shard)
+    assert rec["V"] > 10000 and rec["merges"] > 10 and rec["device_shares"] == bool(device_shares)
 
 
 def test_cli_slabs_prints_the_same_merge_sequence(selftest, small_frame, tmp_path):
