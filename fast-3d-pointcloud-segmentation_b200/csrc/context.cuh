@@ -123,10 +123,12 @@ struct f3ps_ctx {
     cudaEvent_t ev_batch = nullptr;    // f3ps_merge_batch: set-up done / grid done
     cudaEvent_t ev_wait = nullptr;     // blocking-sync event for sweeps (f3ps_set_blocking_wait)
     bool blocking_wait = false;
-    // slab mode (f3ps_slab_*): injected global frame, owned voxel range
+    // slab mode (f3ps_slab_*): injected global frame, histogram binning of f3ps_slab_keys (bin = key >> slab_shift,
+    // 1 << slab_bits bins; 0 bits: keys have not run), owned voxel range
     bool slab_frame = false; f3ps::FrameParams slab_fp{};
+    int slab_bits = 0, slab_shift = 0;
     bool slab_range = false; unsigned own_begin = 0, own_end = 0;
-    f3ps::DevBuf slab_dest, slab_tot;
+    f3ps::DevBuf slab_dest, slab_tot, slab_spare;   // slab_spare: this rank's voxel slice while f3ps_slab_set_voxels moves it
     f3ps::DevBuf ev_dense, ev_truth, ev_table;   // f3ps_eval_thresholds, f3ps_eval_label_pairs
     // segmentation levels (f3ps_merge_levels; every merge records its own threshold as the one level).  The tables are built on
     // the first getter call after the merge: forest, per-level merge counts and per-supervoxel labels, then the voxel table.

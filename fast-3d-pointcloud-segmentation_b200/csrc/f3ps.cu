@@ -1050,9 +1050,10 @@ int f3ps_run(f3ps_ctx* ctx, float threshold) {
 
 // =====================================================================================================
 // Slab mode (SURVEY.md section 8e row 2; BASELINE config 5): one cloud, one slab of the x-major Morton key space per
-// GPU.  The per-rank pieces live here; the host driver (f3ps/slab.py) issues the exchanges between them on this
-// handle's stream: all-reduce of the bounding box and the key histogram, all-to-all of the points, all-gather of the
-// voxel slices and the normal slices.  From f3ps_seeds on, every rank runs the ordinary stages on the whole table.
+// GPU.  The per-rank pieces live here, the splitter rule and the assembly of the replicated voxel table included; the host
+// drivers (f3ps/slab.py, host/slab_host.cpp) issue only the exchanges between them on this handle's stream: all-reduce of
+// the bounding box and the key histogram, all-to-all of the points, all-gather of the voxel slices and the normal slices.
+// From f3ps_seeds on, every rank runs the ordinary stages on the whole table.
 extern "C++" {
 namespace {
 template <typename KeyT>
@@ -1117,41 +1118,64 @@ int f3ps_slab_set_frame(f3ps_ctx* ctx, const uint32_t* d_box8) {
     F3PS_CUDA_OK(cudaMemcpyAsync(SC(fp.any_finite), d_box8 + 6, 4, cudaMemcpyDeviceToDevice, ctx->stream));
     LAUNCH(ctx, frame_setup_kernel, 1, 1, 0, SC(fp), ctx->vp.voxel_res);
     rc = pull_scalars(ctx); if (rc) return rc;
-    ctx->slab_fp = ctx->h_sc->fp; ctx->slab_frame = true;
+    ctx->slab_fp = ctx->h_sc->fp; ctx->slab_frame = true; ctx->slab_bits = 0;
     ctx->depth = ctx->slab_fp.depth;
     if (ctx->depth > 21) return ctx_fail(ctx, F3PS_ERR_CAPACITY, "adjacency octree depth > 21");
     ctx->key64 = 3 * ctx->depth > 32;
     return F3PS_OK;
 }
 
-// Morton keys of this rank's valid points + histogram of their top `top_bits` bits (d_hist: 1 << top_bits counters, device);
-// *used_bits / *shift describe the binning: bin = key >> shift, min(top_bits, 3 * depth) bits
-int f3ps_slab_keys(f3ps_ctx* ctx, int top_bits, uint32_t* d_hist, int* used_bits, int* shift_out) {
+// Morton keys of this rank's valid points + histogram of their top `top_bits` bits (d_hist: 1 << top_bits counters, device).
+// The handle keeps the binning for f3ps_slab_route: bin = key >> shift, min(top_bits, 3 * depth) bits
+int f3ps_slab_keys(f3ps_ctx* ctx, int top_bits, uint32_t* d_hist) {
     if (!ctx || !d_hist || top_bits < 1 || top_bits > kSlabHistBitsMax) return F3PS_ERR_INVALID_ARGUMENT;
     int rc = need(ctx, P_INPUT, "f3ps_slab_keys"); if (rc) return rc;
     if (!ctx->slab_frame) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_keys: f3ps_slab_set_frame has not run");
     cudaSetDevice(ctx->device);
     const int kb = 3 * ctx->depth, tb = std::min(top_bits, std::max(1, kb)), shift = std::max(0, kb - tb);
-    if (used_bits) *used_bits = tb;
-    if (shift_out) *shift_out = shift;
+    ctx->slab_bits = tb; ctx->slab_shift = shift;
     F3PS_CUDA_OK(cudaMemsetAsync(d_hist, 0, (size_t)4 << top_bits, ctx->stream));
     PointLoader pl{ctx->d_points, ctx->stride, ctx->vp.fold_negative_z};
     if (ctx->n_points == 0) { F3PS_CUDA_OK(cudaMemsetAsync(SC(n_valid), 0, 4, ctx->stream)); return F3PS_OK; }
     return ctx->key64 ? slab_keys_typed<uint64_t>(ctx, pl, shift, 1u << tb, d_hist) : slab_keys_typed<uint32_t>(ctx, pl, shift, 1u << tb, d_hist);
 }
 
-// splitters[world - 1]: ascending Morton keys, rank r owns [splitters[r-1], splitters[r]).  Packs this rank's valid points as
-// 16-byte records {x, y, z, rgba} into d_send (capacity: n points), grouped by destination rank, input order kept inside
-// a group; counts[world] = records per destination.
-int f3ps_slab_route(f3ps_ctx* ctx, int world, const uint64_t* splitters, void* d_send, int64_t* counts) {
-    if (!ctx || world < 1 || world > kSlabMaxWorld || (world > 1 && !splitters) || !counts) return F3PS_ERR_INVALID_ARGUMENT;
+// Equal-count cuts of the key space: cut r is the first bin boundary at or after r/world of the points, never below the cut
+// before it, shifted to a Morton key.  out[world - 1] ascend; rank r owns [out[r-1], out[r]).  Host only: no CUDA call.
+int f3ps_slab_choose_splitters(const uint32_t* hist, int n_bins, int world, int shift, uint64_t* out) {
+    if (!hist || n_bins < 1 || world < 1 || shift < 0 || shift > 63 || !out) return F3PS_ERR_INVALID_ARGUMENT;
+    std::vector<uint64_t> cum((size_t)n_bins);
+    uint64_t total = 0;
+    for (int i = 0; i < n_bins; ++i) cum[(size_t)i] = total += hist[i];
+    uint64_t prev = 0;
+    for (int r = 1; r < world; ++r) {
+        const uint64_t target = total * (uint64_t)r / (uint64_t)world;
+        uint64_t b = (uint64_t)(std::lower_bound(cum.begin(), cum.end(), target) - cum.begin()) + 1;
+        b = prev = std::min<uint64_t>(std::max(b, prev), (uint64_t)n_bins);
+        out[r - 1] = b << shift;
+    }
+    return F3PS_OK;
+}
+
+// d_hist: the histogram of f3ps_slab_keys, all-reduced over the ranks (device; may be NULL when world == 1).  Cuts the key space
+// with f3ps_slab_choose_splitters and packs this rank's valid points as 16-byte records {x, y, z, rgba} into d_send (capacity:
+// n points), grouped by destination rank, input order kept inside a group; counts[world] = records per destination.
+int f3ps_slab_route(f3ps_ctx* ctx, int world, const uint32_t* d_hist, void* d_send, int64_t* counts) {
+    if (!ctx || world < 1 || world > kSlabMaxWorld || (world > 1 && !d_hist) || !counts) return F3PS_ERR_INVALID_ARGUMENT;
     int rc = need(ctx, P_INPUT, "f3ps_slab_route"); if (rc) return rc;
-    if (!ctx->slab_frame) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_route: f3ps_slab_set_frame / f3ps_slab_keys have not run");
+    if (!ctx->slab_frame || !ctx->slab_bits) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_route: f3ps_slab_set_frame / f3ps_slab_keys have not run");
     cudaSetDevice(ctx->device);
     for (int r = 0; r < world; ++r) counts[r] = 0;
     if (ctx->n_points == 0) return F3PS_OK;
     SlabSplitters sp; memset(&sp, 0, sizeof sp); sp.n = world - 1;
-    for (int r = 0; r + 1 < world; ++r) { sp.key[r] = splitters[r]; if (r && splitters[r] < splitters[r - 1]) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "splitters must ascend"); }
+    if (world > 1) {
+        std::vector<uint32_t> hist((size_t)1 << ctx->slab_bits);
+        F3PS_CUDA_OK(cudaMemcpyAsync(hist.data(), d_hist, hist.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        F3PS_CUDA_OK(wait_stream(ctx));
+        uint64_t cut[kSlabMaxWorld];
+        rc = f3ps_slab_choose_splitters(hist.data(), (int)hist.size(), world, ctx->slab_shift, cut); if (rc) return rc;
+        for (int r = 0; r + 1 < world; ++r) { sp.key[r] = cut[r]; if (r && cut[r] < cut[r - 1]) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "splitters must ascend"); }
+    }
     F3PS_CUDA_OK(ctx->slab_tot.ensure(kSlabMaxWorld * 4));
     F3PS_CUDA_OK(cudaMemsetAsync(ctx->slab_tot.p, 0, kSlabMaxWorld * 4, ctx->stream));
     PointLoader pl{ctx->d_points, ctx->stride, ctx->vp.fold_negative_z};
@@ -1179,27 +1203,37 @@ int f3ps_slab_array(f3ps_ctx* ctx, int which, void** ptr, int64_t* n, int* elem_
     return F3PS_OK;
 }
 
-// the voxel table of the WHOLE cloud (every rank's slice, leaf order) and the slice [own_begin, own_end) this rank computes
-int f3ps_slab_set_voxels(f3ps_ctx* ctx, const void* d_xyz, const void* d_rgb, const void* d_key, int64_t n_voxels, int64_t own_begin, int64_t own_end) {
-    if (!ctx || n_voxels < 0 || own_begin < 0 || own_end < own_begin || own_end > n_voxels) return F3PS_ERR_INVALID_ARGUMENT;
+// Right after f3ps_voxelize on the received points (ctx->V = this rank's v_local voxels): the voxel tables grow to the WHOLE
+// cloud's n_voxels, this rank's slice moves to [own_begin, own_begin + v_local), the slice it computes from here on.  The caller
+// then fills the other ranks' slices in place (f3ps_slab_array) before f3ps_neighbors.
+int f3ps_slab_set_voxels(f3ps_ctx* ctx, int64_t n_voxels, int64_t own_begin) {
+    if (!ctx || n_voxels < 0 || own_begin < 0) return F3PS_ERR_INVALID_ARGUMENT;
     if (n_voxels >= (1ll << 30)) return ctx_fail(ctx, F3PS_ERR_CAPACITY, "more than 2^30 voxels");
     if (!ctx->slab_frame) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_set_voxels: f3ps_slab_set_frame has not run");
+    if (ctx->progress != P_VOXELS || ctx->slab_range) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_slab_set_voxels: must follow f3ps_voxelize");
+    const size_t v_local = ctx->V, V = (size_t)n_voxels, Vc = std::max<size_t>(1, V), at = (size_t)own_begin;
+    if (at + v_local > V) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "f3ps_slab_set_voxels: own_begin + this rank's voxels > n_voxels");
     cudaSetDevice(ctx->device);
-    const size_t V = (size_t)n_voxels, Vc = std::max<size_t>(1, V);
-    if (d_xyz != ctx->vox_xyz.p) {
+    f3ps::DevBuf* tab[3] = {&ctx->vox_xyz, &ctx->vox_rgb, &ctx->vox_key};
+    const size_t eb[3] = {16, 16, 8}, off[3] = {0, 16, 32};          // bytes per voxel; the slice's place in the spare buffer
+    bool move = at != 0;
+    for (int i = 0; i < 3; ++i) move = move || tab[i]->cap < Vc * eb[i];
+    if (move) {        // through the spare buffer: growing a table frees its contents, and the slice's two places may overlap
+        F3PS_CUDA_OK(ctx->slab_spare.ensure(std::max<size_t>(1, v_local) * 40));
+        char* spare = ctx->slab_spare.as<char>();
+        for (int i = 0; i < 3 && v_local; ++i)
+            F3PS_CUDA_OK(cudaMemcpyAsync(spare + off[i] * v_local, tab[i]->p, v_local * eb[i], cudaMemcpyDeviceToDevice, ctx->stream));
         F3PS_CUDA_OK(wait_stream(ctx));
-        F3PS_CUDA_OK(ctx->vox_xyz.ensure(Vc * 16)); F3PS_CUDA_OK(ctx->vox_rgb.ensure(Vc * 16)); F3PS_CUDA_OK(ctx->vox_key.ensure(Vc * 8));
-        if (V) {
-            F3PS_CUDA_OK(cudaMemcpyAsync(ctx->vox_xyz.p, d_xyz, V * 16, cudaMemcpyDeviceToDevice, ctx->stream));
-            F3PS_CUDA_OK(cudaMemcpyAsync(ctx->vox_rgb.p, d_rgb, V * 16, cudaMemcpyDeviceToDevice, ctx->stream));
-            F3PS_CUDA_OK(cudaMemcpyAsync(ctx->vox_key.p, d_key, V * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        for (int i = 0; i < 3; ++i) {
+            F3PS_CUDA_OK(tab[i]->ensure(Vc * eb[i]));
+            if (v_local) F3PS_CUDA_OK(cudaMemcpyAsync(tab[i]->as<char>() + at * eb[i], spare + off[i] * v_local, v_local * eb[i], cudaMemcpyDeviceToDevice, ctx->stream));
         }
     }
     ctx->V = (unsigned)V;
     const unsigned v32 = (unsigned)V;
     F3PS_CUDA_OK(cudaMemcpyAsync(SC(n_voxels), &v32, 4, cudaMemcpyHostToDevice, ctx->stream));
     F3PS_CUDA_OK(wait_stream(ctx));
-    ctx->own_begin = (unsigned)own_begin; ctx->own_end = (unsigned)own_end; ctx->slab_range = true;
+    ctx->own_begin = (unsigned)at; ctx->own_end = (unsigned)(at + v_local); ctx->slab_range = true;
     ctx->progress = P_VOXELS;
     return mark(ctx, 1);
 }

@@ -115,10 +115,11 @@ def lib():
         "f3ps_slab_reset": (C.c_int, [vp]),
         "f3ps_slab_bbox": (C.c_int, [vp, vp]),
         "f3ps_slab_set_frame": (C.c_int, [vp, vp]),
-        "f3ps_slab_keys": (C.c_int, [vp, C.c_int, vp, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+        "f3ps_slab_keys": (C.c_int, [vp, C.c_int, vp]),
         "f3ps_slab_route": (C.c_int, [vp, C.c_int, vp, vp, vp]),
+        "f3ps_slab_choose_splitters": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp]),
         "f3ps_slab_array": (C.c_int, [vp, C.c_int, C.POINTER(vp), C.POINTER(i64), C.POINTER(C.c_int)]),
-        "f3ps_slab_set_voxels": (C.c_int, [vp, vp, vp, vp, i64, i64, i64]),
+        "f3ps_slab_set_voxels": (C.c_int, [vp, i64, i64]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -139,11 +140,22 @@ EXPORTED = ["f3ps_create", "f3ps_destroy", "f3ps_last_error", "f3ps_version", "f
             "f3ps_get_level_point_labels", "f3ps_stage_ms", "f3ps_launch_count", "f3ps_merge_profile", "f3ps_merge_trace", "f3ps_expand_profile", "f3ps_test_rgb2lab",
             "f3ps_test_lab_ciede00", "f3ps_test_rgb_eucl", "f3ps_test_sort_pairs",
             "f3ps_merge_batch", "f3ps_set_expand_sharing", "f3ps_set_expand_kernel", "f3ps_refine", "f3ps_eval_thresholds", "f3ps_eval_label_pairs", "f3ps_slab_reset", "f3ps_slab_bbox", "f3ps_slab_set_frame", "f3ps_slab_keys", "f3ps_slab_route", "f3ps_slab_array",
-            "f3ps_slab_set_voxels"]
+            "f3ps_slab_choose_splitters", "f3ps_slab_set_voxels"]
 
 
 def _p(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
+
+
+def slab_choose_splitters(hist, world, shift):
+    """Slab mode's equal-count cuts of the key space (f3ps_slab_choose_splitters, no device needed): world-1 ascending
+    Morton keys from a histogram of the keys' top bits (bin = key >> shift); rank r owns [splitters[r-1], splitters[r])."""
+    h = np.ascontiguousarray(hist, np.uint32)
+    out = np.zeros(max(1, world - 1), np.uint64)
+    rc = lib().f3ps_slab_choose_splitters(_p(h), h.shape[0], world, shift, _p(out))
+    if rc:
+        raise ValueError("f3ps_slab_choose_splitters: bad arguments (status %d)" % rc)
+    return out[:world - 1]
 
 
 def merge_batch(segs, threshold):
@@ -475,15 +487,12 @@ class Segmenter:
     def slab_bbox(self, d_box8): self._chk(self.L.f3ps_slab_bbox(self.h, C.c_void_p(d_box8)))
     def slab_set_frame(self, d_box8): self._chk(self.L.f3ps_slab_set_frame(self.h, C.c_void_p(d_box8)))
 
-    def slab_keys(self, top_bits, d_hist):
-        used, shift = C.c_int(), C.c_int()
-        self._chk(self.L.f3ps_slab_keys(self.h, top_bits, C.c_void_p(d_hist), C.byref(used), C.byref(shift)))
-        return used.value, shift.value
+    def slab_keys(self, top_bits, d_hist): self._chk(self.L.f3ps_slab_keys(self.h, top_bits, C.c_void_p(d_hist)))
 
-    def slab_route(self, world, splitters, d_send):
-        sp = np.ascontiguousarray(splitters, np.uint64)
+    def slab_route(self, world, d_hist, d_send):
+        """d_hist: the all-reduced key histogram (device pointer).  Returns the records packed for each destination rank."""
         counts = np.zeros(world, np.int64)
-        self._chk(self.L.f3ps_slab_route(self.h, world, _p(sp) if world > 1 else None, C.c_void_p(d_send), _p(counts)))
+        self._chk(self.L.f3ps_slab_route(self.h, world, C.c_void_p(d_hist), C.c_void_p(d_send), _p(counts)))
         return counts
 
     def slab_array(self, name):
@@ -492,8 +501,7 @@ class Segmenter:
         self._chk(self.L.f3ps_slab_array(self.h, self.SLAB_ARRAYS[name], C.byref(ptr), C.byref(n), C.byref(eb)))
         return (ptr.value or 0), n.value, eb.value
 
-    def slab_set_voxels(self, d_xyz, d_rgb, d_key, n_voxels, own_begin, own_end):
-        self._chk(self.L.f3ps_slab_set_voxels(self.h, C.c_void_p(d_xyz), C.c_void_p(d_rgb), C.c_void_p(d_key), n_voxels, own_begin, own_end))
+    def slab_set_voxels(self, n_voxels, own_begin): self._chk(self.L.f3ps_slab_set_voxels(self.h, n_voxels, own_begin))
 
     # ---- device self tests ----
     def test_rgb2lab(self, rgb255):

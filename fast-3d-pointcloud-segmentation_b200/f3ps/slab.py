@@ -8,11 +8,15 @@ key order IS PCL's leaf order, a slab's voxels are a contiguous slice of the sin
 ordered float sum keeps its order, so the result is bit-identical to one handle processing the whole cloud
 (tests/test_gpu_slab.py).
 
+Everything but the exchanges is a library call (include/f3ps.h, f3ps_slab_*), the splitter rule and the assembly of the
+replicated voxel table included, so this driver and host/slab_host.cpp (the same protocol over NCCL from C++) cut a cloud
+in the same place by construction.
+
 Exchanges (all on the stream the handle runs on; NCCL over NVLink when the backend is nccl):
   K1  all-reduce MIN/MAX of the transformed bounding box (6 floats)      -> same frame / key grid on every rank
-      all-reduce SUM of a 4096-bin histogram of the keys' top bits       -> equal-count splitters
+      all-reduce SUM of a 4096-bin histogram of the keys' top bits       -> equal-count splitters (f3ps_slab_route)
       all-to-all of the points, 16 bytes each, to the rank owning their key range (stable: input order survives)
-      all-gather of the voxel slices (40 bytes per voxel)                -> replicated voxel table
+      all-gather of the voxel slices (40 bytes per voxel), in place      -> replicated voxel table
   K3  normals of the owned slice, all-gather of the slices (20 bytes per voxel)
   K2 (hash + 27 probes), K4 (seed grid), K5 (the expansion kernel of one handle) and K6 run on the replicated
   tables on every rank; K7 does not shard ("replicas only": one graph, strictly serial order) and is replayed by
@@ -36,21 +40,6 @@ def device_view(torch, ptr, n, elem_bytes, dtype, device):
         return torch.empty((0, max(1, elem_bytes // torch.empty((), dtype=dtype).element_size())), dtype=dtype, device=device)
     raw = torch.as_tensor(_DevView(ptr, n * elem_bytes), device=device)
     return raw.view(dtype).view(n, -1)
-
-
-def choose_splitters(hist, world, shift):
-    """Equal-count cuts of the key space from the global histogram of the keys' top bits.
-    Returns world-1 ascending Morton keys; rank r owns [splitters[r-1], splitters[r])."""
-    hist = np.asarray(hist, np.int64)
-    total = int(hist.sum())
-    cum = np.cumsum(hist)
-    cuts = []
-    for r in range(1, world):
-        target = (total * r) // world
-        b = int(np.searchsorted(cum, target, side="left")) + 1      # first bin boundary at or after the target
-        b = min(max(b, cuts[-1] if cuts else 0), hist.shape[0])
-        cuts.append(b)
-    return np.array([np.uint64(b) << np.uint64(shift) for b in cuts], np.uint64)
 
 
 def slice_bounds(counts):
@@ -227,11 +216,10 @@ class SlabSegmenter:
             seg.slab_set_frame(box.data_ptr())
             # ---- K1b: keys, splitters, routing ----
             hist = torch.zeros(1 << self.TOP_BITS, dtype=torch.int32, device=self.device)
-            used, shift = seg.slab_keys(self.TOP_BITS, hist.data_ptr())
+            seg.slab_keys(self.TOP_BITS, hist.data_ptr())
             comm.all_reduce(hist, "sum")
-            splitters = choose_splitters(hist[: 1 << used].cpu().numpy(), comm.world, shift)
             send = torch.empty((max(1, n_local), 4), dtype=torch.float32, device=self.device)
-            send_counts = seg.slab_route(comm.world, splitters, send.data_ptr())
+            send_counts = seg.slab_route(comm.world, hist.data_ptr(), send.data_ptr())
             tick("route")
             count_matrix = comm.all_gather_vec(send_counts)      # [src, dst]
             recv_counts = count_matrix[:, comm.rank]
@@ -249,17 +237,13 @@ class SlabSegmenter:
             vb = slice_bounds(comm.all_gather_int(v_local))
             V = int(vb[-1])
             lo, hi = int(vb[comm.rank]), int(vb[comm.rank + 1])
-            full_xyz = torch.empty((V, 4), dtype=torch.float32, device=self.device)
-            full_rgb = torch.empty((V, 4), dtype=torch.float32, device=self.device)
-            full_key = torch.empty((V, 1), dtype=torch.int64, device=self.device)
-            if v_local:
-                full_xyz[lo:hi].copy_(self._view("vox_xyz", torch.float32)[:v_local])
-                full_rgb[lo:hi].copy_(self._view("vox_rgb", torch.float32)[:v_local])
-                full_key[lo:hi].copy_(self._view("vox_key", torch.int64)[:v_local])
+            seg.slab_set_voxels(V, lo)
             tick("voxelize")
-            comm.gather_slices(full_xyz, vb); comm.gather_slices(full_rgb, vb); comm.gather_slices(full_key, vb)
-            seg.slab_set_voxels(full_xyz.data_ptr(), full_rgb.data_ptr(), full_key.data_ptr(), V, lo, hi)
-            del full_xyz, full_rgb, full_key, recv
+            if V:
+                comm.gather_slices(self._view("vox_xyz", torch.float32), vb)
+                comm.gather_slices(self._view("vox_rgb", torch.float32), vb)
+                comm.gather_slices(self._view("vox_key", torch.int64), vb)
+            del recv
             tick("gather_voxels")
             # ---- K2 (replicated), K3 (owned slice + exchange), K4 (replicated) ----
             seg.neighbors()
@@ -288,6 +272,6 @@ class SlabSegmenter:
             ms[n1] = e0.elapsed_time(e1)
         ms["total"] = ev[0][1].elapsed_time(ev[-1][1])
         self.info = {"n_local": n_local, "n_received": n_recv, "v_local": v_local, "V": V, "own": (lo, hi), "sweeps": sweeps,
-                     "splitters": [int(x) for x in splitters], "send_counts": [int(c) for c in send_counts],
+                     "send_counts": [int(c) for c in send_counts],
                      "stage_ms": ms, "bytes_exchanged": comm.bytes_moved}
         return self.info

@@ -1,6 +1,7 @@
 // slab_host.cpp -- see slab_host.h.  One host thread per GPU; every exchange is an NCCL collective on the rank's stream, so it
 // orders against the f3ps kernels without extra events.  The protocol follows f3ps/slab.py step by step (the Python driver stays
-// for the torch.distributed / gloo tests); stage names and the exchanged-byte count are the same.
+// for the torch.distributed / gloo tests); stage names and the exchanged-byte count are the same.  The splitter rule and the
+// assembly of the replicated voxel table are library calls, so both drivers cut a cloud in the same place by construction.
 #include "slab_host.h"
 
 #include <cuda_runtime.h>
@@ -30,35 +31,8 @@ struct DevMem {                                    // cudaMalloc'ed buffer of on
         return p;
     }
 };
-struct RankMem { int device = 0; DevMem small, send, recv, fx, fr, fk; };   // exchange buffers of one rank, reused by every run
+struct RankMem { int device = 0; DevMem small, send, recv; };   // exchange buffers of one rank, reused by every run
 }  // namespace
-
-std::vector<uint64_t> choose_splitters(const std::vector<uint32_t>& hist, int world, int shift) {
-    uint64_t total = 0;
-    for (uint32_t h : hist) total += h;
-    std::vector<uint64_t> cum(hist.size());
-    uint64_t run = 0;
-    for (size_t i = 0; i < hist.size(); ++i) { run += hist[i]; cum[i] = run; }
-    std::vector<uint64_t> cuts;
-    for (int r = 1; r < world; ++r) {
-        const uint64_t target = total * (uint64_t)r / (uint64_t)world;
-        uint64_t b = (uint64_t)(std::lower_bound(cum.begin(), cum.end(), target) - cum.begin()) + 1;     // first bin boundary at or after the target
-        b = std::min<uint64_t>(std::max<uint64_t>(b, cuts.empty() ? 0 : cuts.back()), hist.size());
-        cuts.push_back(b);
-    }
-    for (auto& c : cuts) c <<= shift;
-    return cuts;
-}
-
-}  // namespace f3ps_host
-// plain-C view of choose_splitters for the CPU test (tests/test_slab_host_logic.py compares it with f3ps/slab.py's)
-extern "C" int f3ps_host_choose_splitters(const uint32_t* hist, int n_bins, int world, int shift, uint64_t* out) {
-    if (!hist || n_bins < 1 || world < 1 || !out) return F3PS_ERR_INVALID_ARGUMENT;
-    const std::vector<uint64_t> cuts = f3ps_host::choose_splitters(std::vector<uint32_t>(hist, hist + n_bins), world, shift);
-    for (size_t i = 0; i < cuts.size(); ++i) out[i] = cuts[i];
-    return F3PS_OK;
-}
-namespace f3ps_host {
 
 SlabRun::SlabRun(const std::vector<int>& devices) : devices_(devices) {
     const size_t w = devices_.size();
@@ -133,7 +107,7 @@ void SlabRun::rank_main(int rank, const SlabShare& share, const SlabParams& p) {
         };
         auto slab_array = [&](int which, void*& ptr, int64_t& n, int& eb) { ok(f3ps_slab_array(ctx, which, &ptr, &n, &eb), "f3ps_slab_array"); };
         RankMem& M = *(RankMem*)mem_[(size_t)rank].get();
-        DevMem &small = M.small, &send = M.send, &recv = M.recv, &fx = M.fx, &fr = M.fr, &fk = M.fk;
+        DevMem &small = M.small, &send = M.send, &recv = M.recv;
 
         ok(f3ps_set_vccs_params(ctx, p.voxel_res, p.seed_res, p.color_imp, p.spatial_imp, p.normal_imp, p.use_transform, p.fold_negative_z), "f3ps_set_vccs_params");
         ok(f3ps_set_merge_params(ctx, p.color_distance, p.geometric_distance, p.merging, p.lambda, p.bins), "f3ps_set_merge_params");
@@ -154,16 +128,11 @@ void SlabRun::rank_main(int rank, const SlabShare& share, const SlabParams& p) {
         ok(f3ps_slab_set_frame(ctx, d_box), "f3ps_slab_set_frame");
         // ---- K1b: keys, splitters, routing ----
         cu(cudaMemsetAsync(d_hist, 0, ((size_t)4) << kTopBits, st), "memset");
-        int used = 0, shift = 0;
-        ok(f3ps_slab_keys(ctx, kTopBits, d_hist, &used, &shift), "f3ps_slab_keys");
+        ok(f3ps_slab_keys(ctx, kTopBits, d_hist), "f3ps_slab_keys");
         all_reduce(d_hist, (size_t)1 << kTopBits, ncclUint32, ncclSum, 4);
-        std::vector<uint32_t> hist((size_t)1 << used);
-        cu(cudaMemcpyAsync(hist.data(), d_hist, hist.size() * 4, cudaMemcpyDeviceToHost, st), "memcpy hist");
-        cu(cudaStreamSynchronize(st), "sync");
-        const std::vector<uint64_t> splitters = choose_splitters(hist, world, shift);
         void* d_send = send.ensure((size_t)std::max<int64_t>(1, n_local) * 16);
         std::vector<int64_t> send_counts((size_t)world, 0);
-        ok(f3ps_slab_route(ctx, world, world > 1 ? splitters.data() : nullptr, d_send, send_counts.data()), "f3ps_slab_route");
+        ok(f3ps_slab_route(ctx, world, d_hist, d_send, send_counts.data()), "f3ps_slab_route");
         tick("route");
         // count matrix [src][dst] (all-gather of the rows), then the points to the rank owning their key range
         std::vector<int64_t> mat((size_t)world * (size_t)world, 0);
@@ -210,18 +179,12 @@ void SlabRun::rank_main(int rank, const SlabShare& share, const SlabParams& p) {
         } else vb[1] = v_local;
         const int64_t V = vb[(size_t)world], lo = vb[(size_t)rank], hi = vb[(size_t)rank + 1];
         info.V = V; info.own_lo = lo; info.own_hi = hi;
-        char* full_xyz = (char*)fx.ensure((size_t)std::max<int64_t>(1, V) * 16);
-        char* full_rgb = (char*)fr.ensure((size_t)std::max<int64_t>(1, V) * 16);
-        char* full_key = (char*)fk.ensure((size_t)std::max<int64_t>(1, V) * 8);
-        if (v_local) {
-            void* ptr; int64_t n; int eb;
-            slab_array(F3PS_SLAB_VOX_XYZ, ptr, n, eb); cu(cudaMemcpyAsync(full_xyz + (size_t)lo * 16, ptr, (size_t)v_local * 16, cudaMemcpyDeviceToDevice, st), "copy xyz");
-            slab_array(F3PS_SLAB_VOX_RGB, ptr, n, eb); cu(cudaMemcpyAsync(full_rgb + (size_t)lo * 16, ptr, (size_t)v_local * 16, cudaMemcpyDeviceToDevice, st), "copy rgb");
-            slab_array(F3PS_SLAB_VOX_KEY, ptr, n, eb); cu(cudaMemcpyAsync(full_key + (size_t)lo * 8, ptr, (size_t)v_local * 8, cudaMemcpyDeviceToDevice, st), "copy key");
-        }
+        ok(f3ps_slab_set_voxels(ctx, V, lo), "f3ps_slab_set_voxels");
         tick("voxelize");
-        gather_slices(full_xyz, vb, 16); gather_slices(full_rgb, vb, 16); gather_slices(full_key, vb, 8);
-        ok(f3ps_slab_set_voxels(ctx, full_xyz, full_rgb, full_key, V, lo, hi), "f3ps_slab_set_voxels");
+        if (V) {
+            void* ptr; int64_t n; int eb;
+            for (int which : {F3PS_SLAB_VOX_XYZ, F3PS_SLAB_VOX_RGB, F3PS_SLAB_VOX_KEY}) { slab_array(which, ptr, n, eb); gather_slices(ptr, vb, (size_t)eb); }
+        }
         tick("gather_voxels");
         // ---- K2 (replicated), K3 (owned slice + exchange), K4 (replicated) ----
         ok(f3ps_neighbors(ctx), "f3ps_neighbors");

@@ -4,7 +4,8 @@
 // one f3ps handle per GPU, one ncclComm_t each) starts with an arbitrary share of the points and the cloud is cut into
 // contiguous ranges of the x-major Morton key -- PCL's leaf order -- so every ordered float sum keeps its order and the result is
 // bit-identical to one handle processing the whole cloud.  Same protocol as f3ps/slab.py (torch.distributed), same per-rank C-ABI
-// pieces (include/f3ps.h: f3ps_slab_*); the exchanges are NCCL collectives issued on the handle's stream.
+// pieces (include/f3ps.h: f3ps_slab_*, splitter choice and voxel-table assembly included); this driver adds only the exchanges,
+// NCCL collectives issued on the handle's stream.
 #pragma once
 #include <cstdint>
 #include <map>
@@ -65,10 +66,4 @@ private:
     std::string init_error_;
 };
 
-// Equal-count cuts of the key space from the global histogram of the keys' top bits (f3ps/slab.py: choose_splitters):
-// world-1 ascending Morton keys; rank r owns [splitters[r-1], splitters[r]).
-std::vector<uint64_t> choose_splitters(const std::vector<uint32_t>& hist, int world, int shift);
-
 }  // namespace f3ps_host
-
-extern "C" int f3ps_host_choose_splitters(const uint32_t* hist, int n_bins, int world, int shift, uint64_t* out /*[world-1]*/);

@@ -219,12 +219,12 @@ int f3ps_get_level_point_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacit
  * (pcl::SupervoxelClustering::extract, supervoxel_clustering.cpp:357).  A slab is a contiguous range of the x-major
  * Morton key, i.e. of PCL's leaf index, so every rank's voxels are a contiguous slice of the single-GPU voxel table and
  * all ordered sums keep their order: results are bit-identical to one handle processing the whole cloud.
- * These entry points are the per-rank pieces; the caller issues the exchanges between them on the handle's stream
- * (f3ps/slab.py does it with torch.distributed / NCCL):
+ * These entry points are the per-rank pieces; the caller issues only the exchanges between them, on the handle's stream
+ * (f3ps/slab.py does it with torch.distributed, host/slab_host.cpp with NCCL):
  *   f3ps_set_input(local points) -> f3ps_slab_bbox -> [all-reduce MIN/MAX] -> f3ps_slab_set_frame -> f3ps_slab_keys
- *   -> [all-reduce SUM histogram; choose splitters] -> f3ps_slab_route -> [all-to-all points] -> f3ps_set_input(received,
- *   stride 16, on device) -> f3ps_voxelize -> [all-gather voxel slices] -> f3ps_slab_set_voxels -> f3ps_neighbors ->
- *   f3ps_normals (owned slice) -> [all-gather normal slices] -> f3ps_seeds -> f3ps_expand -> f3ps_graph -> f3ps_merge.
+ *   -> [all-reduce SUM histogram] -> f3ps_slab_route -> [all-to-all points] -> f3ps_set_input(received, stride 16, on device)
+ *   -> f3ps_voxelize -> [all-gather v_local] -> f3ps_slab_set_voxels -> [all-gather voxel slices, in place] -> f3ps_neighbors
+ *   -> f3ps_normals (owned slice) -> [all-gather normal slices] -> f3ps_seeds -> f3ps_expand -> f3ps_graph -> f3ps_merge.
  * From f3ps_seeds on every rank works on the whole gathered table; K7 does not shard (strictly serial order over one graph). */
 enum f3ps_slab_array_id {
     F3PS_SLAB_VOX_XYZ = 0, F3PS_SLAB_VOX_RGB = 1, F3PS_SLAB_VOX_KEY = 2, F3PS_SLAB_VOX_NORMAL = 3, F3PS_SLAB_VOX_CURV = 4
@@ -232,11 +232,21 @@ enum f3ps_slab_array_id {
 int f3ps_slab_reset(f3ps_ctx* ctx);
 int f3ps_slab_bbox(f3ps_ctx* ctx, uint32_t* d_box8);
 int f3ps_slab_set_frame(f3ps_ctx* ctx, const uint32_t* d_box8);
-int f3ps_slab_keys(f3ps_ctx* ctx, int top_bits, uint32_t* d_hist, int* used_bits, int* shift);
-int f3ps_slab_route(f3ps_ctx* ctx, int world, const uint64_t* splitters, void* d_send, int64_t* counts);
+/* Morton keys of the local points and the histogram of their top bits into d_hist (1 << top_bits counters, device, top_bits
+ * <= 15); the handle keeps the binning for f3ps_slab_route. */
+int f3ps_slab_keys(f3ps_ctx* ctx, int top_bits, uint32_t* d_hist);
+/* d_hist: the all-reduced histogram (device; may be NULL when world == 1), cut by f3ps_slab_choose_splitters.  Packs the local
+ * points as 16-byte records into d_send (capacity: n points), grouped by destination rank; counts[world] = records per rank. */
+int f3ps_slab_route(f3ps_ctx* ctx, int world, const uint32_t* d_hist, void* d_send, int64_t* counts);
+/* The splitter rule, without a handle or a device: equal-count cuts of hist[n_bins] (bin = key >> shift) into world slabs,
+ * each at the first bin boundary at or after its share of the points and never below the cut before it.  out[world - 1]
+ * ascend; rank r owns the keys [out[r-1], out[r]). */
+int f3ps_slab_choose_splitters(const uint32_t* hist, int n_bins, int world, int shift, uint64_t* out);
+/* device arrays the caller exchanges in place: pointer, elements (V), bytes per element */
 int f3ps_slab_array(f3ps_ctx* ctx, int which, void** ptr, int64_t* n, int* elem_bytes);
-int f3ps_slab_set_voxels(f3ps_ctx* ctx, const void* d_xyz, const void* d_rgb, const void* d_key, int64_t n_voxels,
-                         int64_t own_begin, int64_t own_end);
+/* Right after f3ps_voxelize on the received points: grows the voxel tables to the whole cloud's n_voxels (< 2^30) and moves
+ * this rank's v_local voxels to [own_begin, own_begin + v_local), the slice it owns; the caller fills the other slices. */
+int f3ps_slab_set_voxels(f3ps_ctx* ctx, int64_t n_voxels, int64_t own_begin);
 
 /* ---- "next" row f1: the auto-threshold sweep ------------------------------------------------------------------------
  * Clustering::all_thresh (clustering.cpp:691-729) with Testing::eval_performance (testing.cpp:239-362) from ONE merge replay:

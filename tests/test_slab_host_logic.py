@@ -1,21 +1,29 @@
-"""Host logic of slab mode on CPU: splitter choice, slice bookkeeping and the collectives wrapper over a
+"""Host logic of slab mode on CPU: the library's splitter rule, slice bookkeeping and the collectives wrapper over a
 world_size-2 gloo group (the GPU pieces between the exchanges are covered by tests/test_gpu_slab.py)."""
 import os
 import socket
 
 import numpy as np
+import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 
-def test_choose_splitters_equal_count():
+@pytest.fixture(scope="module")
+def binding():
+    from f3ps import binding
+    binding.build()
+    return binding
+
+
+def test_choose_splitters_equal_count(binding):
     from f3ps import slab
     rng = np.random.default_rng(5)
     hist = rng.integers(0, 1000, 4096)
     hist[:700] = 0
     for world in (1, 2, 3, 4, 8):
-        sp = slab.choose_splitters(hist, world, shift=9)
+        sp = binding.slab_choose_splitters(hist, world, shift=9)
         assert sp.shape == (world - 1,) and np.all(np.diff(sp.astype(np.int64)) >= 0)
         cuts = [0] + [int(x) >> 9 for x in sp] + [4096]
         loads = [int(hist[cuts[i]:cuts[i + 1]].sum()) for i in range(world)]
@@ -24,24 +32,27 @@ def test_choose_splitters_equal_count():
             assert max(loads) - min(loads) <= 2 * int(hist.max()) + 1
     # degenerate: everything in one bin -> one rank owns it all, splitters still ascend
     h = np.zeros(64, np.int64); h[10] = 99
-    sp = slab.choose_splitters(h, 4, shift=0)
+    sp = binding.slab_choose_splitters(h, 4, shift=0)
     assert list(sp) == sorted(sp) and all(int(x) <= 64 for x in sp)
     assert list(slab.slice_bounds([3, 0, 5])) == [0, 3, 3, 8]
 
 
-def test_cpp_choose_splitters_equals_python():
-    """host/slab_host.cpp (the C++ NCCL slab host) cuts the key space exactly where f3ps/slab.py does: the two hosts drive the same
-    protocol, so a cloud lands in the same slabs whichever one runs it."""
-    import ctypes as C
-    import os
-    import subprocess
-    from f3ps import slab
-    host = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "fast-3d-pointcloud-segmentation_b200", "host")
-    subprocess.check_call(["make", "-C", os.path.dirname(host), "-s"])
-    subprocess.check_call(["make", "-C", host, "-s", "libf3ps_slab.so"])
-    lib = C.CDLL(os.path.join(host, "libf3ps_slab.so"))
-    lib.f3ps_host_choose_splitters.restype = C.c_int
-    lib.f3ps_host_choose_splitters.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]
+def _splitters_reference(hist, world, shift):
+    """The splitter rule restated in numpy: cut r is the first bin boundary at or after r/world of the points (cumulative
+    count >= total * r // world), never below the cut before it, at most the bin count, shifted left by `shift`."""
+    hist = np.asarray(hist, np.int64)
+    total = int(hist.sum())
+    cum = np.cumsum(hist)
+    cuts = []
+    for r in range(1, world):
+        b = int(np.searchsorted(cum, (total * r) // world, side="left")) + 1
+        cuts.append(min(max(b, cuts[-1] if cuts else 0), hist.shape[0]))
+    return np.array([np.uint64(b) << np.uint64(shift) for b in cuts], np.uint64)
+
+
+def test_library_choose_splitters_equals_reference(binding):
+    """f3ps_slab_choose_splitters, the one splitter rule both slab drivers (f3ps/slab.py, host/slab_host.cpp) call, against
+    its restatement above, over bin counts, rank counts, shifts and degenerate histograms."""
     rng = np.random.default_rng(17)
     cases = []
     for n_bins in (1, 2, 64, 4096):
@@ -54,10 +65,9 @@ def test_cpp_choose_splitters_equals_python():
     for h in cases:
         for world in (1, 2, 3, 8):
             for shift in (0, 9, 33):
-                want = slab.choose_splitters(h, world, shift)
-                got = np.zeros(max(1, world - 1), np.uint64)
-                assert lib.f3ps_host_choose_splitters(h.ctypes.data, len(h), world, shift, got.ctypes.data) == 0
-                assert np.array_equal(got[:world - 1], want), (len(h), world, shift)
+                want = _splitters_reference(h, world, shift)
+                got = binding.slab_choose_splitters(h, world, shift)
+                assert np.array_equal(got, want), (len(h), world, shift)
 
 
 def _oracle_keys(pts):
@@ -84,7 +94,7 @@ def _worker(rank, world, port, q):
         os.environ["MASTER_ADDR"] = "127.0.0.1"
         os.environ["MASTER_PORT"] = str(port)
         dist.init_process_group("gloo", rank=rank, world_size=world)
-        from f3ps import slab, synth
+        from f3ps import binding, slab, synth
         comm = slab.Comm(dist, torch)
         assert comm.staged and comm.world == world
         pts = synth.make_frame(seed=11, width=160, height=120)
@@ -97,7 +107,7 @@ def _worker(rank, world, port, q):
         shift = max(0, 3 * depth - 12)
         hist = torch.from_numpy(np.bincount((keys >> np.uint64(shift)).astype(np.int64), minlength=4096).astype(np.int32))
         comm.all_reduce(hist, "sum")
-        sp = slab.choose_splitters(hist.numpy(), world, shift)
+        sp = binding.slab_choose_splitters(hist.numpy(), world, shift)
         dest = np.searchsorted(sp, keys, side="right")
         order = np.argsort(dest, kind="stable")
         send_counts = np.bincount(dest, minlength=world).astype(np.int64)
@@ -128,7 +138,7 @@ def _worker(rank, world, port, q):
         q.put((rank, False, "%s\n%s" % (e, traceback.format_exc())))
 
 
-def test_two_rank_gloo_exchange_protocol(oracle_mod):
+def test_two_rank_gloo_exchange_protocol(oracle_mod, binding):
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
