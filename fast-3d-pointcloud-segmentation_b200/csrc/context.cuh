@@ -120,7 +120,10 @@ struct f3ps_ctx {
     static constexpr int kEvents = 11;   // 0..8 stage boundaries, 9/10 around the merge kernel alone
     cudaEvent_t ev[kEvents] = {};
     bool ev_valid[kEvents] = {};
-    cudaEvent_t ev_batch = nullptr;    // f3ps_merge_batch: set-up done / grid done
+    cudaEvent_t ev_batch = nullptr;    // f3ps_merge_batch: set-up done
+    // f3ps_merge_batch, as the lead of a chunk: the DevScalars of the chunk's frames, gathered on the device and their pinned mirror
+    f3ps::DevBuf batch_sc;
+    f3ps::DevScalars* h_batch_sc = nullptr;
     cudaEvent_t ev_wait = nullptr;     // blocking-sync event for sweeps (f3ps_set_blocking_wait)
     bool blocking_wait = false;
     // slab mode (f3ps_slab_*): injected global frame, histogram binning of f3ps_slab_keys (bin = key >> slab_shift,

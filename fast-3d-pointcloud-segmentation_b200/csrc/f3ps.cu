@@ -261,6 +261,7 @@ void f3ps_destroy(f3ps_ctx* ctx) {
     for (int i = 0; i < f3ps_ctx::kEvents; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->ev_wait) cudaEventDestroy(ctx->ev_wait);
     if (ctx->ev_batch) cudaEventDestroy(ctx->ev_batch);
+    if (ctx->h_batch_sc) cudaFreeHost(ctx->h_batch_sc);
     if (ctx->private_stream) cudaStreamDestroy(ctx->private_stream);
     delete ctx;
 }
@@ -872,6 +873,18 @@ int merge_labels(f3ps_ctx* ctx) {
                   ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>());
     return F3PS_OK;
 }
+LabelArgs label_args(const f3ps_ctx* ctx) {
+    LabelArgs A;
+    A.R = ctx->R1; A.n_sv_ptr = SC(xctl.n_sv); A.run_start = ctx->run_start.as<unsigned>(); A.run_end = ctx->run_end.as<unsigned>();
+    A.run_out_off = ctx->run_out_off.as<unsigned>(); A.run_dense = ctx->run_dense.as<unsigned>(); A.region_dense = ctx->region_dense.as<unsigned>();
+    A.n_out = SC(n_out);
+    A.pos_run = ctx->pos_run.as<unsigned>(); A.n_pos = ctx->n_pos; A.order = ctx->order; A.vox_xyz = ctx->gxyz;
+    A.out_xyz = ctx->out_xyz.as<float>(); A.out_label = ctx->out_label.as<unsigned>(); A.out_voxel = ctx->out_voxel.as<unsigned>();
+    A.vox_segment = ctx->vox_segment.as<unsigned>();
+    A.pos_label = ctx->graph_from_host ? nullptr : ctx->sorted_label; A.owner = ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>();
+    A.scalars = (const unsigned*)ctx->d_sc;
+    return A;
+}
 // after the replay's scalars reached the host; the merged state is one level, its threshold (f3ps_merge_levels records more)
 int merge_done(f3ps_ctx* ctx, float threshold) {
     if (ctx->h_sc->mctl.error) return ctx_fail(ctx, F3PS_ERR_CAPACITY, "merge kernel reported an internal capacity error");
@@ -942,6 +955,12 @@ int f3ps_merge(f3ps_ctx* ctx, float threshold) {
 // single-CTA merge kernels overlap); one grid of n CTAs runs n frames side by side.  Every handle must be on the same device,
 // with its graph built (f3ps_graph); handles whose plan is not the shared-memory kernel without phase counters run on their own.
 // Results per handle are exactly those of f3ps_merge(handle, threshold).
+//
+// Everything that follows a chunk's grid (labelled clouds, the scalars' read-back, the stage marks 10 and 8 of every frame) runs
+// on the lead's stream, as launches over the whole chunk.  No member stream waits for the grid: a stream parked behind a grid
+// that runs for tens of milliseconds would hold its hardware queue, and the work other handles enqueue on that queue (the next
+// group's front stages in a pipelined sweep) would wait for the grid too.  The function returns only after the host has seen
+// every lead stream finish, so later work on a member's own stream (getters, levels, the next frame) needs no event wait.
 int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
     if (!ctxs || n < 1) return F3PS_ERR_INVALID_ARGUMENT;
     for (int i = 0; i < n; ++i) {
@@ -960,9 +979,13 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
         plans[i] = plan_merge(ctx);
         (ctx->S > 0 && plans[i].kind == kMergeShared && !plans[i].prof ? batch : solo).push_back(i);
     }
+    const size_t sc_words = sizeof(DevScalars) / 4;
+    static_assert(sizeof(DevScalars) % 4 == 0, "DevScalars is gathered as words");
     for (size_t g0 = 0; g0 < batch.size(); g0 += kFastBatchMax) {
         const size_t g1 = std::min(batch.size(), g0 + (size_t)kFastBatchMax);
+        const unsigned nf = (unsigned)(g1 - g0);
         static thread_local FastBatch B;                     // 32 KB: not on the stack
+        static thread_local LabelBatch L;
         size_t bytes = 0;                                    // every frame brings its own table capacities (the layout is per CTA)
         f3ps_ctx* lead = ctxs[batch[g0]];
         for (size_t k = g0; k < g1; ++k) {
@@ -977,30 +1000,46 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
                 F3PS_CUDA_OK(cudaStreamWaitEvent(lead->stream, ctx->ev_batch, 0));
             }
         }
-        {
-            f3ps_ctx* ctx = lead;
-            rc = smem_opt_in(ctx, (const void*)merge_fast_batch_kernel, kSmemMax); if (rc) return rc;
-            LAUNCH(ctx, merge_fast_batch_kernel, (unsigned)(g1 - g0), kFastThreads, bytes, B);
-            F3PS_CUDA_OK(cudaEventRecord(ctx->ev_batch, ctx->stream));
+        f3ps_ctx* ctx = lead;
+        rc = smem_opt_in(ctx, (const void*)merge_fast_batch_kernel, kSmemMax); if (rc) return rc;
+        LAUNCH(ctx, merge_fast_batch_kernel, nf, kFastThreads, bytes, B);
+        int gx = 1;
+        for (size_t k = g0; k < g1; ++k) {
+            f3ps_ctx* m = ctxs[batch[k]];
+            F3PS_CUDA_OK(cudaEventRecord(m->ev[10], lead->stream)); m->ev_valid[10] = true;
+            m->merge_path = kMergeShared;
+            L.a[k - g0] = label_args(m);
+            gx = std::max(gx, grid_for(m->n_pos, 256));
         }
-        for (size_t k = g0; k < g1; ++k) {                   // every handle continues on its own stream after the grid
-            f3ps_ctx* ctx = ctxs[batch[k]];
-            if (ctx->stream != lead->stream) F3PS_CUDA_OK(cudaStreamWaitEvent(ctx->stream, lead->ev_batch, 0));
-            ctx->merge_path = kMergeShared;
-            rc = merge_labels(ctx); if (rc) return rc;
-            rc = mark(ctx, 8); if (rc) return rc;
+        LAUNCH(ctx, dense_label_batch_kernel, nf, 1024, 0, L);
+        LAUNCH(ctx, labeled_cloud_batch_kernel, dim3(gx, nf), 256, 0, L);
+        for (size_t k = g0; k < g1; ++k) {
+            f3ps_ctx* m = ctxs[batch[k]];
+            F3PS_CUDA_OK(cudaEventRecord(m->ev[8], lead->stream)); m->ev_valid[8] = true;
         }
+        F3PS_CUDA_OK(lead->batch_sc.ensure(kFastBatchMax * sizeof(DevScalars)));
+        if (!lead->h_batch_sc) F3PS_CUDA_OK(cudaMallocHost(&lead->h_batch_sc, kFastBatchMax * sizeof(DevScalars)));
+        LAUNCH(ctx, scalars_gather_kernel, nf, 128, 0, L, (unsigned)sc_words, lead->batch_sc.as<unsigned>());
+        F3PS_CUDA_OK(cudaMemcpyAsync(lead->h_batch_sc, lead->batch_sc.p, nf * sizeof(DevScalars), cudaMemcpyDeviceToHost, lead->stream));
     }
     // the other handles one by one, next to the grids already in flight
     for (int i : solo) { rc = merge_one(ctxs[i], threshold, kStartFresh); if (rc) return rc; }
     // results only after EVERY chunk's grid is in flight (a batch larger than one parameter block must not run its chunks back to back);
     // a frame whose CTA stopped continues alone
-    for (int i : batch) {
-        f3ps_ctx* ctx = ctxs[i];
-        rc = pull_scalars(ctx); if (rc) return rc;
-        const unsigned err = ctx->h_sc->mctl.error;
-        rc = err ? merge_one(ctx, threshold, err == kFastErrTouched ? kStartContinue : kStartGeneral) : merge_done(ctx, threshold);
-        if (rc) return rc;
+    for (size_t g0 = 0; g0 < batch.size(); g0 += kFastBatchMax) {
+        const size_t g1 = std::min(batch.size(), g0 + (size_t)kFastBatchMax);
+        f3ps_ctx* lead = ctxs[batch[g0]];
+        {
+            f3ps_ctx* ctx = lead;
+            F3PS_CUDA_OK(wait_stream(ctx));
+        }
+        for (size_t k = g0; k < g1; ++k) {
+            f3ps_ctx* ctx = ctxs[batch[k]];
+            memcpy(ctx->h_sc, lead->h_batch_sc + (k - g0), sizeof(DevScalars));
+            const unsigned err = ctx->h_sc->mctl.error;
+            rc = err ? merge_one(ctx, threshold, err == kFastErrTouched ? kStartContinue : kStartGeneral) : merge_done(ctx, threshold);
+            if (rc) return rc;
+        }
     }
     return F3PS_OK;
 }

@@ -501,7 +501,8 @@ __global__ void __launch_bounds__(kMergeThreads, 1) merge_kernel(RegionArrays R,
 // dense labels 0..K-1 in ascending region label order; output offset of every run of every rope.
 // One block: two exclusive scans over the regions (alive flag -> dense label, voxel count -> output offset), then one
 // thread per surviving region walks its rope.
-__global__ void __launch_bounds__(1024) dense_label_kernel(RegionArrays R, const unsigned* __restrict__ n_sv_ptr, const unsigned* __restrict__ run_start,
+// The bodies are shared with the batched kernels of f3ps_merge_batch (kernels_merge_lean.cuh), one frame per CTA / grid row.
+__device__ __forceinline__ void dense_label_body(RegionArrays R, const unsigned* __restrict__ n_sv_ptr, const unsigned* __restrict__ run_start,
         const unsigned* __restrict__ run_end, unsigned* __restrict__ run_out_off, unsigned* __restrict__ run_dense,
         unsigned* __restrict__ region_dense, unsigned* __restrict__ n_out) {
     __shared__ unsigned s_wa[32], s_wn[32];
@@ -543,20 +544,29 @@ __global__ void __launch_bounds__(1024) dense_label_kernel(RegionArrays R, const
     }
     if (threadIdx.x == 0) *n_out = s_cn;
 }
+__global__ void __launch_bounds__(1024) dense_label_kernel(RegionArrays R, const unsigned* __restrict__ n_sv_ptr, const unsigned* __restrict__ run_start,
+        const unsigned* __restrict__ run_end, unsigned* __restrict__ run_out_off, unsigned* __restrict__ run_dense,
+        unsigned* __restrict__ region_dense, unsigned* __restrict__ n_out) {
+    dense_label_body(R, n_sv_ptr, run_start, run_end, run_out_off, run_dense, region_dense, n_out);
+}
+// The loop of labeled_cloud_kernel, over the names of its parameters.  A macro rather than a function: inlined, a function's
+// __restrict__ parameters no longer let the compiler load owner[] through the non-coherent path.
+#define F3PS_LABELED_CLOUD_LOOP                                                                                                    \
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += gridDim.x * blockDim.x) {                                \
+        const unsigned run = pos_run[i];                                                                                           \
+        if (run == 0xffffffffu) continue;                 /* unowned voxel: absent from every region */                            \
+        const unsigned o = run_out_off[run] + (i - run_start[run]);                                                                \
+        const unsigned v = order[i];                                                                                               \
+        const float4 p = vox_xyz[v];                                                                                               \
+        out_xyz[3 * (size_t)o] = p.x; out_xyz[3 * (size_t)o + 1] = p.y; out_xyz[3 * (size_t)o + 2] = p.z;                          \
+        out_label[o] = run_dense[run]; out_voxel[o] = v;                                                                           \
+        if (!owner || owner[v] == pos_label[i]) vox_segment[v] = run_dense[run];   /* a phantom leaf does not relabel its voxel */ \
+    }
 __global__ void __launch_bounds__(256) labeled_cloud_kernel(const unsigned* __restrict__ pos_run, unsigned n_pos, const unsigned* __restrict__ order,
         const unsigned* __restrict__ run_start, const unsigned* __restrict__ run_out_off, const unsigned* __restrict__ run_dense,
         const float4* __restrict__ vox_xyz, float* __restrict__ out_xyz, unsigned* __restrict__ out_label, unsigned* __restrict__ out_voxel,
         unsigned* __restrict__ vox_segment, const unsigned* __restrict__ pos_label, const unsigned* __restrict__ owner) {
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += gridDim.x * blockDim.x) {
-        const unsigned run = pos_run[i];
-        if (run == 0xffffffffu) continue;                 // unowned voxel: absent from every region
-        const unsigned o = run_out_off[run] + (i - run_start[run]);
-        const unsigned v = order[i];
-        const float4 p = vox_xyz[v];
-        out_xyz[3 * (size_t)o] = p.x; out_xyz[3 * (size_t)o + 1] = p.y; out_xyz[3 * (size_t)o + 2] = p.z;
-        out_label[o] = run_dense[run]; out_voxel[o] = v;
-        if (!owner || owner[v] == pos_label[i]) vox_segment[v] = run_dense[run];   // a phantom leaf does not relabel its voxel
-    }
+    F3PS_LABELED_CLOUD_LOOP
 }
 
 } // namespace f3ps

@@ -1131,4 +1131,34 @@ struct FastBatch { FastArgs a[kFastBatchMax]; };
 static_assert(sizeof(FastBatch) <= 32764, "kernel parameter space");
 __global__ void __launch_bounds__(kFastThreads, 1) merge_fast_batch_kernel(const __grid_constant__ FastBatch B) { merge_lean_body<false>(B.a[blockIdx.x]); }
 
+// What follows a batch grid, for all its frames in three launches on the grid's stream (f3ps_merge_batch): the labelled cloud
+// of every frame (CTA i / grid row i = frame i, the bodies of dense_label_kernel and labeled_cloud_kernel), then every frame's
+// device scalars gathered into one array for a single copy to the host.
+struct LabelArgs {
+    RegionArrays R; const unsigned* n_sv_ptr; const unsigned* run_start; const unsigned* run_end;
+    unsigned* run_out_off; unsigned* run_dense; unsigned* region_dense; unsigned* n_out;
+    const unsigned* pos_run; unsigned n_pos; const unsigned* order; const float4* vox_xyz;
+    float* out_xyz; unsigned* out_label; unsigned* out_voxel; unsigned* vox_segment; const unsigned* pos_label; const unsigned* owner;
+    const unsigned* scalars;         // the frame's DevScalars, as words
+};
+struct LabelBatch { LabelArgs a[kFastBatchMax]; };
+static_assert(sizeof(LabelBatch) <= 32764, "kernel parameter space");
+__global__ void __launch_bounds__(1024) dense_label_batch_kernel(const __grid_constant__ LabelBatch B) {
+    const LabelArgs& A = B.a[blockIdx.x];
+    dense_label_body(A.R, A.n_sv_ptr, A.run_start, A.run_end, A.run_out_off, A.run_dense, A.region_dense, A.n_out);
+}
+__global__ void __launch_bounds__(256) labeled_cloud_batch_kernel(const __grid_constant__ LabelBatch B) {
+    const LabelArgs& A = B.a[blockIdx.y];
+    const unsigned* __restrict__ pos_run = A.pos_run; const unsigned n_pos = A.n_pos; const unsigned* __restrict__ order = A.order;
+    const unsigned* __restrict__ run_start = A.run_start; const unsigned* __restrict__ run_out_off = A.run_out_off;
+    const unsigned* __restrict__ run_dense = A.run_dense; const float4* __restrict__ vox_xyz = A.vox_xyz;
+    float* __restrict__ out_xyz = A.out_xyz; unsigned* __restrict__ out_label = A.out_label; unsigned* __restrict__ out_voxel = A.out_voxel;
+    unsigned* __restrict__ vox_segment = A.vox_segment; const unsigned* __restrict__ pos_label = A.pos_label; const unsigned* __restrict__ owner = A.owner;
+    F3PS_LABELED_CLOUD_LOOP
+}
+__global__ void scalars_gather_kernel(const __grid_constant__ LabelBatch B, unsigned words, unsigned* __restrict__ out) {
+    const unsigned* __restrict__ src = B.a[blockIdx.x].scalars;
+    for (unsigned w = threadIdx.x; w < words; w += blockDim.x) out[(size_t)blockIdx.x * words + w] = src[w];
+}
+
 } // namespace f3ps
