@@ -14,6 +14,7 @@
 #include "kernels_merge.cuh"
 #include "kernels_merge_lean.cuh"
 #include "kernels_eval.cuh"
+#include "kernels_segments.cuh"
 
 namespace f3ps {
 
@@ -36,6 +37,16 @@ struct DevBuf {
     }
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
     template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
+};
+
+// the members of every segment of one level, grouped (f3ps_get_segment_points / _voxels): sort buffers, offsets[K+1] and the
+// partial offsets (kernels_segments.cuh), and where the grouped indices ended up; level -1 = nothing grouped since the last merge
+struct SegCsr {
+    DevBuf keys_a, keys_b, vals_a, vals_b, offsets, counts;
+    const unsigned* index = nullptr;
+    int level = -1; unsigned n = 0, K = 0;
+    long long* off() const { return offsets.as<long long>(); }
+    unsigned* chunk_off() const { return reinterpret_cast<unsigned*>(offsets.as<long long>() + K + 1); }
 };
 
 // everything the kernels count or decide lives here, on the device; the host mirrors it on demand
@@ -140,6 +151,9 @@ struct f3ps_ctx {
     int lv_built = 0;                   // 0 nothing, 1 level tables of lv_thr, 2 and the voxel table
     std::vector<int32_t> lv_m_h, lv_nseg_h;
     f3ps::DevBuf lv_small, lv_parent, lv_when, lv_dense, lv_seg, lv_vox, lv_points;
+    // segment extraction: the point and the voxel grouping of the last level asked for, kept until the next merge
+    f3ps::SegCsr seg_points, seg_voxels;
+    f3ps::DevBuf seg_part, seg_info;
     f3ps::DevBuf graph_vox;             // f3ps_set_graph: voxel index as passed in, per position
     int expand_kernel_choice = 0;       // f3ps_set_expand_kernel: 0 auto, 1 cooperative grid, 2 one cluster
     int expand_cluster_ctas = 0;        // cap of the cluster size (0 = by V, at most 16)

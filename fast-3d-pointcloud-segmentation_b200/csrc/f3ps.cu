@@ -792,6 +792,7 @@ int merge_restart(f3ps_ctx* ctx) {
 int merge_begin(f3ps_ctx* ctx, bool restart) {
     int rc = mark(ctx, 7); if (rc) return rc;
     ctx->lv_thr.clear(); ctx->lv_built = 0;
+    ctx->seg_points.level = ctx->seg_voxels.level = -1;
     if (restart && (rc = merge_restart(ctx))) return rc;
     const size_t Sc = std::max(1u, ctx->S), Pc = std::max(1u, ctx->n_pos);
     F3PS_CUDA_OK(ctx->mlog.ensure(Sc * 20));
@@ -1701,6 +1702,58 @@ int level_labels(f3ps_ctx* ctx, const int* pv, int64_t n, uint32_t* labels, int6
     }
     return fin(ctx);
 }
+// segment extraction (kernels_segments.cuh): the members of segments 0..K-1 of `level` grouped into g -- the points (pv =
+// point_voxel over the n input points) or the n voxels (pv == nullptr) -- unless g already holds that level.  One wait, for the
+// two sizes the host needs to size the sort (members, segments).
+int segment_group(f3ps_ctx* ctx, int level, const int* pv, int64_t n, SegCsr& g) {
+    if (g.level == level) return F3PS_OK;
+    g.level = -1;
+    const int Lp = level_row((int)ctx->lv_thr.size());
+    const size_t nc = (size_t)std::max<int64_t>(n, 1), Sc = (size_t)ctx->S + 1;     // K <= S
+    F3PS_CUDA_OK(g.keys_a.ensure(nc * 4)); F3PS_CUDA_OK(g.keys_b.ensure(nc * 4));
+    F3PS_CUDA_OK(g.vals_a.ensure(nc * 4)); F3PS_CUDA_OK(g.vals_b.ensure(nc * 4));
+    F3PS_CUDA_OK(g.counts.ensure((Sc + 1) * 4)); F3PS_CUDA_OK(g.offsets.ensure(Sc * 12));
+    unsigned* sizes = g.counts.as<unsigned>();              // [0] members, [1] segments, then the K counts
+    SegmentKeyOp op{pv, ctx->lv_vox.as<unsigned>(), Lp, level, g.keys_a.as<unsigned>(), g.vals_a.as<unsigned>()};
+    int rc = run_compact(ctx, op, nullptr, n, sizes); if (rc) return rc;
+    F3PS_CUDA_OK(cudaMemcpyAsync(sizes + 1, levels_nseg(ctx) + level, 4, cudaMemcpyDeviceToDevice, ctx->stream));
+    unsigned h[2];
+    if ((rc = d2h(ctx, h, sizes, sizeof h)) || (rc = fin(ctx))) return rc;
+    g.n = h[0]; g.K = h[1];
+    unsigned* counts = sizes + 2;
+    const unsigned* keys = g.keys_a.as<unsigned>();
+    g.index = g.vals_a.as<unsigned>();
+    if (g.K > 1 && g.n > 1) {                                // one segment: the compaction's index order is the grouping
+        unsigned *sk, *sv;
+        rc = sort_pairs<unsigned>(ctx, g.keys_a.as<unsigned>(), g.vals_a.as<unsigned>(), g.keys_b.as<unsigned>(), g.vals_b.as<unsigned>(),
+                                  g.keys_a.as<unsigned>(), g.vals_a.as<unsigned>(), nullptr, g.n, bits_for(g.K - 1), &sk, &sv);
+        if (rc) return rc;
+        keys = sk; g.index = sv;
+    }
+    if (g.K) F3PS_CUDA_OK(cudaMemsetAsync(counts, 0, (size_t)g.K * 4, ctx->stream));
+    if (g.n) LAUNCH(ctx, segment_count_kernel, grid_for((g.n + kSegRun - 1) / kSegRun, 256), 256, 0, keys, sizes, counts);
+    LAUNCH(ctx, segment_offsets_kernel, 1, 1024, 0, counts, g.K, g.off(), g.chunk_off());
+    g.level = level;
+    return F3PS_OK;
+}
+// checks shared by the segment getters; points: the getter needs the handle's input cloud
+int segments_ready(f3ps_ctx* ctx, int level, bool points, const char* what) {
+    if (points && ctx->graph_from_host) return ctx_fail(ctx, F3PS_ERR_LOGIC, std::string(what) + ": no input cloud, the graph was supplied by the caller");
+    if (points && ctx->slab_range) return ctx_fail(ctx, F3PS_ERR_LOGIC, std::string(what) + ": slab mode, the handle holds no input cloud of its own voxels");
+    int rc = levels_ready(ctx, true, what); if (rc) return rc;
+    if (level < 0 || level >= (int)ctx->lv_thr.size()) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, std::string(what) + ": level out of range");
+    return F3PS_OK;
+}
+// offsets[K+1] and index[n] of g into caller memory: enqueued (device) or copied and waited for (host)
+int segment_copy(f3ps_ctx* ctx, const SegCsr& g, int64_t* offsets, int32_t* index, int32_t cap_segments, int64_t cap_index, int on_device) {
+    int rc;
+    if ((rc = cap_check(ctx, (int64_t)g.K + 1, cap_segments)) || (rc = cap_check(ctx, g.n, cap_index))) return rc;
+    if (!offsets || (g.n && !index)) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "no output buffer");
+    const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    F3PS_CUDA_OK(cudaMemcpyAsync(offsets, g.off(), ((size_t)g.K + 1) * 8, kind, ctx->stream));
+    if (g.n) F3PS_CUDA_OK(cudaMemcpyAsync(index, g.index, (size_t)g.n * 4, kind, ctx->stream));
+    return on_device ? F3PS_OK : fin(ctx);
+}
 } // namespace
 } // extern "C++"
 
@@ -1747,6 +1800,46 @@ int f3ps_get_level_point_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacit
     if (ctx->slab_range) return ctx_fail(ctx, F3PS_ERR_LOGIC, "f3ps_get_level_point_labels: slab mode, the handle holds no input cloud of its own voxels");
     int rc = levels_ready(ctx, true, "f3ps_get_level_point_labels"); if (rc) return rc;
     return level_labels(ctx, ctx->point_voxel.as<int>(), ctx->n_points, labels, capacity, on_device);
+}
+
+int f3ps_get_segment_points(f3ps_ctx* ctx, int level, int64_t* offsets, int32_t* point_index, int32_t capacity_segments, int64_t capacity_points,
+                            int on_device) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    int rc = segments_ready(ctx, level, true, "f3ps_get_segment_points"); if (rc) return rc;
+    if ((rc = segment_group(ctx, level, ctx->point_voxel.as<int>(), ctx->n_points, ctx->seg_points))) return rc;
+    return segment_copy(ctx, ctx->seg_points, offsets, point_index, capacity_segments, capacity_points, on_device);
+}
+
+int f3ps_get_segment_voxels(f3ps_ctx* ctx, int level, int64_t* offsets, int32_t* voxel_index, int32_t capacity_segments, int64_t capacity_voxels,
+                            int on_device) {
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    int rc = segments_ready(ctx, level, false, "f3ps_get_segment_voxels"); if (rc) return rc;
+    if ((rc = segment_group(ctx, level, nullptr, ctx->V, ctx->seg_voxels))) return rc;
+    return segment_copy(ctx, ctx->seg_voxels, offsets, voxel_index, capacity_segments, capacity_voxels, on_device);
+}
+
+int f3ps_get_segment_info(f3ps_ctx* ctx, int level, f3ps_segment_info* out, int32_t capacity) {
+    static_assert(sizeof(f3ps_segment_info) == 64, "f3ps_segment_info is 64 bytes");
+    if (!ctx) return F3PS_ERR_INVALID_ARGUMENT;
+    int rc = segments_ready(ctx, level, true, "f3ps_get_segment_info"); if (rc) return rc;
+    if ((rc = segment_group(ctx, level, ctx->point_voxel.as<int>(), ctx->n_points, ctx->seg_points)) ||
+        (rc = segment_group(ctx, level, nullptr, ctx->V, ctx->seg_voxels))) return rc;
+    const SegCsr& g = ctx->seg_points;
+    const unsigned K = g.K;
+    if ((rc = cap_check(ctx, K, capacity))) return rc;
+    if (!K) return F3PS_OK;
+    if (!out) return ctx_fail(ctx, F3PS_ERR_INVALID_ARGUMENT, "no output buffer");
+    const size_t chunks = ((size_t)g.n + kSegChunk - 1) / kSegChunk + K;     // >= the partials of all segments
+    F3PS_CUDA_OK(ctx->seg_part.ensure(chunks * sizeof(SegPartial))); F3PS_CUDA_OK(ctx->seg_info.ensure((size_t)K * sizeof(f3ps_segment_info)));
+    f3ps_segment_info* info = ctx->seg_info.as<f3ps_segment_info>();
+    PointLoader pl{ctx->d_points, ctx->stride, ctx->vp.fold_negative_z};
+    if (g.n) LAUNCH(ctx, segment_partials_kernel, (int)chunks, kSegThreads, 0, pl, g.index, g.off(), g.chunk_off(), K, ctx->seg_part.as<SegPartial>());
+    LAUNCH(ctx, segment_info_kernel, (int)(((size_t)K * 32 + 255) / 256), 256, 0, ctx->seg_part.as<SegPartial>(), g.chunk_off(), g.off(),
+           ctx->seg_voxels.off(), K, info);
+    if (ctx->S) LAUNCH(ctx, segment_region_kernel, grid_for(ctx->S, 256), 256, 0, ctx->lv_dense.as<unsigned>() + (size_t)level * ctx->S,
+                       ctx->sv_label.as<unsigned>(), ctx->S, info);
+    if ((rc = d2h(ctx, out, info, (size_t)K * sizeof(f3ps_segment_info)))) return rc;
+    return fin(ctx);
 }
 
 // ---- device self tests ------------------------------------------------------------------------------

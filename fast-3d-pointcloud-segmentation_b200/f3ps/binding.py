@@ -39,6 +39,16 @@ class Counts(C.Structure):
                 ("fold_steps", C.c_int64), ("nan_weights", C.c_int32), ("merge_path", C.c_int32)]
 
 
+class SegmentInfo(C.Structure):
+    """f3ps_segment_info, one 64-byte record per segment."""
+    _fields_ = [("region_label", C.c_uint32), ("n_voxels", C.c_int32), ("n_points", C.c_int64),
+                ("min_xyz", C.c_float * 3), ("max_xyz", C.c_float * 3), ("centroid", C.c_float * 3), ("mean_rgb", C.c_float * 3)]
+
+
+SEGMENT_INFO_DTYPE = np.dtype({"names": [f[0] for f in SegmentInfo._fields_],
+                               "formats": [np.uint32, np.int32, np.int64] + [(np.float32, 3)] * 4,
+                               "offsets": [getattr(SegmentInfo, f[0]).offset for f in SegmentInfo._fields_], "itemsize": 64})
+
 _lib = None
 
 
@@ -96,6 +106,9 @@ def lib():
         "f3ps_get_levels": (C.c_int, [vp, C.POINTER(i32), vp, vp, vp, i32]),
         "f3ps_get_level_voxel_labels": (C.c_int, [vp, vp, i64, C.c_int]),
         "f3ps_get_level_point_labels": (C.c_int, [vp, vp, i64, C.c_int]),
+        "f3ps_get_segment_points": (C.c_int, [vp, C.c_int, vp, vp, i32, i64, C.c_int]),
+        "f3ps_get_segment_voxels": (C.c_int, [vp, C.c_int, vp, vp, i32, i64, C.c_int]),
+        "f3ps_get_segment_info": (C.c_int, [vp, C.c_int, vp, i32]),
         "f3ps_stage_ms": (C.c_int, [vp, C.c_int, C.POINTER(f32)]),
         "f3ps_launch_count": (i64, [vp]),
         "f3ps_merge_profile": (C.c_int, [vp, C.POINTER(C.c_uint64 * 32)]),
@@ -137,7 +150,7 @@ EXPORTED = ["f3ps_create", "f3ps_destroy", "f3ps_last_error", "f3ps_version", "f
             "f3ps_get_supervoxels", "f3ps_get_supervoxel_voxels", "f3ps_get_adjacency", "f3ps_get_edges", "f3ps_get_cdf",
             "f3ps_get_merge_log", "f3ps_get_state_regions", "f3ps_get_state_edges", "f3ps_get_labeled_cloud", "f3ps_get_region_mean_color",
             "f3ps_get_voxel_segments_device", "f3ps_merge_levels", "f3ps_get_levels", "f3ps_get_level_voxel_labels",
-            "f3ps_get_level_point_labels", "f3ps_stage_ms", "f3ps_launch_count", "f3ps_merge_profile", "f3ps_merge_trace", "f3ps_expand_profile", "f3ps_test_rgb2lab",
+            "f3ps_get_level_point_labels", "f3ps_get_segment_points", "f3ps_get_segment_voxels", "f3ps_get_segment_info", "f3ps_stage_ms", "f3ps_launch_count", "f3ps_merge_profile", "f3ps_merge_trace", "f3ps_expand_profile", "f3ps_test_rgb2lab",
             "f3ps_test_lab_ciede00", "f3ps_test_rgb_eucl", "f3ps_test_sort_pairs",
             "f3ps_merge_batch", "f3ps_set_expand_sharing", "f3ps_set_expand_kernel", "f3ps_refine", "f3ps_eval_thresholds", "f3ps_eval_label_pairs", "f3ps_slab_reset", "f3ps_slab_bbox", "f3ps_slab_set_frame", "f3ps_slab_keys", "f3ps_slab_route", "f3ps_slab_array",
             "f3ps_slab_choose_splitters", "f3ps_slab_set_voxels"]
@@ -413,6 +426,45 @@ class Segmenter:
         """point_labels() into a CUDA buffer of `capacity` uint32 elements (e.g. a torch tensor's data_ptr()), enqueued on the
         handle's stream without waiting: sync() before reading it from another stream or the host."""
         self._chk(self.L.f3ps_get_level_point_labels(self.h, C.c_void_p(dev_ptr), capacity, 1))
+
+    # ---- segment extraction: the members of every segment of one level, and one descriptor per segment ----
+    def _level(self, level):
+        """level index of the recorded levels; negative counts from the end (out of range: the C call's ValueError)"""
+        return level + self._n_levels() if level < 0 else level
+
+    def _segments(self, fn, level, n_members):
+        k = self._level(level)
+        lv = self.levels()
+        K = int(lv["n_segments"][k]) if 0 <= k < len(lv["n_segments"]) else 0
+        off = np.empty(K + 1, np.int64); idx = np.empty(n_members, np.int32)
+        self._chk(fn(self.h, k, _p(off), _p(idx), off.size, idx.size, 0))
+        return off, idx[:off[-1]]
+
+    def segment_points(self, level=-1):
+        """(offsets int64 [K+1], index int32 [n]): the input points of segment j of the level at index[offsets[j]:offsets[j+1]],
+        ascending; points without a segment are left out."""
+        return self._segments(self.L.f3ps_get_segment_points, level, self.counts().n_points)
+
+    def segment_voxels(self, level=-1):
+        """segment_points() over voxels (after set_graph voxel i is the i-th voxel passed in)."""
+        return self._segments(self.L.f3ps_get_segment_voxels, level, self.counts().n_voxels)
+
+    def segment_points_device(self, level, offsets_ptr, index_ptr, cap_segments, cap_points):
+        """segment_points() into CUDA buffers (e.g. torch tensors' data_ptr(): int64 offsets, int32 index), enqueued on the
+        handle's stream: sync() before reading them from another stream or the host."""
+        self._chk(self.L.f3ps_get_segment_points(self.h, self._level(level), C.c_void_p(offsets_ptr), C.c_void_p(index_ptr),
+                                                 cap_segments, cap_points, 1))
+
+    def segment_info(self, level=-1):
+        """One descriptor per segment of the level, as numpy arrays: region_label, n_voxels, n_points, min_xyz, max_xyz, centroid,
+        mean_rgb (the last four [K, 3] float32)."""
+        k = self._level(level)
+        n = self._n_levels()
+        K = int(self.levels()["n_segments"][k]) if 0 <= k < n else 0
+        recs = (SegmentInfo * max(K, 1))()
+        self._chk(self.L.f3ps_get_segment_info(self.h, k, recs, K))
+        a = np.frombuffer(recs, SEGMENT_INFO_DTYPE, count=K)
+        return {name: np.ascontiguousarray(a[name]) for name in a.dtype.names}
 
     def supervoxel_voxels(self):
         c = self.counts()

@@ -10,7 +10,8 @@
 // classes instead of the fused path, --gpus N shards the files of a -d sweep over N GPUs (no collective), --inflight K =
 // files per group of a sweep: K1..K6 of a file on its own handle + stream, ONE merge launch per group (f3ps_merge_batch),
 // the next group's front stages overlapping it.  --levels t1,t2,... prints the segmentation at several thresholds from one
-// extra merge replay, --point-labels <file.pcd> writes the input cloud with every point's segment (one file per level).
+// extra merge replay, --point-labels <file.pcd> writes the input cloud with every point's segment (one file per level),
+// --segments <file.csv> writes one row per segment (point and voxel counts, bounds, centroid, mean colour) of every level.
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -47,7 +48,7 @@ struct Options {
     float thresh = 0; bool thresh_specified = true; bool rgb = false, cvx = false, ml = false, al = false, eq = false, disable_transform = false, verbose = false, facade = false;
     float lambda = 0; int bin_num = 0; std::string out;
     bool remove_label = false; uint32_t label_to_be_removed = 0; std::string test_filename = "test"; bool eval = true;
-    std::vector<float> levels; std::string point_labels;
+    std::vector<float> levels; std::string point_labels, segments;
 };
 struct FileScores { bool have_best = false; f3ps_performance best; std::vector<std::pair<float, f3ps_performance>> all; };
 
@@ -74,6 +75,8 @@ void usage(const char* a0) {
            "\t -o <file.pcd>                  (writes the labelled voxel cloud) \n"
            "\t --levels <t1,t2,...>           (prints the segment counts at these ascending thresholds, one extra merge replay) \n"
            "\t --point-labels <file.pcd>      (writes every input point with its segment; with --levels one file <stem>_<k>.pcd per level)\n"
+           "\t --segments <file.csv>          (writes one row per segment: counts, bounds, centroid and mean colour of its points; with\n"
+           "\t                                 --levels the segments of every level in the one file) \n"
            "\t --facade                       (runs through the Clustering / SupervoxelClustering classes) \n"
            "\t --gpus <N>                     (shards the files of -d over N GPUs) \n"
            "\t --inflight <K>                 (frames in flight per GPU during a -d sweep, default 8) \n"
@@ -372,7 +375,7 @@ int process_file(const std::string& file, const Options& o, int device, std::str
         return (op.parent_path() / (std::filesystem::path(file).stem().string() + "_" + op.filename().string())).string();
     };
     if (!o.out.empty()) f3ps::savePCDFileASCII(per_file(o.out), *labeled);
-    if (hp && (!o.levels.empty() || !o.point_labels.empty())) {         // one more replay; the segmentation above stays f3ps_merge(thresh)'s
+    if (hp && (!o.levels.empty() || !o.point_labels.empty() || !o.segments.empty())) {         // one more replay; the segmentation above stays f3ps_merge(thresh)'s
         f3ps::Handle& h = *hp;
         const std::vector<float> thr = o.levels.empty() ? std::vector<float>(1, thresh) : o.levels;
         h.check(f3ps_merge_levels(h.get(), thr.data(), (int)thr.size()));
@@ -397,6 +400,23 @@ int process_file(const std::string& file, const Options& o, int device, std::str
                     : (base.parent_path() / (base.stem().string() + "_" + std::to_string(k) + base.extension().string())).string();
                 f3ps::savePCDFileASCII(name, pc);
             }
+        }
+        if (!o.segments.empty()) {
+            const std::string name = per_file(o.segments);
+            FILE* f = fopen(name.c_str(), "w");
+            if (!f) throw std::runtime_error("cannot write " + name);
+            fprintf(f, "level,threshold,segment,region_label,n_points,n_voxels,min_x,min_y,min_z,max_x,max_y,max_z,cx,cy,cz,r,g,b\n");
+            for (int k = 0; k < L; ++k) {
+                std::vector<f3ps_segment_info> info((size_t)ns[k]);
+                h.check(f3ps_get_segment_info(h.get(), k, info.data(), ns[k]));
+                for (int j = 0; j < ns[k]; ++j) {
+                    const f3ps_segment_info& q = info[(size_t)j];
+                    fprintf(f, "%d,%.9g,%d,%u,%lld,%d,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g,%.9g\n", k, thr[k], j, q.region_label,
+                            (long long)q.n_points, q.n_voxels, q.min_xyz[0], q.min_xyz[1], q.min_xyz[2], q.max_xyz[0], q.max_xyz[1], q.max_xyz[2],
+                            q.centroid[0], q.centroid[1], q.centroid[2], q.mean_rgb[0], q.mean_rgb[1], q.mean_rgb[2]);
+                }
+            }
+            fclose(f);
         }
     }
     return 0;
@@ -502,8 +522,9 @@ int main(int argc, char** argv) {
         if (o.levels.empty()) { fprintf(stderr, "--levels takes comma-separated thresholds\n"); return 1; }
     }
     parse(argc, argv, "--point-labels", o.point_labels);
-    if ((!o.levels.empty() || !o.point_labels.empty()) && (o.facade || find_switch(argc, argv, "--slabs"))) {
-        fprintf(stderr, "--levels and --point-labels run on the direct path of one GPU per file: drop --facade / --slabs\n"); return 1;
+    parse(argc, argv, "--segments", o.segments);
+    if ((!o.levels.empty() || !o.point_labels.empty() || !o.segments.empty()) && (o.facade || find_switch(argc, argv, "--slabs"))) {
+        fprintf(stderr, "--levels, --point-labels and --segments run on the direct path of one GPU per file: drop --facade / --slabs\n"); return 1;
     }
     int gpus = 1; parse(argc, argv, "--gpus", gpus); gpus = std::max(1, gpus);
     int inflight = 8; parse(argc, argv, "--inflight", inflight); inflight = std::max(1, inflight);
@@ -522,9 +543,9 @@ int main(int argc, char** argv) {
             // -d sweep: files are independent (fresh SupervoxelClustering + Clustering per file in the reference, :348,408).
             // `inflight` frames per GPU, each on its own handle / stream / host thread; reports are printed in file order.
             std::mutex emu; std::string first_error;
-            if (o.thresh_specified && o.out.empty() && o.levels.empty() && o.point_labels.empty()) {
-                // groups of `inflight` files per GPU: front stages per file, ONE merge launch per group (-o, --levels and
-                // --point-labels need the per-file path below)
+            if (o.thresh_specified && o.out.empty() && o.levels.empty() && o.point_labels.empty() && o.segments.empty()) {
+                // groups of `inflight` files per GPU: front stages per file, ONE merge launch per group (-o, --levels,
+                // --point-labels and --segments need the per-file path below)
                 std::vector<std::vector<size_t>> share((size_t)gpus);
                 for (size_t i = 0; i < file_list.size(); ++i) share[i % (size_t)gpus].push_back(i);
                 std::vector<std::thread> th;

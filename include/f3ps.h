@@ -214,6 +214,36 @@ int f3ps_get_levels(f3ps_ctx* ctx, int32_t* n_levels, float* thresholds, int32_t
 int f3ps_get_level_voxel_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacity, int on_device);
 int f3ps_get_level_point_labels(f3ps_ctx* ctx, uint32_t* labels, int64_t capacity, int on_device);
 
+/* ---- segment extraction: the members of every segment of one level, grouped, and one descriptor per segment ----
+ * `level` = 0..L-1 indexes the handle's recorded levels (f3ps_get_levels); segments are that level's dense labels 0..K-1, as
+ * f3ps_get_level_{voxel,point}_labels number them.  Before any merge: F3PS_ERR_LOGIC; a level out of range or a short buffer:
+ * F3PS_ERR_INVALID_ARGUMENT.  The handle keeps the grouping of the last level asked for (points and voxels each) until the next
+ * merge, so f3ps_get_segment_info after f3ps_get_segment_points on the same level does not group again.  Grouping a level waits
+ * once for its two sizes (members, segments).  on_device != 0: `offsets` / the index array are device memory and the copy into
+ * them is enqueued on the handle's stream without a wait; on_device == 0: host memory, read straight from the kept grouping. */
+/* points of every segment: offsets[K+1] (offsets[0] = 0, non-decreasing), point_index[offsets[K]] with the points of segment j
+ * at [offsets[j], offsets[j+1]) in ascending input order.  Points without a voxel and points whose voxel no supervoxel owns are
+ * in no segment.  F3PS_ERR_LOGIC after f3ps_set_graph and in slab mode (as point labels). */
+int f3ps_get_segment_points(f3ps_ctx* ctx, int level, int64_t* offsets, int32_t* point_index,
+                            int32_t capacity_segments /* >= K+1 */, int64_t capacity_points, int on_device);
+/* the same over voxels: voxel indices in ascending order (after f3ps_set_graph voxel i is the i-th voxel passed in); works
+ * wherever voxel labels do, slab mode and f3ps_set_graph included */
+int f3ps_get_segment_voxels(f3ps_ctx* ctx, int level, int64_t* offsets, int32_t* voxel_index,
+                            int32_t capacity_segments, int64_t capacity_voxels, int on_device);
+/* One record per segment, host memory, capacity in records (>= K).  Needs the handle's input cloud (F3PS_ERR_LOGIC after
+ * f3ps_set_graph and in slab mode); for input on the device it reads the caller's point buffer, which f3ps_set_input requires
+ * to stay valid until the next f3ps_set_input.  Sums are reduced in a fixed order (xyz in FP64, rgb in integers): the same
+ * bits from every call.  A segment without points (none today: every voxel holds a point) has NaN bounds, centroid and colour. */
+typedef struct f3ps_segment_info {
+    uint32_t region_label;   /* label of the surviving region (what f3ps_get_state_regions reports at the final level) */
+    int32_t  n_voxels;       /* voxels whose level label is this segment (a phantom leaf counts with its owner's) */
+    int64_t  n_points;       /* = offsets[j+1] - offsets[j] of f3ps_get_segment_points */
+    float    min_xyz[3], max_xyz[3];   /* bounds of its points, coordinates as the path sees them (z<0 -> |z| when folded) */
+    float    centroid[3];    /* mean xyz of its points */
+    float    mean_rgb[3];    /* mean r, g, b of its points, 0..255 */
+} f3ps_segment_info;         /* 64 bytes */
+int f3ps_get_segment_info(f3ps_ctx* ctx, int level, f3ps_segment_info* out, int32_t capacity);
+
 /* ---- slab mode: one very large cloud cut into spatial slabs, one per GPU (SURVEY.md section 8e; BASELINE config 5) ----
  * Replaces, for one scan too large or too slow for one device, the same calls as above
  * (pcl::SupervoxelClustering::extract, supervoxel_clustering.cpp:357).  A slab is a contiguous range of the x-major
