@@ -900,6 +900,7 @@ int merge_done(f3ps_ctx* ctx, float threshold) {
 enum MergeStart { kStartFresh, kStartContinue, kStartGeneral };
 int merge_one(f3ps_ctx* ctx, float threshold, MergeStart start) {
     int rc = merge_begin(ctx, start != kStartContinue); if (rc) return rc;
+    ctx->merge_path = 0;                                     // no supervoxels: no kernel runs (a reused handle must not report its last frame's)
     if (ctx->S) {
         MergePlan p = plan_merge(ctx);
         if (start == kStartGeneral) p.kind = kMergeGeneral;

@@ -71,7 +71,7 @@ typedef struct f3ps_counts {
     int32_t max_touched;   /* largest number of edges re-weighted by one merge */
     int64_t fold_steps;    /* voxel steps folded by the merge loop (sum of |b|) */
     int32_t nan_weights;   /* edge weights that evaluated to NaN (regions with < 3 voxels) */
-    int32_t merge_path;    /* kernel the last f3ps_merge ran: 1 = resident (one SM, weight map in shared memory), 2 = general (also: a resident replay that could not go on, replayed again from the start), 3 = resident with its tables in L2 (graphs too large for an SM), 6 = 1 up to the first merge with more than 928 adjacency entries, then 3 from that state */
+    int32_t merge_path;    /* kernel the last f3ps_merge ran: 0 = none (no supervoxels, or no merge yet), 1 = resident (one SM, weight map in shared memory), 2 = general (also: a resident replay that could not go on, replayed again from the start), 3 = resident with its tables in L2 (graphs too large for an SM), 6 = 1 up to the first merge with more than 928 adjacency entries, then 3 from that state */
 } f3ps_counts;
 
 /* ---- life cycle ------------------------------------------------------------ */
