@@ -9,8 +9,6 @@
 #include "kernels_expand.cuh"
 #include "kernels_slab.cuh"
 #include "kernels_graph.cuh"
-
-#define F3PS_MERGE_ERR_TOUCHED 4u
 #include "kernels_merge.cuh"
 #include "kernels_merge_lean.cuh"
 #include "kernels_eval.cuh"

@@ -788,12 +788,12 @@ int merge_restart(f3ps_ctx* ctx) {
     F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl), 0, sizeof(MergeCtl), ctx->stream));
     return F3PS_OK;
 }
-// start of a replay: restart (unless the working state is the one to continue from), merge log, output buffers
-int merge_begin(f3ps_ctx* ctx, bool restart) {
+// start of a replay: restart, merge log, output buffers
+int merge_begin(f3ps_ctx* ctx) {
     int rc = mark(ctx, 7); if (rc) return rc;
     ctx->lv_thr.clear(); ctx->lv_built = 0;
     ctx->seg_points.level = ctx->seg_voxels.level = -1;
-    if (restart && (rc = merge_restart(ctx))) return rc;
+    if ((rc = merge_restart(ctx))) return rc;
     const size_t Sc = std::max(1u, ctx->S), Pc = std::max(1u, ctx->n_pos);
     F3PS_CUDA_OK(ctx->mlog.ensure(Sc * 20));
     char* lp = (char*)ctx->mlog.p;
@@ -862,18 +862,6 @@ int launch_general(f3ps_ctx* ctx, float threshold) {
            SC(mctl), scr, (PK*)sp, ctx->pos_data);
     return F3PS_OK;
 }
-// Clustering::get_labeled_cloud: dense segment ids, then the labelled voxel cloud
-int merge_labels(f3ps_ctx* ctx) {
-    int rc = mark(ctx, 10); if (rc) return rc;
-    const unsigned P = ctx->n_pos;
-    LAUNCH(ctx, dense_label_kernel, 1, 1024, 0, ctx->R1, SC(xctl.n_sv), ctx->run_start.as<unsigned>(), ctx->run_end.as<unsigned>(), ctx->run_out_off.as<unsigned>(),
-           ctx->run_dense.as<unsigned>(), ctx->region_dense.as<unsigned>(), SC(n_out));
-    if (P) LAUNCH(ctx, labeled_cloud_kernel, grid_for(P, 256), 256, 0, ctx->pos_run.as<unsigned>(), P, ctx->order, ctx->run_start.as<unsigned>(),
-                  ctx->run_out_off.as<unsigned>(), ctx->run_dense.as<unsigned>(), ctx->gxyz, ctx->out_xyz.as<float>(), ctx->out_label.as<unsigned>(),
-                  ctx->out_voxel.as<unsigned>(), ctx->vox_segment.as<unsigned>(), ctx->graph_from_host ? nullptr : ctx->sorted_label,
-                  ctx->graph_from_host ? nullptr : ctx->owner0.as<unsigned>());
-    return F3PS_OK;
-}
 LabelArgs label_args(const f3ps_ctx* ctx) {
     LabelArgs A;
     A.R = ctx->R1; A.n_sv_ptr = SC(xctl.n_sv); A.run_start = ctx->run_start.as<unsigned>(); A.run_end = ctx->run_end.as<unsigned>();
@@ -895,51 +883,121 @@ int merge_done(f3ps_ctx* ctx, float threshold) {
     return F3PS_OK;
 }
 
-// kStartContinue: a batch grid stopped this frame in front of a merge with more adjacency entries than worker threads (the
-// working state and the counters are those after n merges).  kStartGeneral: the batch grid ran out of adjacency pool or stamps.
-enum MergeStart { kStartFresh, kStartContinue, kStartGeneral };
-int merge_one(f3ps_ctx* ctx, float threshold, MergeStart start) {
-    int rc = merge_begin(ctx, start != kStartContinue); if (rc) return rc;
-    ctx->merge_path = 0;                                     // no supervoxels: no kernel runs (a reused handle must not report its last frame's)
+// stage mark i of every frame of a chunk, on the stream of its first frame (the lead), which runs the chunk's kernels
+int mark_chunk(f3ps_ctx** ctxs, const std::vector<int>& chunk, int i) {
+    f3ps_ctx* ctx = ctxs[chunk[0]];
+    for (int f : chunk) { F3PS_CUDA_OK(cudaEventRecord(ctxs[f]->ev[i], ctx->stream)); ctxs[f]->ev_valid[i] = true; }
+    return F3PS_OK;
+}
+// One round of a chunk on its lead's stream, without a host wait: the merge kernel (a grid whose CTA k replays frame k, or the
+// frame's own kernel), then -- with supervoxels -- Clustering::get_labeled_cloud (dense segment ids, the labelled voxel cloud),
+// then the scalars' read-back (a chunk of one copies its own; a grid gathers every frame's on the device for one copy).
+int launch_chunk(f3ps_ctx** ctxs, const std::vector<int>& chunk, const std::vector<MergePlan>& step, const std::vector<char>& resume,
+                 float threshold) {
+    static thread_local FastBatch B;                         // 32 KB each: not on the stack
+    static thread_local LabelBatch L;
+    f3ps_ctx* ctx = ctxs[chunk[0]];
+    const unsigned nf = (unsigned)chunk.size();
+    int rc;
     if (ctx->S) {
-        MergePlan p = plan_merge(ctx);
-        if (start == kStartGeneral) p.kind = kMergeGeneral;
-        ctx->merge_path = p.kind;
-        rc = mark(ctx, 9); if (rc) return rc;
-        if (p.kind != kMergeGeneral) {
-            unsigned err = kFastErrTouched;
-            if (start == kStartFresh) {
-                rc = launch_resident(ctx, p, threshold, false); if (rc) return rc;
-                rc = pull_scalars(ctx); if (rc) return rc;   // did the resident kernel finish?
-                err = ctx->h_sc->mctl.error;
+        if (nf > 1) {
+            size_t bytes = 0;                                // every frame brings its own table capacities (the layout is per CTA)
+            for (unsigned k = 0; k < nf; ++k) {
+                f3ps_ctx* m = ctxs[chunk[k]];
+                rc = fast_args(m, step[chunk[k]], threshold, false, B.a[k]); if (rc) return rc;
+                bytes = std::max(bytes, step[chunk[k]].smem);
+                if (m->stream != ctx->stream) {              // the lead's stream runs the grid: it waits for everybody's set-up
+                    F3PS_CUDA_OK(cudaEventRecord(m->ev_batch, m->stream));
+                    F3PS_CUDA_OK(cudaStreamWaitEvent(ctx->stream, m->ev_batch, 0));
+                }
             }
-            // The shared-memory variant stops IN FRONT of a merge whose two adjacency lists hold more entries than it has worker
-            // threads (nothing of that merge has happened): the L2 variant continues from that state.
-            if (err == kFastErrTouched && p.to_l2) {
-                F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl.error), 0, 4, ctx->stream));
-                p = plan_l2(ctx);
-                ctx->merge_path = 6;
-                rc = launch_resident(ctx, p, threshold, true); if (rc) return rc;
-                rc = pull_scalars(ctx); if (rc) return rc;
-                err = ctx->h_sc->mctl.error;
-            }
-            // Any other stop (adjacency pool or stamp range exhausted, a merge with more than 65,534 entries on the L2 variant): the
-            // general kernel replays the whole sequence from the initial state.
-            if (err) {
-                rc = merge_restart(ctx); if (rc) return rc;
-                p.kind = kMergeGeneral;
-                ctx->merge_path = kMergeGeneral;
-            }
-        }
-        if (p.kind == kMergeGeneral) {
-            rc = ctx->S < 65536u ? launch_general<unsigned>(ctx, threshold) : launch_general<unsigned long long>(ctx, threshold);
+            rc = smem_opt_in(ctx, (const void*)merge_fast_batch_kernel, kSmemMax); if (rc) return rc;
+            LAUNCH(ctx, merge_fast_batch_kernel, nf, kFastThreads, bytes, B);
+        } else {
+            const MergePlan& p = step[chunk[0]];
+            rc = p.kind != kMergeGeneral ? launch_resident(ctx, p, threshold, resume[chunk[0]])
+               : ctx->S < 65536u ? launch_general<unsigned>(ctx, threshold) : launch_general<unsigned long long>(ctx, threshold);
             if (rc) return rc;
         }
-        rc = merge_labels(ctx); if (rc) return rc;
+        rc = mark_chunk(ctxs, chunk, 10); if (rc) return rc;
+        int gx = 1;
+        for (unsigned k = 0; k < nf; ++k) {
+            f3ps_ctx* m = ctxs[chunk[k]];
+            m->merge_path = resume[chunk[k]] ? 6 : step[chunk[k]].kind;
+            L.a[k] = label_args(m);
+            gx = std::max(gx, grid_for(m->n_pos, 256));
+        }
+        LAUNCH(ctx, dense_label_batch_kernel, nf, 1024, 0, L);
+        LAUNCH(ctx, labeled_cloud_batch_kernel, dim3(gx, nf), 256, 0, L);
     }
-    rc = mark(ctx, 8); if (rc) return rc;
-    rc = pull_scalars(ctx); if (rc) return rc;
-    return merge_done(ctx, threshold);
+    rc = mark_chunk(ctxs, chunk, 8); if (rc) return rc;
+    if (nf == 1) {
+        F3PS_CUDA_OK(cudaMemcpyAsync(ctx->h_sc, ctx->d_sc, sizeof(DevScalars), cudaMemcpyDeviceToHost, ctx->stream));
+        return F3PS_OK;
+    }
+    static_assert(sizeof(DevScalars) % 4 == 0, "DevScalars is gathered as words");
+    F3PS_CUDA_OK(ctx->batch_sc.ensure(kFastBatchMax * sizeof(DevScalars)));
+    if (!ctx->h_batch_sc) F3PS_CUDA_OK(cudaMallocHost(&ctx->h_batch_sc, kFastBatchMax * sizeof(DevScalars)));
+    LAUNCH(ctx, scalars_gather_kernel, nf, 128, 0, L, (unsigned)(sizeof(DevScalars) / 4), ctx->batch_sc.as<unsigned>());
+    F3PS_CUDA_OK(cudaMemcpyAsync(ctx->h_batch_sc, ctx->batch_sc.p, nf * sizeof(DevScalars), cudaMemcpyDeviceToHost, ctx->stream));
+    return F3PS_OK;
+}
+// Clustering::cluster(threshold) of n handles on one device, graphs built: f3ps_merge (n = 1) and f3ps_merge_batch.
+// The replay runs in rounds, one step per frame and round: a fresh replay from the frame's plan; a continuation on the L2 variant
+// (merge_path 6) when the shared-memory variant stopped IN FRONT of a merge whose two adjacency lists hold more entries than it
+// has worker threads (nothing of that merge has happened); or, after any other stop (adjacency pool or stamp range exhausted, a
+// merge with more than 65,534 entries on the L2 variant), the general kernel replaying the whole sequence from the initial state.
+// Fresh frames of the shared-memory kernel without phase counters share grids of at most kFastBatchMax frames: independent
+// streams share at most 32 hardware queues, so at most 32 single-CTA merge kernels overlap, and a grid has no such cap.  Every
+// other frame, one left alone in its chunk included, is a chunk of one that runs its plan's own kernel on its own stream.  The
+// host waits only after every chunk of a round is in flight.
+//
+// No member stream waits for a grid: a stream parked behind a grid that runs for tens of milliseconds would hold its hardware
+// queue, and the work other handles enqueue on that queue (the next group's front stages in a pipelined sweep) would wait for
+// the grid too.  The call returns only after the host has seen every lead stream finish, so later work on a member's own stream
+// (getters, levels, the next frame) needs no event wait.
+int merge_frames(f3ps_ctx** ctxs, int n, float threshold) {
+    std::vector<MergePlan> step(n);                          // each frame's kernel in the current round
+    std::vector<char> resume(n, 0);                          // that kernel continues from the stopped state
+    std::vector<int> grid, single;
+    for (int i = 0; i < n; ++i) {
+        f3ps_ctx* ctx = ctxs[i];
+        int rc = merge_begin(ctx); if (rc) return rc;
+        ctx->merge_path = 0;                                 // no supervoxels: no kernel runs (a reused handle must not report its last frame's)
+        step[i] = plan_merge(ctx);
+        if (ctx->S && (rc = mark(ctx, 9))) return rc;
+        (ctx->S && step[i].kind == kMergeShared && !step[i].prof ? grid : single).push_back(i);
+    }
+    std::vector<std::vector<int>> chunks;
+    for (size_t g0 = 0; g0 < grid.size(); g0 += kFastBatchMax)
+        chunks.emplace_back(grid.begin() + g0, grid.begin() + std::min(grid.size(), g0 + (size_t)kFastBatchMax));
+    for (int i : single) chunks.push_back({i});
+    while (!chunks.empty()) {
+        for (const auto& c : chunks) { int rc = launch_chunk(ctxs, c, step, resume, threshold); if (rc) return rc; }
+        std::vector<std::vector<int>> next;
+        for (const auto& c : chunks) {
+            f3ps_ctx* lead = ctxs[c[0]];
+            { f3ps_ctx* ctx = lead; F3PS_CUDA_OK(wait_stream(ctx)); }
+            for (size_t k = 0; k < c.size(); ++k) {
+                f3ps_ctx* ctx = ctxs[c[k]];
+                MergePlan& p = step[c[k]];
+                if (c.size() > 1) memcpy(ctx->h_sc, lead->h_batch_sc + k, sizeof(DevScalars));
+                int rc;
+                if (!ctx->h_sc->mctl.error || p.kind == kMergeGeneral) { if ((rc = merge_done(ctx, threshold))) return rc; continue; }
+                resume[c[k]] = ctx->h_sc->mctl.error == kFastErrTouched && p.to_l2;
+                if (resume[c[k]]) {
+                    F3PS_CUDA_OK(cudaMemsetAsync(SC(mctl.error), 0, 4, ctx->stream));
+                    p = plan_l2(ctx);
+                } else {
+                    if ((rc = merge_restart(ctx))) return rc;
+                    p.kind = kMergeGeneral;
+                }
+                next.push_back({c[k]});
+            }
+        }
+        chunks.swap(next);
+    }
+    return F3PS_OK;
 }
 }
 }
@@ -949,20 +1007,10 @@ int f3ps_merge(f3ps_ctx* ctx, float threshold) {
         return ctx_fail(ctx, F3PS_ERR_LOGIC, "Cannot call 'cluster' before setting an initial state with 'set_initialstate'");
     cudaSetDevice(ctx->device);
     if (ctx->progress < P_GRAPH) { int rc = f3ps_graph(ctx); if (rc) return rc; }   // if (!init_initial_weights) init_weights()  (:675-676)
-    return merge_one(ctx, threshold, kStartFresh);
+    return merge_frames(&ctx, 1, threshold);
 }
 
-// Clustering::cluster(threshold) for MANY frames with ONE launch of the resident merge kernel: CTA i of the grid replays frame i.
-// A sweep that keeps frames in flight on independent streams is capped by the 32 hardware queues of a context (at most 32
-// single-CTA merge kernels overlap); one grid of n CTAs runs n frames side by side.  Every handle must be on the same device,
-// with its graph built (f3ps_graph); handles whose plan is not the shared-memory kernel without phase counters run on their own.
-// Results per handle are exactly those of f3ps_merge(handle, threshold).
-//
-// Everything that follows a chunk's grid (labelled clouds, the scalars' read-back, the stage marks 10 and 8 of every frame) runs
-// on the lead's stream, as launches over the whole chunk.  No member stream waits for the grid: a stream parked behind a grid
-// that runs for tens of milliseconds would hold its hardware queue, and the work other handles enqueue on that queue (the next
-// group's front stages in a pipelined sweep) would wait for the grid too.  The function returns only after the host has seen
-// every lead stream finish, so later work on a member's own stream (getters, levels, the next frame) needs no event wait.
+// Every handle must be on the same device; the results per handle are exactly those of f3ps_merge(handle, threshold).
 int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
     if (!ctxs || n < 1) return F3PS_ERR_INVALID_ARGUMENT;
     for (int i = 0; i < n; ++i) {
@@ -972,78 +1020,9 @@ int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold) {
             return ctx_fail(ctxs[i], F3PS_ERR_LOGIC, "Cannot call 'cluster' before setting an initial state with 'set_initialstate'");
     }
     cudaSetDevice(ctxs[0]->device);
-    int rc;
-    std::vector<int> batch, solo;
-    std::vector<MergePlan> plans(n);
-    for (int i = 0; i < n; ++i) {
-        f3ps_ctx* ctx = ctxs[i];
-        if (ctx->progress < P_GRAPH) { rc = f3ps_graph(ctx); if (rc) return rc; }
-        plans[i] = plan_merge(ctx);
-        (ctx->S > 0 && plans[i].kind == kMergeShared && !plans[i].prof ? batch : solo).push_back(i);
-    }
-    const size_t sc_words = sizeof(DevScalars) / 4;
-    static_assert(sizeof(DevScalars) % 4 == 0, "DevScalars is gathered as words");
-    for (size_t g0 = 0; g0 < batch.size(); g0 += kFastBatchMax) {
-        const size_t g1 = std::min(batch.size(), g0 + (size_t)kFastBatchMax);
-        const unsigned nf = (unsigned)(g1 - g0);
-        static thread_local FastBatch B;                     // 32 KB: not on the stack
-        static thread_local LabelBatch L;
-        size_t bytes = 0;                                    // every frame brings its own table capacities (the layout is per CTA)
-        f3ps_ctx* lead = ctxs[batch[g0]];
-        for (size_t k = g0; k < g1; ++k) {
-            f3ps_ctx* ctx = ctxs[batch[k]];
-            const MergePlan& p = plans[batch[k]];
-            rc = merge_begin(ctx, true); if (rc) return rc;
-            rc = fast_args(ctx, p, threshold, false, B.a[k - g0]); if (rc) return rc;
-            bytes = std::max(bytes, p.smem);
-            rc = mark(ctx, 9); if (rc) return rc;
-            if (ctx->stream != lead->stream) {               // the lead's stream runs the grid: it waits for everybody's set-up
-                F3PS_CUDA_OK(cudaEventRecord(ctx->ev_batch, ctx->stream));
-                F3PS_CUDA_OK(cudaStreamWaitEvent(lead->stream, ctx->ev_batch, 0));
-            }
-        }
-        f3ps_ctx* ctx = lead;
-        rc = smem_opt_in(ctx, (const void*)merge_fast_batch_kernel, kSmemMax); if (rc) return rc;
-        LAUNCH(ctx, merge_fast_batch_kernel, nf, kFastThreads, bytes, B);
-        int gx = 1;
-        for (size_t k = g0; k < g1; ++k) {
-            f3ps_ctx* m = ctxs[batch[k]];
-            F3PS_CUDA_OK(cudaEventRecord(m->ev[10], lead->stream)); m->ev_valid[10] = true;
-            m->merge_path = kMergeShared;
-            L.a[k - g0] = label_args(m);
-            gx = std::max(gx, grid_for(m->n_pos, 256));
-        }
-        LAUNCH(ctx, dense_label_batch_kernel, nf, 1024, 0, L);
-        LAUNCH(ctx, labeled_cloud_batch_kernel, dim3(gx, nf), 256, 0, L);
-        for (size_t k = g0; k < g1; ++k) {
-            f3ps_ctx* m = ctxs[batch[k]];
-            F3PS_CUDA_OK(cudaEventRecord(m->ev[8], lead->stream)); m->ev_valid[8] = true;
-        }
-        F3PS_CUDA_OK(lead->batch_sc.ensure(kFastBatchMax * sizeof(DevScalars)));
-        if (!lead->h_batch_sc) F3PS_CUDA_OK(cudaMallocHost(&lead->h_batch_sc, kFastBatchMax * sizeof(DevScalars)));
-        LAUNCH(ctx, scalars_gather_kernel, nf, 128, 0, L, (unsigned)sc_words, lead->batch_sc.as<unsigned>());
-        F3PS_CUDA_OK(cudaMemcpyAsync(lead->h_batch_sc, lead->batch_sc.p, nf * sizeof(DevScalars), cudaMemcpyDeviceToHost, lead->stream));
-    }
-    // the other handles one by one, next to the grids already in flight
-    for (int i : solo) { rc = merge_one(ctxs[i], threshold, kStartFresh); if (rc) return rc; }
-    // results only after EVERY chunk's grid is in flight (a batch larger than one parameter block must not run its chunks back to back);
-    // a frame whose CTA stopped continues alone
-    for (size_t g0 = 0; g0 < batch.size(); g0 += kFastBatchMax) {
-        const size_t g1 = std::min(batch.size(), g0 + (size_t)kFastBatchMax);
-        f3ps_ctx* lead = ctxs[batch[g0]];
-        {
-            f3ps_ctx* ctx = lead;
-            F3PS_CUDA_OK(wait_stream(ctx));
-        }
-        for (size_t k = g0; k < g1; ++k) {
-            f3ps_ctx* ctx = ctxs[batch[k]];
-            memcpy(ctx->h_sc, lead->h_batch_sc + (k - g0), sizeof(DevScalars));
-            const unsigned err = ctx->h_sc->mctl.error;
-            rc = err ? merge_one(ctx, threshold, err == kFastErrTouched ? kStartContinue : kStartGeneral) : merge_done(ctx, threshold);
-            if (rc) return rc;
-        }
-    }
-    return F3PS_OK;
+    for (int i = 0; i < n; ++i)
+        if (ctxs[i]->progress < P_GRAPH) { int rc = f3ps_graph(ctxs[i]); if (rc) return rc; }
+    return merge_frames(ctxs, n, threshold);
 }
 
 // ctas_per_frame = 0: K5's cooperative grid covers the whole GPU (lowest latency for a single frame, the default);

@@ -6,7 +6,7 @@
 //   dense   one block per level: dense label of every root alive after m_k merges, ascending rank = ascending label
 //   roots   one thread per supervoxel walks the levels in ascending order, each walk continuing from the previous root
 //           (a root at m_k is an ancestor of the one at m_{k-1}): seg[s][k] = dense label of s's region at level k
-//   voxels  positions -> voxel table [V][Lp] with the owner rule of labeled_cloud_kernel (a phantom leaf keeps its owner's)
+//   voxels  positions -> voxel table [V][Lp] with the owner rule of labeled_cloud_batch_kernel (a phantom leaf keeps its owner's)
 //   points  out[k][p] = table[point_voxel[p]][k], the HBM-bound gather
 // f3ps_eval_thresholds uses the first four stages for its contingency tables.
 #pragma once

@@ -497,76 +497,4 @@ __global__ void __launch_bounds__(kMergeThreads, 1) merge_kernel(RegionArrays R,
     }
 }
 
-// ---- result extraction: Clustering::get_labeled_cloud (:640-663) ---------------------------------
-// dense labels 0..K-1 in ascending region label order; output offset of every run of every rope.
-// One block: two exclusive scans over the regions (alive flag -> dense label, voxel count -> output offset), then one
-// thread per surviving region walks its rope.
-// The bodies are shared with the batched kernels of f3ps_merge_batch (kernels_merge_lean.cuh), one frame per CTA / grid row.
-__device__ __forceinline__ void dense_label_body(RegionArrays R, const unsigned* __restrict__ n_sv_ptr, const unsigned* __restrict__ run_start,
-        const unsigned* __restrict__ run_end, unsigned* __restrict__ run_out_off, unsigned* __restrict__ run_dense,
-        unsigned* __restrict__ region_dense, unsigned* __restrict__ n_out) {
-    __shared__ unsigned s_wa[32], s_wn[32];
-    __shared__ unsigned s_ca, s_cn;
-    const unsigned S = *n_sv_ptr;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) { s_ca = 0; s_cn = 0; }
-    __syncthreads();
-    for (unsigned base = 0; base < S; base += blockDim.x) {
-        const unsigned s = base + threadIdx.x;
-        const int nv = s < S ? R.n[s] : 0;
-        const unsigned alive = nv > 0 ? 1u : 0u, cnt = nv > 0 ? (unsigned)nv : 0u;
-        unsigned ia = alive, in = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned ta = __shfl_up_sync(kFull, ia, o), tn = __shfl_up_sync(kFull, in, o);
-            if (lane >= o) { ia += ta; in += tn; }
-        }
-        if (lane == 31) { s_wa[warp] = ia; s_wn[warp] = in; }
-        __syncthreads();
-        unsigned wa = 0, wn = 0;
-        for (int w = 0; w < warp; ++w) { wa += s_wa[w]; wn += s_wn[w]; }
-        const unsigned ca = s_ca, cn = s_cn;
-        if (s < S) {
-            if (!alive) region_dense[s] = 0xffffffffu;
-            else {
-                const unsigned dense = ca + wa + ia - 1u;
-                unsigned off = cn + wn + in - cnt;
-                region_dense[s] = dense;
-                for (int run = R.head[s]; run >= 0; run = R.next_run[run]) {
-                    run_out_off[run] = off; run_dense[run] = dense;
-                    off += run_end[run] - run_start[run];
-                }
-            }
-        }
-        __syncthreads();
-        if (threadIdx.x == blockDim.x - 1) { s_ca = ca + wa + ia; s_cn = cn + wn + in; }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *n_out = s_cn;
-}
-__global__ void __launch_bounds__(1024) dense_label_kernel(RegionArrays R, const unsigned* __restrict__ n_sv_ptr, const unsigned* __restrict__ run_start,
-        const unsigned* __restrict__ run_end, unsigned* __restrict__ run_out_off, unsigned* __restrict__ run_dense,
-        unsigned* __restrict__ region_dense, unsigned* __restrict__ n_out) {
-    dense_label_body(R, n_sv_ptr, run_start, run_end, run_out_off, run_dense, region_dense, n_out);
-}
-// The loop of labeled_cloud_kernel, over the names of its parameters.  A macro rather than a function: inlined, a function's
-// __restrict__ parameters no longer let the compiler load owner[] through the non-coherent path.
-#define F3PS_LABELED_CLOUD_LOOP                                                                                                    \
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += gridDim.x * blockDim.x) {                                \
-        const unsigned run = pos_run[i];                                                                                           \
-        if (run == 0xffffffffu) continue;                 /* unowned voxel: absent from every region */                            \
-        const unsigned o = run_out_off[run] + (i - run_start[run]);                                                                \
-        const unsigned v = order[i];                                                                                               \
-        const float4 p = vox_xyz[v];                                                                                               \
-        out_xyz[3 * (size_t)o] = p.x; out_xyz[3 * (size_t)o + 1] = p.y; out_xyz[3 * (size_t)o + 2] = p.z;                          \
-        out_label[o] = run_dense[run]; out_voxel[o] = v;                                                                           \
-        if (!owner || owner[v] == pos_label[i]) vox_segment[v] = run_dense[run];   /* a phantom leaf does not relabel its voxel */ \
-    }
-__global__ void __launch_bounds__(256) labeled_cloud_kernel(const unsigned* __restrict__ pos_run, unsigned n_pos, const unsigned* __restrict__ order,
-        const unsigned* __restrict__ run_start, const unsigned* __restrict__ run_out_off, const unsigned* __restrict__ run_dense,
-        const float4* __restrict__ vox_xyz, float* __restrict__ out_xyz, unsigned* __restrict__ out_label, unsigned* __restrict__ out_voxel,
-        unsigned* __restrict__ vox_segment, const unsigned* __restrict__ pos_label, const unsigned* __restrict__ owner) {
-    F3PS_LABELED_CLOUD_LOOP
-}
-
 } // namespace f3ps

@@ -24,7 +24,7 @@
 // BIG -- the per-edge / per-region tables in global memory with per-block minima in shared memory (S < 65535, 32-bit edge ids,
 // E bounded by 16 bytes of shared memory per block of 32 edges: C4 / C5-size scenes).  Shared-memory variant: a merge whose two
 // adjacency lists hold more than 928 entries is not started: every role stops in front of it, the state written back is that
-// after n merges, and the host relaunches the BIG variant from that state with A.resume (f3ps.cu: merge_one).  BIG variant:
+// after n merges, and the host relaunches the BIG variant from that state with A.resume (f3ps.cu: merge_frames).  BIG variant:
 // such a merge runs in lean_wide_merge (every worker thread loops over the entries, per-entry state in a global scratch); it
 // stops only in front of a merge with more than 65,534 entries.  That stop, an exhausted adjacency pool or an exhausted stamp
 // range makes the host replay the whole sequence again on merge_kernel (kernels_merge.cuh), from the initial state.
@@ -44,7 +44,7 @@ constexpr int kLeanRing = 2, kLeanSlotVox = 256;     // (four slots measured no 
 constexpr unsigned kDeadKey = 0xffffffffu;
 constexpr unsigned long long kDeadKey64 = ~0ull;
 constexpr unsigned kNil16 = 0xffffu;
-constexpr unsigned kFastErrTouched = 4u;      // == F3PS_MERGE_ERR_TOUCHED
+constexpr unsigned kFastErrTouched = 4u;
 constexpr unsigned kFastErrStamp = 8u;
 constexpr unsigned kFastErrPool = 16u;
 // BIG variant: a merge whose two adjacency lists hold more entries than there are worker threads (a floor or a wall of a dense scene
@@ -1123,7 +1123,7 @@ constexpr int kFastThreadsSolo = 768;                // one frame alone (f3ps_me
 template <bool PROF>
 __global__ void __launch_bounds__(kFastThreads, 1) merge_fast_big_kernel(const __grid_constant__ FastArgs A) { merge_lean_body<PROF, true>(A); }
 
-// A batch of frames in ONE launch, CTA i replays frame i (f3ps_merge_batch).  Independent streams share at most 32 hardware
+// A batch of frames in ONE launch, CTA i replays frame i (f3ps.cu: merge_frames).  Independent streams share at most 32 hardware
 // queues (CUDA_DEVICE_MAX_CONNECTIONS), so at most 32 single-CTA merge kernels ever overlap; one grid has no such limit.
 // The per-frame arguments travel in the kernel parameter space (<= 32,764 bytes on sm_70+ with CUDA >= 12.1).
 constexpr int kFastBatchMax = 32764 / (int)sizeof(FastArgs) < 96 ? 32764 / (int)sizeof(FastArgs) : 96;
@@ -1131,9 +1131,10 @@ struct FastBatch { FastArgs a[kFastBatchMax]; };
 static_assert(sizeof(FastBatch) <= 32764, "kernel parameter space");
 __global__ void __launch_bounds__(kFastThreads, 1) merge_fast_batch_kernel(const __grid_constant__ FastBatch B) { merge_lean_body<false>(B.a[blockIdx.x]); }
 
-// What follows a batch grid, for all its frames in three launches on the grid's stream (f3ps_merge_batch): the labelled cloud
-// of every frame (CTA i / grid row i = frame i, the bodies of dense_label_kernel and labeled_cloud_kernel), then every frame's
-// device scalars gathered into one array for a single copy to the host.
+// What follows a merge kernel, for every frame of its chunk in launches on the chunk's stream (f3ps.cu: launch_chunk):
+// Clustering::get_labeled_cloud (:640-663) of every frame (CTA i / grid row i = frame i), then, for a chunk of several frames,
+// their device scalars gathered into one array for a single copy to the host.  The kernels read the arrays through __restrict__
+// locals: that lets the compiler load them, owner[] among them, through the non-coherent path.
 struct LabelArgs {
     RegionArrays R; const unsigned* n_sv_ptr; const unsigned* run_start; const unsigned* run_end;
     unsigned* run_out_off; unsigned* run_dense; unsigned* region_dense; unsigned* n_out;
@@ -1143,9 +1144,53 @@ struct LabelArgs {
 };
 struct LabelBatch { LabelArgs a[kFastBatchMax]; };
 static_assert(sizeof(LabelBatch) <= 32764, "kernel parameter space");
+// dense labels 0..K-1 in ascending region label order; output offset of every run of every rope.  One block per frame: two
+// exclusive scans over the regions (alive flag -> dense label, voxel count -> output offset), then one thread per surviving
+// region walks its rope.
 __global__ void __launch_bounds__(1024) dense_label_batch_kernel(const __grid_constant__ LabelBatch B) {
     const LabelArgs& A = B.a[blockIdx.x];
-    dense_label_body(A.R, A.n_sv_ptr, A.run_start, A.run_end, A.run_out_off, A.run_dense, A.region_dense, A.n_out);
+    const RegionArrays R = A.R;
+    const unsigned* __restrict__ n_sv_ptr = A.n_sv_ptr; const unsigned* __restrict__ run_start = A.run_start;
+    const unsigned* __restrict__ run_end = A.run_end; unsigned* __restrict__ run_out_off = A.run_out_off;
+    unsigned* __restrict__ run_dense = A.run_dense; unsigned* __restrict__ region_dense = A.region_dense; unsigned* __restrict__ n_out = A.n_out;
+    __shared__ unsigned s_wa[32], s_wn[32];
+    __shared__ unsigned s_ca, s_cn;
+    const unsigned S = *n_sv_ptr;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) { s_ca = 0; s_cn = 0; }
+    __syncthreads();
+    for (unsigned base = 0; base < S; base += blockDim.x) {
+        const unsigned s = base + threadIdx.x;
+        const int nv = s < S ? R.n[s] : 0;
+        const unsigned alive = nv > 0 ? 1u : 0u, cnt = nv > 0 ? (unsigned)nv : 0u;
+        unsigned ia = alive, in = cnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned ta = __shfl_up_sync(kFull, ia, o), tn = __shfl_up_sync(kFull, in, o);
+            if (lane >= o) { ia += ta; in += tn; }
+        }
+        if (lane == 31) { s_wa[warp] = ia; s_wn[warp] = in; }
+        __syncthreads();
+        unsigned wa = 0, wn = 0;
+        for (int w = 0; w < warp; ++w) { wa += s_wa[w]; wn += s_wn[w]; }
+        const unsigned ca = s_ca, cn = s_cn;
+        if (s < S) {
+            if (!alive) region_dense[s] = 0xffffffffu;
+            else {
+                const unsigned dense = ca + wa + ia - 1u;
+                unsigned off = cn + wn + in - cnt;
+                region_dense[s] = dense;
+                for (int run = R.head[s]; run >= 0; run = R.next_run[run]) {
+                    run_out_off[run] = off; run_dense[run] = dense;
+                    off += run_end[run] - run_start[run];
+                }
+            }
+        }
+        __syncthreads();
+        if (threadIdx.x == blockDim.x - 1) { s_ca = ca + wa + ia; s_cn = cn + wn + in; }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *n_out = s_cn;
 }
 __global__ void __launch_bounds__(256) labeled_cloud_batch_kernel(const __grid_constant__ LabelBatch B) {
     const LabelArgs& A = B.a[blockIdx.y];
@@ -1154,7 +1199,16 @@ __global__ void __launch_bounds__(256) labeled_cloud_batch_kernel(const __grid_c
     const unsigned* __restrict__ run_dense = A.run_dense; const float4* __restrict__ vox_xyz = A.vox_xyz;
     float* __restrict__ out_xyz = A.out_xyz; unsigned* __restrict__ out_label = A.out_label; unsigned* __restrict__ out_voxel = A.out_voxel;
     unsigned* __restrict__ vox_segment = A.vox_segment; const unsigned* __restrict__ pos_label = A.pos_label; const unsigned* __restrict__ owner = A.owner;
-    F3PS_LABELED_CLOUD_LOOP
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += gridDim.x * blockDim.x) {
+        const unsigned run = pos_run[i];
+        if (run == 0xffffffffu) continue;                 // unowned voxel: absent from every region
+        const unsigned o = run_out_off[run] + (i - run_start[run]);
+        const unsigned v = order[i];
+        const float4 p = vox_xyz[v];
+        out_xyz[3 * (size_t)o] = p.x; out_xyz[3 * (size_t)o + 1] = p.y; out_xyz[3 * (size_t)o + 2] = p.z;
+        out_label[o] = run_dense[run]; out_voxel[o] = v;
+        if (!owner || owner[v] == pos_label[i]) vox_segment[v] = run_dense[run];   // a phantom leaf does not relabel its voxel
+    }
 }
 __global__ void scalars_gather_kernel(const __grid_constant__ LabelBatch B, unsigned words, unsigned* __restrict__ out) {
     const unsigned* __restrict__ src = B.a[blockIdx.x].scalars;

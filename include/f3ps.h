@@ -104,7 +104,8 @@ int f3ps_normals(f3ps_ctx* ctx);    /* K3 computeVoxelData */
 int f3ps_seeds(f3ps_ctx* ctx);      /* K4 selectInitialSupervoxelSeeds */
 int f3ps_expand(f3ps_ctx* ctx);     /* K5 expandSupervoxels */
 int f3ps_graph(f3ps_ctx* ctx);      /* K6 makeSupervoxels + getSupervoxelAdjacency + set_initialstate + init_weights */
-int f3ps_merge(f3ps_ctx* ctx, float threshold); /* K7 Clustering::cluster(threshold): restarts from the initial state */
+/* K7 Clustering::cluster(threshold): restarts from the initial state.  The same as f3ps_merge_batch of this one handle. */
+int f3ps_merge(f3ps_ctx* ctx, float threshold);
 /* Grid of K5's cooperative launch.  ctas_per_frame = 0 (default): the whole GPU -- lowest latency for one frame, but
  * cooperative launches of concurrent frames run one at a time.  ctas_per_frame > 0: the grid is capped at that many CTAs (a
  * sweep trades the latency of one frame for more frames side by side).  max_concurrent must be 0; other values, and
@@ -128,7 +129,8 @@ int f3ps_set_expand_kernel(f3ps_ctx* ctx, int which, int cluster_ctas);
  * CTA i replays frame i.  Independent streams share at most 32 hardware queues per context, so a sweep with one merge
  * kernel per stream never overlaps more than 32 of them; a grid has no such limit.  Same results per handle as f3ps_merge;
  * handles whose graph does not fit the resident kernel's shared memory, or whose kernel choice is not 0, are clustered
- * individually, as f3ps_merge would. */
+ * individually, as f3ps_merge would, next to the grids.  A batch of one handle is f3ps_merge, and a grid-able frame left
+ * alone (one handle, or the last of more than a grid holds) runs the kernel f3ps_merge would give it, not a one-CTA grid. */
 int f3ps_merge_batch(f3ps_ctx** ctxs, int n, float threshold);
 /* How the host waits where it needs a size from the device: 0 = spin (lowest latency, the default), 1 = sleep on a
  * blocking event.  Sweeps that keep more frames in flight than there are host cores must use 1. */

@@ -106,6 +106,27 @@ def test_members_usable_on_their_own_streams_right_after(gpu):
             assert np.array_equal(r[n], a), (k, n)
 
 
+@pytest.mark.parametrize("kind,path", [("c2", 1), ("hub", 6)])
+def test_batch_of_one_is_merge(gpu, kind, path):
+    """A batch of one handle is f3ps_merge: a lone frame that fits the shared-memory kernel runs its own build rather than a
+    one-CTA grid (path 1), and a hub graph continues on the L2 variant in front of its first wide merge (path 6)."""
+    from f3ps import synth
+
+    def handle():
+        if kind == "c2":
+            return frame_handle(gpu, synth.make_frame(seed=20020))
+        h = gpu.Segmenter(); h.set_merge_params(**AL); h.set_graph(*hub_graph(1500))
+        return h
+    a, b = handle(), handle()
+    la, lb = a.launch_count(), b.launch_count()
+    a.merge(THR)
+    gpu.merge_batch([b], THR)
+    assert a.counts().merge_path == b.counts().merge_path == path
+    assert a.launch_count() - la == b.launch_count() - lb
+    assert sorted(a.stage_ms()) == sorted(b.stage_ms())
+    assert_same(result(gpu, b, kind == "c2"), result(gpu, a, kind == "c2"), kind)
+
+
 def test_chunk_launches_do_not_grow_with_frames(gpu):
     from f3ps import synth
     segs = [frame_handle(gpu, synth.make_frame(seed=700 + i, width=160, height=120)) for i in range(8)]

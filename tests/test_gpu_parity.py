@@ -540,9 +540,13 @@ def test_general_merge_kernel_hub_graph(gpu, oracle_mod, n_leaves, mode):
     assert same(g.array("merges_w"), o.array("merges_w"))
     assert np.array_equal(g.array("out_label"), o.array("out_label"))
     if S <= 4096:
-        # one grid for many frames (f3ps_merge_batch): this frame's CTA stops in front of its first wide merge and the handle
-        # continues from that state on the L2 variant
-        gpu.merge_batch([g], thr)
+        # one grid for many frames (f3ps_merge_batch; a 160x120 frame beside it makes the pair a grid): this frame's CTA stops in
+        # front of its first wide merge and the handle continues from that state on the L2 variant
+        from f3ps import synth
+        p = gpu.Segmenter(); p.set_vccs_params(); p.set_merge_params(**flags)
+        p.set_input(synth.make_frame(seed=11, width=160, height=120)); p.extract(); p.graph()
+        gpu.merge_batch([g, p], thr)
+        assert p.counts().merge_path == 1
         assert g.counts().merge_path == 6, g.counts().merge_path
         assert np.array_equal(g.array("merges_ab"), o.array("merges_ab")) and same(g.array("merges_w"), o.array("merges_w"))
         assert np.array_equal(g.array("out_label"), o.array("out_label"))
